@@ -889,8 +889,8 @@ def jacobian(arr, kin, body, point):
 
 
 def default_assets_root() -> Optional[Path]:
-    """Where the reference's ``hsr/`` package directory (models + meshes) lives, if present."""
-    for cand in (os.environ.get("HSR_ASSETS"), "/root/reference/hsr"):
-        if cand and Path(cand, "models", "world.xml").exists():
-            return Path(cand)
+    """Where the reference's ``hsr/`` package directory (models + meshes) lives: ``$HSR_ASSETS``, if it holds the models."""
+    cand = os.environ.get("HSR_ASSETS")
+    if cand and Path(cand, "models", "world.xml").exists():
+        return Path(cand)
     return None

@@ -1,15 +1,16 @@
-"""Runs the REFERENCE's own ``mutate_xml`` (/root/reference/hsr/util.py:87-182) under stubbed ``gym`` / ``mujoco_py``
+"""Runs the REFERENCE's own ``mutate_xml`` (hsr/util.py:87-182) under stubbed ``gym`` / ``mujoco_py``
 and writes a digest of the mutated MJCF trees (sha256 of their canonical form + the joints / actuators / block bodies
 that survive the mutation) to tests/golden/mutate.json, the fixture tests/test_mutate_xml.py compares
 hsr_env_b200.mjcf.mutate_tree with.  (The trees themselves are the reference's model files and are not copied here.)
 
-    python tests/golden/make_mutate_golden.py        # needs /root/reference (this container only)
+    HSR_REFERENCE=<checkout of the reference> python tests/golden/make_mutate_golden.py
 """
 import contextlib
 import hashlib
 import json
 import importlib.util
 import io
+import os
 import sys
 import types
 import xml.etree.ElementTree as ET
@@ -17,7 +18,7 @@ from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference")
+REF = Path(os.environ["HSR_REFERENCE"]) if os.environ.get("HSR_REFERENCE") else None   # the reference's repository
 OUT = Path(__file__).resolve().parent / "mutate.json"
 
 ALL_DOFS = ["slide_x", "slide_y", "arm_lift_joint", "arm_flex_joint", "wrist_roll_joint", "hand_l_proximal_joint", "hand_r_proximal_joint"]
@@ -116,6 +117,8 @@ def digest(trees):
 
 
 def main():
+    if REF is None:
+        sys.exit("set HSR_REFERENCE to a checkout of the reference's repository")
     mod = load_reference_util()
     res = {case: digest(reference_mutation(mod, case)) for case in CASES}
     OUT.write_text(json.dumps(res, indent=1))

@@ -1,17 +1,20 @@
-"""Golden fixture of the reference's own ReplayBuffer (rl_utils/replay_buffer.py, imported from /root/reference under a
-stubbed gym): a scripted sequence of extend / append / indexed reads, with everything the reference returned.  The GPU
-test replays the script on the device-resident buffer (the reference tree does not exist on the GPU box).
+"""Golden fixture of the reference's own ReplayBuffer (rl_utils/replay_buffer.py, imported from a checkout of the
+reference under a stubbed gym): a scripted sequence of extend / append / indexed reads, with everything the reference
+returned.  The tests replay the script on the buffer, on the host and on the device, without the reference.
 
-    python tests/golden/make_replay_golden.py   ->  tests/golden/replay.npz
+    HSR_REFERENCE=<checkout of the reference> python tests/golden/make_replay_golden.py   ->  tests/golden/replay.npz
 """
 import importlib
+import os
 import sys
 import types
 from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference")
+if not os.environ.get("HSR_REFERENCE"):
+    sys.exit("set HSR_REFERENCE to a checkout of the reference's repository")
+REF = Path(os.environ["HSR_REFERENCE"])
 gym = types.ModuleType("gym"); gym.spaces = types.ModuleType("gym.spaces")
 gym.Env = object; gym.Space = object; gym.Wrapper = object
 for n in ("Box", "Discrete", "Dict", "Tuple", "Space"):

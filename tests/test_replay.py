@@ -1,7 +1,8 @@
 """Row f3 (SURVEY.md §8f): the device-resident replay buffer keeps the ring semantics of the reference's
-rl_utils.replay_buffer.ReplayBuffer.  Compared with the reference implementation itself where /root/reference is present
-(this container), and through self-contained properties everywhere."""
+rl_utils.replay_buffer.ReplayBuffer.  Compared with the reference implementation itself where HSR_REFERENCE names a
+checkout of it, with its recorded outputs (tests/golden/replay.npz), and through self-contained properties everywhere."""
 import importlib
+import os
 import sys
 import types
 from pathlib import Path
@@ -10,25 +11,25 @@ import numpy as np
 import pytest
 
 torch = pytest.importorskip("torch")
-REF = Path("/root/reference")
+REF = os.environ.get("HSR_REFERENCE", "")   # a checkout of the reference's repository
 
 
 def reference_buffer_class():
-    if not (REF / "rl_utils" / "replay_buffer.py").exists():
-        pytest.skip("reference tree not present")
+    if not REF or not Path(REF, "rl_utils", "replay_buffer.py").exists():
+        pytest.skip("the reference's repository is not part of this one: set HSR_REFERENCE")
     if "gym" not in sys.modules:   # rl_utils/__init__ imports gym; only its names are needed to import the package
         gym = types.ModuleType("gym"); gym.spaces = types.ModuleType("gym.spaces")
         gym.Env = object; gym.Space = object; gym.Wrapper = object
         for n in ("Box", "Discrete", "Dict", "Tuple", "Space"):
             setattr(gym.spaces, n, type(n, (), {}))
         sys.modules["gym"] = gym; sys.modules["gym.spaces"] = gym.spaces
-    sys.path.insert(0, str(REF))
+    sys.path.insert(0, REF)
     try:
         return importlib.import_module("rl_utils.replay_buffer").ReplayBuffer
     except Exception as e:  # noqa: BLE001
         pytest.skip(f"reference rl_utils not importable here: {e!r}")
     finally:
-        sys.path.remove(str(REF))
+        sys.path.remove(REF)
 
 
 def batches(rng, k):
