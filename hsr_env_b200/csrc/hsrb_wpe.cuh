@@ -20,7 +20,9 @@
 #pragma once
 #include "hsrb_push.cuh"
 
+#ifndef WPE_MAXCON
 #define WPE_MAXCON 8                       // contacts per environment (as the lock-step kernel)
+#endif
 #define WPE_GROUPS (WPE_MAXCON + 2)        // constraint groups: contacts + the two slide limits
 #define WPE_SLOTS (6 * WPE_GROUPS)         // six row slots per group (rows >= the group's dimension are zero rows)
 #define WPE_MAXROW (6 * WPE_MAXCON + 2)    // MuJoCo's nefc at capacity

@@ -15,7 +15,9 @@ void run(const KArgs& a, int grid, size_t smem) {
 }
 }  // namespace
 
-extern "C" int emu_general_step(const void* blob, size_t bytes, int G, int n, int nsub, const double* qpos, const double* qvel,
+// ncon_max / nefc_max > 0 replace the model's capacities (as hsrb_config does on the device)
+extern "C" int emu_general_step(const void* blob, size_t bytes, int G, int n, int nsub, int ncon_max, int nefc_max,
+                                const double* qpos, const double* qvel,
                                 const double* warm, const double* ctrl, double* qpos_o, double* qvel_o, double* warm_o,
                                 int* taken, unsigned char* flags, long long* stats_out) {
   HostModel<float> hm;
@@ -36,6 +38,8 @@ extern "C" int emu_general_step(const void* blob, size_t bytes, int G, int n, in
   KArgs a;
   memset(&a, 0, sizeof(a));
   a.m = m;
+  if (ncon_max > 0) a.m.ncon_max = ncon_max;
+  if (nefc_max > 0) a.m.nefc_max = nefc_max;
   a.n = n; a.S = S; a.nsub = nsub; a.mode = MODE_STEP;
   a.ws_bytes = (unsigned)ws_carve<float>(a.m, nullptr, nullptr);
   a.state = state.data(); a.ctrl = c32.data(); a.obs = obs.data(); a.reward = reward.data(); a.done = done.data();
