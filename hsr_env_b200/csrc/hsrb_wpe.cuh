@@ -52,6 +52,11 @@ struct alignas(16) Tab {   // block-shared model tables (one copy per block)
   int gmove[WPE_MAXGEOM], geom_type[WPE_MAXGEOM], geom_vertadr[WPE_MAXGEOM], geom_vertnum[WPE_MAXGEOM];
   int pair_geom1[WPE_MAXPAIR], pair_geom2[WPE_MAXPAIR], pair_func[WPE_MAXPAIR], pair_condim[WPE_MAXPAIR];
   float pair_sr[WPE_MAXPAIR], pair_sb[WPE_MAXPAIR];   // sign of the pair's contact Jacobian on the robot / block dofs
+  // per-block constants read where they are used instead of being held in registers across the substep
+  int gb0;                                   // first geom riding on the block
+  float blk_radius;                          // farthest point of the block's geoms from its body origin
+  int wpt;                                   // warps per team (phase-locked variant)
+  unsigned char team[WPE_MAXWARPS];          // team of each warp
 };
 
 struct alignas(16) Slice {   // per-warp (= per-environment) slice
@@ -83,8 +88,13 @@ static_assert(offsetof(Slice, J) % 16 == 0 && offsetof(Slice, PQ) % 16 == 0 && o
               offsetof(Slice, warm) % 16 == 0 && offsetof(Slice, as) % 16 == 0 && sizeof(Slice) % 16 == 0,
               "128-bit shared-memory accesses (push::ld8 / st8) need 16-byte aligned fields");
 __host__ __device__ inline size_t slice_bytes() { return sizeof(Slice); }
-// block-shared tail after the slices: the tables, the job queue, then the hull vertices as float4
-__host__ __device__ inline size_t shared_tail(const ModelT<float>& m) { return sizeof(Tab) + sizeof(Queue) + (size_t)m.nvert * 16 + 16; }
+// Shared memory of a block: [Tab | Queue | slice 0 .. wpb-1 | hull vertices as float4].  The tables and the queue sit at
+// offset 0, so their fields are LDS / STS with absolute addresses and no register holds their base; a slice is one 32-bit
+// offset from the warp index.
+constexpr unsigned SMEM_HEAD = (unsigned)(sizeof(Tab) + sizeof(Queue));
+static_assert(SMEM_HEAD % 16 == 0, "the slices start 16-byte aligned");
+// block-shared bytes besides the slices: the tables, the job queue and the hull vertices
+__host__ __device__ inline size_t shared_tail(const ModelT<float>& m) { return SMEM_HEAD + (size_t)m.nvert * 16 + 16; }
 
 }  // namespace wpe
 
@@ -93,6 +103,17 @@ __host__ __device__ inline size_t shared_tail(const ModelT<float>& m) { return s
 namespace wpe {
 
 typedef V3<double> V3d;
+
+__device__ __forceinline__ unsigned char* smem_base() {
+  HSRB_DYN_SMEM(smem);
+  return smem;
+}
+__device__ __forceinline__ Tab& tab() { return *reinterpret_cast<Tab*>(smem_base()); }
+__device__ __forceinline__ Queue& queue() { return *reinterpret_cast<Queue*>(smem_base() + sizeof(Tab)); }
+__device__ __forceinline__ Slice& slice(int w) { return *reinterpret_cast<Slice*>(smem_base() + SMEM_HEAD + (unsigned)w * (unsigned)sizeof(Slice)); }
+__device__ __forceinline__ float* hull_verts4() {
+  return reinterpret_cast<float*>(smem_base() + SMEM_HEAD + (blockDim.x >> 5) * (unsigned)sizeof(Slice));
+}
 
 // -DWPE_CHAIN_CLOCKS: cycle counters of the sections of ONE environment's dependent chain (lane 0 of every warp, clock64
 // deltas accumulated with fire-and-forget atomics); read with hsrb_debug_chain_clocks().  Meant for the free-running
@@ -185,10 +206,17 @@ __device__ __forceinline__ void pcopy(Slice& s, int dst, int src) {
 // hsr::mpr_penetration_inl, restructured around ONE support evaluation site (a state machine) with the portal in shared
 // memory: a few hundred instructions of code and a handful of live doubles instead of five 9-double vertices in
 // registers.  `sep`: cached separating direction of the pair (see hsr::mpr_penetration_inl).  Result -> s.mres.
-// o: the slice of the environment the pair belongs to (poses, cached direction); s: the executing warp's slice (portal
-// scratch, result) - the same slice unless the warp serves another environment's job (phase-locked variant).
-__device__ __noinline__ bool mpr(const Tab& t, const Slice& o, Slice& s, const float* verts4, int g1, int g2, int gb0, double tol,
-                                 int max_iter, float* sep) {
+// ow: the warp whose slice holds the environment the pair belongs to (poses, cached direction o.sep + 4 sepk, none if
+// sepk < 0); s: the executing warp's slice (portal scratch, result) - the same slice unless the warp serves another
+// environment's job (phase-locked variant).  Every argument is one 32-bit register: the tables, the slices and the hull
+// vertices are addressed from the fixed shared-memory layout, so the call carries no 64-bit pointers.
+__device__ __noinline__ bool mpr(int ow, int g1, int g2, int gb0, float tol_f, int max_iter, int sepk) {
+  const Tab& t = tab();
+  const Slice& o = slice(ow);
+  Slice& s = slice(threadIdx.x >> 5);
+  const float* const verts4 = hull_verts4();
+  float* const sep = sepk >= 0 ? slice(ow).sep + 4 * sepk : nullptr;
+  const double tol = (double)tol_f;
   double* const out7 = s.mres;   // depth, direction, position (written by lane 0)
   double* const P = s.portal;    // P[9 k ..]: portal vertex k = v | v1 | v2 (k = 0 .. 4), P[45 .. 47]: the current direction
   const int lane = threadIdx.x & 31;
@@ -354,6 +382,8 @@ __device__ __noinline__ bool mpr(const Tab& t, const Slice& o, Slice& s, const f
 #undef WPE_NEXT_DIR
 }
 
+__device__ __forceinline__ int* team_jobs(Queue& Q, const Tab& t, int w) { return Q.jobs + t.team[w] * t.wpt * WPE_ENVJOBS; }
+
 }  // namespace wpe
 
 // ---------------------------------------------------------------------------------------------------- the kernel
@@ -373,14 +403,13 @@ __device__ __noinline__ bool mpr(const Tab& t, const Slice& o, Slice& s, const f
 #endif
 template <bool LOCK>
 __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const __grid_constant__ KArgs a, const __grid_constant__ PushInfo fi) {
-  HSRB_DYN_SMEM(smem);
   constexpr unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
   const ModelT<float>& m = a.m;
-  // ---- block-shared: model tables + hull vertices as float4 (one copy per block), after the warps' slices
-  wpe::Tab& tw = *reinterpret_cast<wpe::Tab*>(smem + (size_t)wpb * sizeof(wpe::Slice));
-  wpe::Queue& Q = *reinterpret_cast<wpe::Queue*>(smem + (size_t)wpb * sizeof(wpe::Slice) + sizeof(wpe::Tab));
-  float* const v4w = reinterpret_cast<float*>(smem + (size_t)wpb * sizeof(wpe::Slice) + sizeof(wpe::Tab) + sizeof(wpe::Queue));
+  // ---- block-shared: model tables + hull vertices as float4 (one copy per block); layout: wpe::SMEM_HEAD
+  wpe::Tab& tw = wpe::tab();
+  wpe::Queue& Q = wpe::queue();
+  float* const v4w = wpe::hull_verts4();
   {
     const int ng = m.ngeom, np = m.npair;
     for (int i = threadIdx.x; i < m.nvert * 4; i += blockDim.x) v4w[i] = fi.verts4[i];
@@ -393,6 +422,19 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
       int gb0_ = ng;
       for (int i = ng - 1; i >= 0; i--) if (fi.gmove[i] == 2) gb0_ = i;
       for (int i = threadIdx.x; i < (ng - gb0_) * 9 && i < WPE_MAXBG * 9; i += blockDim.x) tw.bgeom_mat[i] = m.geom_mat[9 * gb0_ + i];
+      if (threadIdx.x == 0) {
+        float blk_radius = 0.f;
+        for (int i = gb0_; i < ng; i++) {
+          const double* o3 = fi.gbase + 3 * i;
+          blk_radius = fmaxf(blk_radius, (float)sqrt(o3[0] * o3[0] + o3[1] * o3[1] + o3[2] * o3[2]) * 1.001f + m.geom_rbound[i]);
+        }
+        tw.gb0 = gb0_; tw.blk_radius = blk_radius;
+      }
+      // teams of the phase-locked variant: opts bits 4..7 = number of teams (0 -> 1); the warps of a team are contiguous
+      int nteam = LOCK ? (int)((a.opts >> 4) & 15u) : 1;
+      if (nteam < 1 || nteam > WPE_MAXTEAMS || wpb % nteam != 0) nteam = 1;
+      if (threadIdx.x == 0) tw.wpt = wpb / nteam;
+      if (threadIdx.x < wpb) tw.team[threadIdx.x] = (unsigned char)(threadIdx.x / (wpb / nteam));
     }
     TAB_COPY(gmove, fi.gmove, ng) TAB_COPY(geom_type, m.geom_type, ng)
     TAB_COPY(geom_vertadr, m.geom_vertadr, ng) TAB_COPY(geom_vertnum, m.geom_vertnum, ng)
@@ -409,38 +451,26 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
   }
   const wpe::Tab& t = tw;
   const float* const verts4 = v4w;
-  wpe::Slice& s = *reinterpret_cast<wpe::Slice*>(smem + (size_t)wib * sizeof(wpe::Slice));
+  wpe::Slice& s = wpe::slice(wib);
   const int NV = fi.nv;
   const bool HASB = NV == 8;
   const int nq = m.nq;
   const float dt = m.timestep;
-  const float scale = 1.0f / (m.meaninertia * (float)(NV > 1 ? NV : 1));
   const int li = lane & 7, sub = lane >> 3;   // dof owned by this lane, row stripe of this lane
-  int gb0 = m.ngeom;                          // first geom riding on the block
-  for (int i = m.ngeom - 1; i >= 0; i--) if (t.gmove[i] == 2) gb0 = i;
+  const float scale = 1.0f / (m.meaninertia * (float)(NV > 1 ? NV : 1));
   const float Mi = li < NV ? fi.Mdiag[li] : 1.0f, dampi = li < NV ? fi.damp[li] : 0.f;
   const bool use_sep = !(a.opts & 1u);
   const bool use_gap = use_sep && !(a.opts & 0x10000u);   // opts bit 16: no gap budget (every cached direction is re-checked every substep)
-  float blk_radius = 0.f;   // farthest point of the block's geoms from its body origin
-  for (int i = gb0; i < m.ngeom; i++) {
-    const double* o3 = t.gbase + 3 * i;
-    blk_radius = fmaxf(blk_radius, (float)sqrt(o3[0] * o3[0] + o3[1] * o3[1] + o3[2] * o3[2]) * 1.001f + t.geom_rbound[i]);
-  }
-  // teams of the phase-locked variant: opts bits 4..7 = number of teams (0 -> 1); the warps of a team are contiguous
-  int nteam = LOCK ? (int)((a.opts >> 4) & 15u) : 1;
-  if (nteam < 1 || nteam > WPE_MAXTEAMS || wpb % nteam != 0) nteam = 1;
-  const int wpt = wpb / nteam, team = wib / wpt, tthreads = 32 * wpt;
-  int* const qcnt = Q.cnt[team];
+  // this warp's team t.team[wib] (t.wpt warps) and its share of the job queue (Q.cnt[team], wpe::team_jobs) are read from
+  // the tables where used instead of being held in registers
 #if !defined(HSRB_SIMT_EMU)
   // experiment: opts bits 8..15 = start stagger of team k in units of 4 us x k (teams that start in phase stay in phase on
   // uniform work and then compete for the same pipes in every phase)
-  if (LOCK && team > 0 && ((a.opts >> 8) & 255u)) {
-    const long long t0 = clock64(), wait = (long long)((a.opts >> 8) & 255u) * 4 * 1965 * team;
+  if (LOCK && t.team[wib] > 0 && ((a.opts >> 8) & 255u)) {
+    const long long t0 = clock64(), wait = (long long)((a.opts >> 8) & 255u) * 4 * 1965 * t.team[wib];
     while (clock64() - t0 < wait) __nanosleep(1000);
   }
 #endif
-  int* const qjobs = Q.jobs + team * wpt * WPE_ENVJOBS;
-  const int qcap = wpt * WPE_ENVJOBS;
 #if defined(WPE_DEBUG_JOBS)
   long long dbg_long = 0, dbg_quick = 0; int dbg_nlong = 0, dbg_nquick = 0, dbg_hits = 0, dbg_jobs_total = 0, dbg_long_total = 0, dbg_sub = 0;
 #endif
@@ -487,7 +517,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
 
 #pragma unroll 1
     for (int sb_ = 0; sb_ < a.nsub; sb_++) {
-      if (LOCK) { if (wpe::team_and(team, tthreads, finished)) break; }
+      if (LOCK) { if (wpe::team_and(t.team[wib], 32 * t.wpt, finished)) break; }
       else if (finished) break;
 #if defined(HSRB_PHASE_CLOCKS)
       if (LOCK && threadIdx.x == 0) tlast = clock64();
@@ -523,15 +553,15 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
             const double* Rb = s.Rb;
             const wpe::V3d p = ld3(s.xb) + mulv(Rb, ld3(t.gbase + 3 * gg));
             st3(s.gpos + 3 * gg, p);
-            mulm(Rb, t.gmatw + 9 * gg, s.bmat + 9 * (gg - gb0));
+            mulm(Rb, t.gmatw + 9 * gg, s.bmat + 9 * (gg - t.gb0));
             float Rbf[9], Rg[9];
 #pragma unroll
             for (int k = 0; k < 9; k++) Rbf[k] = (float)Rb[k];
-            mulm(Rbf, t.bgeom_mat + 9 * (gg - gb0), Rg);
+            mulm(Rbf, t.bgeom_mat + 9 * (gg - t.gb0), Rg);
             const float* h = t.geom_aabb + 3 * gg;
 #pragma unroll
             for (int i = 0; i < 3; i++)
-              s.baabb[4 * (gg - gb0) + i] = fabsf(Rg[3 * i]) * h[0] + fabsf(Rg[3 * i + 1]) * h[1] + fabsf(Rg[3 * i + 2]) * h[2];
+              s.baabb[4 * (gg - t.gb0) + i] = fabsf(Rg[3 * i]) * h[0] + fabsf(Rg[3 * i + 1]) * h[1] + fabsf(Rg[3 * i + 2]) * h[2];
           }
         }
       }
@@ -584,8 +614,8 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
           } else {
             const float rr = t.geom_rbound[ga] + t.geom_rbound[gb];
             hit = dot(dp, dp) <= rr * rr;
-            const float* ha = t.gmove[ga] == 2 ? s.baabb + 4 * (ga - gb0) : t.ghalf + 3 * ga;
-            const float* hb = t.gmove[gb] == 2 ? s.baabb + 4 * (gb - gb0) : t.ghalf + 3 * gb;
+            const float* ha = t.gmove[ga] == 2 ? s.baabb + 4 * (ga - t.gb0) : t.ghalf + 3 * ga;
+            const float* hb = t.gmove[gb] == 2 ? s.baabb + 4 * (gb - t.gb0) : t.ghalf + 3 * gb;
             hit = hit && fabsf(dp.x) <= ha[0] + hb[0] && fabsf(dp.y) <= ha[1] + hb[1] && fabsf(dp.z) <= ha[2] + hb[2];
           }
         }
@@ -598,7 +628,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
           float f = s.sep[4 * k + 3];
           if (f < 0.f) {
             const float moved = dt * 1.001f * (fabsf(s.qvel[0]) + fabsf(s.qvel[1]) + fabsf(s.qvel[2]) + fabsf(s.qvel[3]) + fabsf(s.qvel[4]) +
-                                               (fabsf(s.qvel[5]) + fabsf(s.qvel[6]) + fabsf(s.qvel[7])) * blk_radius) + 5e-8f;
+                                               (fabsf(s.qvel[5]) + fabsf(s.qvel[6]) + fabsf(s.qvel[7])) * t.blk_radius) + 5e-8f;
             f += moved;
             if (f < -1e-6f) skip = hit; else f = 1.f;   // budget used up: the next query re-measures the gap with one support evaluation
             s.sep[4 * k + 3] = f;
@@ -606,6 +636,13 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
         }
         bits = __ballot_sync(FULL, hit && !skip);
         nskip = __popc(__ballot_sync(FULL, skip));
+        // narrowphase work counters of the substep, counted here rather than carried through the collision loop: one query
+        // per candidate; pairs settled by the gap budget still count as the reference's convex-convex query
+        const int fk = (hit && !skip) ? t.pair_func[k] : -1;
+        const int npb = __popc(__ballot_sync(FULL, fk == NP_PLANE_BOX)), npc = __popc(__ballot_sync(FULL, fk == NP_PLANE_CONVEX)),
+                  nbb = __popc(__ballot_sync(FULL, fk == NP_BOX_BOX));
+        narrow = __popc(bits) + nskip;
+        npflop = 80 * npb + 100 * npc + 500 * nbb + 5000 * (narrow - npb - npc - nbb);
       }
       WPE_CK(1);
       if (LOCK && lane == 0) {
@@ -621,8 +658,8 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
           if (kc < WPE_ENVJOBS) {
             const bool quick = use_sep && (s.sep[4 * pk + 3] == 1.f || s.sep[4 * pk + 3] < 0.f);
             const int code = (wib << 16) | (kc << 8) | pk;
-            if (quick) qjobs[qcap - 1 - atomicAdd(&qcnt[1], 1)] = code;
-            else qjobs[atomicAdd(&qcnt[0], 1)] = code;
+            if (quick) wpe::team_jobs(Q, t, wib)[(t.wpt * WPE_ENVJOBS) - 1 - atomicAdd(&Q.cnt[t.team[wib]][1], 1)] = code;
+            else wpe::team_jobs(Q, t, wib)[atomicAdd(&Q.cnt[t.team[wib]][0], 1)] = code;
           }
           kc++;
         }
@@ -630,27 +667,27 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
       }
       if (LOCK) {
         WPE_PH(PH_KIN);
-        wpe::team_sync(team, tthreads);
+        wpe::team_sync(t.team[wib], 32 * t.wpt);
         WPE_PH(PH_CRB);
         // ---- every warp of the block (finished ones included) serves jobs: the owner's poses, this warp's portal scratch
         // (a team without jobs in this substep - the usual case for light environments since the gap budget - skips the
         //  service and its closing barrier: the counters are not written again before the next two team barriers)
-        const int nlong = qcnt[0], njobs = nlong + qcnt[1];
+        const int nlong = Q.cnt[t.team[wib]][0], njobs = nlong + Q.cnt[t.team[wib]][1];
         if (njobs > 0 || (a.opts & 0x20000u)) {   // opts bit 17: always run the service and its barrier (experiments)
 #pragma unroll 1
         while (true) {
           int j = 0;
-          if (lane == 0) j = atomicAdd(&qcnt[2], 1);
+          if (lane == 0) j = atomicAdd(&Q.cnt[t.team[wib]][2], 1);
           j = __shfl_sync(FULL, j, 0);
           if (j >= njobs) break;
-          const int code = j < nlong ? qjobs[j] : qjobs[qcap - 1 - (j - nlong)];
+          const int code = j < nlong ? wpe::team_jobs(Q, t, wib)[j] : wpe::team_jobs(Q, t, wib)[(t.wpt * WPE_ENVJOBS) - 1 - (j - nlong)];
 #if defined(WPE_DEBUG_JOBS)
           const long long tj0 = clock64();
 #endif
           const int pk = code & 255;
-          wpe::Slice& o = *reinterpret_cast<wpe::Slice*>(smem + (size_t)(code >> 16) * sizeof(wpe::Slice));
-          const bool hitc = wpe::mpr(t, o, s, verts4, t.pair_geom1[pk], t.pair_geom2[pk], gb0, (double)m.mpr_tolerance, m.mpr_iterations,
-                                     use_sep ? o.sep + 4 * pk : nullptr);
+          wpe::Slice& o = wpe::slice(code >> 16);
+          const bool hitc = wpe::mpr(code >> 16, t.pair_geom1[pk], t.pair_geom2[pk], t.gb0, m.mpr_tolerance, m.mpr_iterations,
+                                     use_sep ? pk : -1);
           if (lane == 0) {
             float* r = o.jres + 14 * ((code >> 8) & 255);
             r[0] = hitc ? 1.f : 0.f;
@@ -669,9 +706,9 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
         if (threadIdx.x == 0) { dbg_jobs_total += njobs; dbg_long_total += nlong; dbg_sub++; }
 #endif
         WPE_PH(PH_SMOOTH);
-        wpe::team_sync(team, tthreads);
+        wpe::team_sync(t.team[wib], 32 * t.wpt);
         WPE_PH(PH_COLLIDE);
-        if (wib == team * wpt && lane < 3) qcnt[lane] = 0;   // empty again; the next jobs are queued after the solver's barrier
+        if (wib == t.team[wib] * t.wpt && lane < 3) Q.cnt[t.team[wib]][lane] = 0;   // empty again; the next jobs are queued after the solver's barrier
         }
       }
       if (!finished) {
@@ -684,8 +721,6 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
           const int func = t.pair_func[pk];
           const int ga = t.pair_geom1[pk], gb = t.pair_geom2[pk];
           const int dim = t.pair_condim[pk];
-          narrow++;
-          npflop += func == NP_PLANE_BOX ? 80 : (func == NP_PLANE_CONVEX ? 100 : (func == NP_BOX_BOX ? 500 : 5000));
           if (func == NP_PLANE_BOX) {
             // mjc_PlaneBox: one corner per lane; the first four penetrating corners (corner order) become contacts
             const double* Ma = t.gmatw + 9 * ga;
@@ -696,7 +731,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
             const float* sz = t.geom_size + 3 * gb;
             const wpe::V3d c = mk<double>((i & 1) ? (double)sz[0] : -(double)sz[0], (i & 2) ? (double)sz[1] : -(double)sz[1],
                                           (i & 4) ? (double)sz[2] : -(double)sz[2]);
-            const wpe::V3d vec = mulv(wpe::geom_mat(t, s, gb, gb0), c);
+            const wpe::V3d vec = mulv(wpe::geom_mat(t, s, gb, t.gb0), c);
             const double ld = dot(n, vec);
             const bool pen = i < 8 && !(dist0 + ld > 0 || ld > 0);
             const unsigned pm = __ballot_sync(FULL, pen);
@@ -737,7 +772,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
             if (func == NP_PLANE_CONVEX) {
               const double* Ma = t.gmatw + 9 * ga;
               const wpe::V3d n = mk<double>(Ma[2], Ma[5], Ma[8]);
-              const wpe::V3d p = wpe::support(t, s, verts4, gb, gb0, -n);
+              const wpe::V3d p = wpe::support(t, s, verts4, gb, t.gb0, -n);
               const double dist = dot(p - ld3(s.gpos + 3 * ga), n);
               hitc = dist <= 0;
               const wpe::V3d pos = p - n * (dist * 0.5);
@@ -745,7 +780,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
               if (lane == 0) { double* r7 = s.mres; r7[0] = -dist; r7[1] = n.x; r7[2] = n.y; r7[3] = n.z; r7[4] = pos.x; r7[5] = pos.y; r7[6] = pos.z; }
               __syncwarp();
             } else {
-              hitc = wpe::mpr(t, s, s, verts4, ga, gb, gb0, (double)m.mpr_tolerance, m.mpr_iterations, use_sep ? s.sep + 4 * pk : nullptr);
+              hitc = wpe::mpr(wib, ga, gb, t.gb0, m.mpr_tolerance, m.mpr_iterations, use_sep ? pk : -1);
             }
             if (hitc) {
               if (func == NP_CONVEX_CONVEX && lane == 0) s.acc[A_HIT]++;
@@ -771,7 +806,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
 #pragma unroll
             for (int q = 0; q < 3; q++) { A.size[q] = t.geom_size[3 * ga + q]; B.size[q] = t.geom_size[3 * gb + q]; }
             A.pos = ld3(s.gpos + 3 * ga); B.pos = ld3(s.gpos + 3 * gb);
-            const double* RA = wpe::geom_mat(t, s, ga, gb0); const double* RB = wpe::geom_mat(t, s, gb, gb0);
+            const double* RA = wpe::geom_mat(t, s, ga, t.gb0); const double* RB = wpe::geom_mat(t, s, gb, t.gb0);
 #pragma unroll
             for (int q = 0; q < 9; q++) { A.mat[q] = RA[q]; B.mat[q] = RB[q]; }
             int nrow_ = nefc;
@@ -786,7 +821,6 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
       __syncwarp();
       ngrp = nlimit + ncon;
       nslot = 6 * ngrp;
-      narrow += nskip; npflop += 5000 * nskip;   // pairs settled by the gap budget still count as the reference's narrowphase work
       if (lane == 0) { s.acc[A_NARROW] += narrow; s.acc[A_CON] += ncon; s.acc[A_EFC] += nefc; }
 
       WPE_CK_RESET();
@@ -1237,7 +1271,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
         __syncwarp();
       }
       WPE_PH(PH_ROWS);
-      if (LOCK) wpe::team_sync(team, tthreads);
+      if (LOCK) wpe::team_sync(t.team[wib], 32 * t.wpt);
       WPE_PH(PH_SOLVE);
       if (!finished) {
       WPE_CK_RESET();
