@@ -13,8 +13,8 @@ from pathlib import Path
 
 CSRC = Path(__file__).resolve().parent / "csrc"
 LIB = CSRC / "libhsrb.so"
-TUS = ["hsrb_api.cu", "hsrb_push.cu", "hsrb_wpe.cu", "hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu"]
-HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "../../include/hsrb.h"]
+TUS = ["hsrb_api.cu", "hsrb_push.cu", "hsrb_wpe.cu", "hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu", "hsrb_episode.cu"]
+HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "hsrb_episode.cuh", "../../include/hsrb.h"]
 # per-TU flags: the fast-path kernel uses the 2-ulp fp32 division / square root (MUFU.RCP / MUFU.RSQ sequences without
 # the IEEE fix-up path; measured +6 % substeps/s, one-step error vs the fp64 oracle unchanged at the 1e-7 level); the
 # general kernel and the reset / forward paths keep IEEE division.
@@ -24,6 +24,8 @@ TU_FLAGS["hsrb_wpe.cu"] = ([] if os.environ.get("HSRB_PRECISE_DIV") else ["--pre
     + os.environ.get("NVCC_WPE_EXTRA", "").split()
 for _g in (4, 8, 16, 32):
     TU_FLAGS[f"hsrb_step_g{_g}.cu"] = os.environ.get("NVCC_STEP_EXTRA", "").split()
+# the episode kernel resets environments with the stages of the lean reset instance above: same (IEEE) flags, same bits
+TU_FLAGS["hsrb_episode.cu"] = TU_FLAGS["hsrb_step_g8.cu"]
 # the phase-locked general kernel takes the same 2-ulp fp32 division / square root as the block-push kernels
 TU_FLAGS["hsrb_step_lock.cu"] = ([] if os.environ.get("HSRB_PRECISE_DIV") else ["--prec-div=false", "--prec-sqrt=false"]) \
     + os.environ.get("NVCC_STEP_EXTRA", "").split()

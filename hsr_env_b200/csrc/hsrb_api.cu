@@ -19,6 +19,7 @@
 
 #include "../../include/hsrb.h"
 #include "hsrb_wpe.cuh"
+#include "hsrb_episode.cuh"
 
 cudaError_t hsrb_push_prepare(int G, int nv, size_t smem, int threads, int* bps);
 cudaError_t hsrb_push_launch(int G, int nv, const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s);
@@ -88,6 +89,15 @@ struct hsrb {
   void* d_sort_tmp = nullptr;
   size_t sort_tmp_bytes = 0;
   bool order_valid = false;
+  // episode loop (hsrb_step_episode), allocated on first use: ages and sums of the running episodes, cumulative counters,
+  // and stand-ins for the step outputs the caller does not want
+  int *d_age = nullptr, *d_ep_sub = nullptr;
+  float* d_ep_ret = nullptr;
+  unsigned long long* d_ep_counters = nullptr;
+  unsigned char *d_ep_term = nullptr, *d_ep_bad = nullptr;
+  float* d_ep_reward = nullptr;
+  int* d_ep_taken = nullptr;
+  int ep_lanes = 0;   // layout the episode kernel was prepared for
 };
 
 namespace {
@@ -350,6 +360,48 @@ int run(hsrb* h, KArgs& a, void* stream) {
   return 0;
 }
 
+// episode buffers, zeroed on the caller's stream
+int episode_alloc(hsrb* h, void* stream) {
+  if (h->d_age) return 0;
+  const size_t n = (size_t)h->n;
+  cudaStream_t s = (cudaStream_t)stream;
+  CU(cudaMalloc(&h->d_age, sizeof(int) * n)); CU(cudaMalloc(&h->d_ep_sub, sizeof(int) * n)); CU(cudaMalloc(&h->d_ep_ret, sizeof(float) * n));
+  CU(cudaMalloc(&h->d_ep_counters, sizeof(unsigned long long) * EP_COUNT));
+  CU(cudaMalloc(&h->d_ep_term, n)); CU(cudaMalloc(&h->d_ep_bad, n));
+  CU(cudaMalloc(&h->d_ep_reward, sizeof(float) * n)); CU(cudaMalloc(&h->d_ep_taken, sizeof(int) * n));
+  CU(cudaMemsetAsync(h->d_age, 0, sizeof(int) * n, s)); CU(cudaMemsetAsync(h->d_ep_sub, 0, sizeof(int) * n, s));
+  CU(cudaMemsetAsync(h->d_ep_ret, 0, sizeof(float) * n, s));
+  CU(cudaMemsetAsync(h->d_ep_counters, 0, sizeof(unsigned long long) * EP_COUNT, s));
+  return 0;
+}
+
+// the episode kernel on the outputs of the step before it, in the lean launch layout of the general path
+int run_episode(hsrb* h, int max_steps, int autoreset, const unsigned char* term, const float* reward, const int* taken,
+                const unsigned char* bad, float* obs, unsigned char* truncated, float* final_obs, int* ep_length, float* ep_return,
+                int* ep_substeps, void* stream) {
+  int rc = episode_alloc(h, stream);
+  if (rc) return rc;
+  rc = configure(h);
+  if (rc) return rc;
+  if (h->ep_lanes != h->lanes) {
+    CU(hsrb_episode_prepare(h->lanes));
+    h->ep_lanes = h->lanes;
+  }
+  EpArgs e;
+  memset(&e, 0, sizeof(e));
+  e.k = base_args(h);
+  e.k.ws_bytes = h->ws_bytes;
+  e.k.obs = obs;
+  e.max_steps = max_steps; e.autoreset = autoreset;
+  e.terminated = term; e.reward = reward; e.taken = taken; e.bad = bad;
+  e.age = h->d_age; e.ret = h->d_ep_ret; e.sub = h->d_ep_sub;
+  e.truncated = truncated; e.final_obs = final_obs; e.ep_length = ep_length; e.ep_return = ep_return; e.ep_substeps = ep_substeps;
+  e.counters = h->d_ep_counters;
+  CU(hsrb_episode_launch(h->lanes, e, h->grid, (size_t)h->ws_bytes * (32 / h->lanes), (cudaStream_t)stream));
+  h->launches++;
+  return 0;
+}
+
 // FP32 FMA-loop peak of the device (the denominator of bench.py's FP32 roofline): 8 independent chains per thread
 __global__ void __launch_bounds__(1024) fma_peak_kernel(float* out, int iters, float a, float b) {
   float x0 = threadIdx.x, x1 = x0 + 1, x2 = x0 + 2, x3 = x0 + 3, x4 = x0 + 4, x5 = x0 + 5, x6 = x0 + 6, x7 = x0 + 7;
@@ -581,6 +633,8 @@ int hsrb_destroy(hsrb_t* h) {
   cudaFree(h->d_fast_tab); cudaFree(h->d_model); cudaFree(h->d_state); cudaFree(h->d_episode); cudaFree(h->d_stats);
   cudaFree(h->d_work); cudaFree(h->d_work_sorted); cudaFree(h->d_iota); cudaFree(h->d_order); cudaFree(h->d_sort_tmp);
   cudaFree(h->d_ctrl); cudaFree(h->d_obs); cudaFree(h->d_reward); cudaFree(h->d_done); cudaFree(h->d_taken);
+  cudaFree(h->d_age); cudaFree(h->d_ep_sub); cudaFree(h->d_ep_ret); cudaFree(h->d_ep_counters);
+  cudaFree(h->d_ep_term); cudaFree(h->d_ep_bad); cudaFree(h->d_ep_reward); cudaFree(h->d_ep_taken);
   delete h;
   return 0;
 }
@@ -681,7 +735,10 @@ int hsrb_reset(hsrb_t* h, const uint8_t* mask, float* obs, void* stream) {
   CU(cudaSetDevice(h->device));
   KArgs a = base_args(h);
   a.mode = MODE_RESET; a.mask = mask; a.obs = obs; a.nsub = 0;
-  return run(h, a, stream);
+  const int rc = run(h, a, stream);
+  if (rc || !h->d_age) return rc;
+  CU(hsrb_episode_clear(mask, h->n, h->d_age, h->d_ep_ret, h->d_ep_sub, (cudaStream_t)stream));
+  return 0;
 }
 
 int hsrb_step(hsrb_t* h, const float* ctrl, int nsubsteps, float* obs, float* reward, uint8_t* done, uint8_t* success,
@@ -694,6 +751,72 @@ int hsrb_step(hsrb_t* h, const float* ctrl, int nsubsteps, float* obs, float* re
   a.mode = MODE_STEP; a.ctrl = ctrl; a.nsub = nsubsteps; a.obs = obs; a.reward = reward; a.done = done;
   a.success = success; a.taken = substeps_taken; a.bad = bad_state;
   return run(h, a, stream);
+}
+
+int hsrb_step_episode(hsrb_t* h, const float* ctrl, int nsubsteps, int max_episode_steps, int autoreset, float* obs, float* reward,
+                      uint8_t* terminated, uint8_t* truncated, float* final_obs, int32_t* ep_length, float* ep_return,
+                      int32_t* ep_substeps, int32_t* substeps_taken, uint8_t* bad_state, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  if (max_episode_steps < 0) return fail(-1, "max_episode_steps < 0");
+  CU(cudaSetDevice(h->device));
+  int rc = episode_alloc(h, stream);
+  if (rc) return rc;
+  // what the episode kernel reads goes to the handle's buffers when the caller does not want it
+  uint8_t* term = terminated ? terminated : h->d_ep_term;
+  float* rew = reward ? reward : h->d_ep_reward;
+  int32_t* taken = substeps_taken ? substeps_taken : h->d_ep_taken;
+  uint8_t* bad = bad_state ? bad_state : h->d_ep_bad;
+  rc = hsrb_step(h, ctrl, nsubsteps, obs, rew, term, nullptr, taken, bad, stream);
+  if (rc) return rc;
+  return run_episode(h, max_episode_steps, autoreset, term, rew, taken, bad, obs, truncated, final_obs, ep_length, ep_return,
+                     ep_substeps, stream);
+}
+
+int hsrb_episode_update(hsrb_t* h, int max_episode_steps, int autoreset, const uint8_t* terminated, const float* reward,
+                        const int32_t* substeps_taken, const uint8_t* bad_state, float* obs, uint8_t* truncated, float* final_obs,
+                        int32_t* ep_length, float* ep_return, int32_t* ep_substeps, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  if (!terminated) return fail(-1, "terminated is NULL");
+  if (max_episode_steps < 0) return fail(-1, "max_episode_steps < 0");
+  CU(cudaSetDevice(h->device));
+  return run_episode(h, max_episode_steps, autoreset, terminated, reward, substeps_taken, bad_state, obs, truncated, final_obs,
+                     ep_length, ep_return, ep_substeps, stream);
+}
+
+int hsrb_set_episode_ages(hsrb_t* h, const int32_t* age, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  CU(cudaSetDevice(h->device));
+  int rc = episode_alloc(h, stream);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t n = (size_t)h->n;
+  if (age) CU(cudaMemcpyAsync(h->d_age, age, sizeof(int) * n, cudaMemcpyDeviceToDevice, s));
+  else CU(cudaMemsetAsync(h->d_age, 0, sizeof(int) * n, s));
+  CU(cudaMemsetAsync(h->d_ep_ret, 0, sizeof(float) * n, s));
+  CU(cudaMemsetAsync(h->d_ep_sub, 0, sizeof(int) * n, s));
+  return 0;
+}
+
+int hsrb_get_episode_ages(hsrb_t* h, int32_t* age, void* stream) {
+  if (!h || !age) return fail(-1, "bad arguments");
+  CU(cudaSetDevice(h->device));
+  int rc = episode_alloc(h, stream);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(age, h->d_age, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int hsrb_episode_stats(hsrb_t* h, int64_t* out8, void* stream) {
+  static_assert(EP_COUNT == 8, "hsrb.h documents 8 counters");
+  if (!h || !out8) return fail(-1, "bad arguments");
+  CU(cudaSetDevice(h->device));
+  int rc = episode_alloc(h, stream);
+  if (rc) return rc;
+  unsigned long long v[EP_COUNT];
+  CU(cudaMemcpyAsync(v, h->d_ep_counters, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  CU(cudaStreamSynchronize((cudaStream_t)stream));
+  for (int i = 0; i < EP_COUNT; i++) out8[i] = (int64_t)v[i];
+  return 0;
 }
 
 int hsrb_step_host(hsrb_t* h, const float* ctrl_host, int nsubsteps, float* obs_host, float* reward_host,

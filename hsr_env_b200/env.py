@@ -86,6 +86,8 @@ class BatchedHSREnv:
             block_quat_index: Sequence[int] = (0, 2),
             lanes_per_env: int = 0,
             kernel: str = "auto",
+            max_episode_steps: Optional[int] = None,
+            autoreset: bool = False,
     ):
         if any([render, record, render_freq, record_freq, record_path]):
             raise NotImplementedError("render/record need an OpenGL viewer and are outside the batched backend "
@@ -131,6 +133,13 @@ class BatchedHSREnv:
         self._qidx = tuple(int(i) for i in block_quat_index)
         self._time_steps = 0
         self._geofence = 0.0
+        # episode loop on the device (hsrb_step_episode): TimeLimit(max_episode_steps), hsr/__init__.py:22, and the
+        # caller's `if done: env.reset()`, hsr/control.py:73-75
+        if max_episode_steps is not None and int(max_episode_steps) < 0:
+            raise ValueError("max_episode_steps must be >= 0 (0 or None: no time limit)")
+        self.max_episode_steps = int(max_episode_steps or 0)
+        self.autoreset = bool(autoreset)
+        self._episodes = self.max_episode_steps > 0 or self.autoreset
         self._parse_goal_specs()
         self._push_starts()
 
@@ -280,9 +289,14 @@ class BatchedHSREnv:
         return self._observation(obs)
 
     def step(self, action: torch.Tensor, steps: Optional[int] = None):
-        """HSREnv.step (hsr/env.py:115-135) for every environment: one kernel launch."""
+        """HSREnv.step (hsr/env.py:115-135) for every environment: one kernel launch.  With ``max_episode_steps`` or
+        ``autoreset`` (the episode loop on the device, hsrb_step_episode): done = terminated | truncated, and info adds
+        ``terminated``, ``truncated``, ``final_observation`` (the step's observation before any auto-reset) and
+        ``episode`` = {"l", "r", "substeps"} (length in actions, summed reward and substeps; valid where done)."""
         steps = steps or self.steps_per_action
         action = torch.as_tensor(action, dtype=torch.float32, device=self.device).reshape(self.n_envs, self.nu).contiguous()
+        if self._episodes:
+            return self._step_episode(action, steps)
         obs = self._empty(self.n_envs, self.state_dim)
         reward = self._empty(self.n_envs)
         done = self._empty(self.n_envs, dtype=torch.uint8)
@@ -296,11 +310,73 @@ class BatchedHSREnv:
         info = {"log count": {"success": done_b}, "substeps_taken": taken, "bad_state": bad}
         return self._observation(obs), reward, done_b, info
 
+    def _step_episode(self, action: torch.Tensor, steps: int):
+        """step() with max_episode_steps / autoreset: the action kernel, then the episode kernel (hsrb_step_episode)."""
+        n = self.n_envs
+        reward = self._empty(n)
+        term = self._empty(n, dtype=torch.uint8)
+        trunc = self._empty(n, dtype=torch.uint8)
+        taken = self._empty(n, dtype=torch.int32)
+        bad = self._empty(n, dtype=torch.uint8)
+        # where not done the episode outputs are left as they are: zero, not garbage
+        ep_l = torch.zeros(n, dtype=torch.int32, device=self.device)
+        ep_r = torch.zeros(n, device=self.device)
+        ep_s = torch.zeros(n, dtype=torch.int32, device=self.device)
+        P = _lib.ptr
+        with torch.cuda.device(self.device):
+            if self._obs_type == "openai":
+                # the 25-d observation of the stepped state before the reset, and of the reset state after it
+                _lib.check(self._lib.hsrb_step(self._h, P(action), int(steps), None, P(reward), P(term), None, P(taken), P(bad),
+                                               self._stream()))
+                final = self._observation(None)
+                _lib.check(self._lib.hsrb_episode_update(self._h, self.max_episode_steps, int(self.autoreset), P(term), P(reward),
+                                                         P(taken), P(bad), None, P(trunc), None, P(ep_l), P(ep_r), P(ep_s),
+                                                         self._stream()))
+                obs = self._observation(None)
+            else:
+                obs = self._empty(n, self.state_dim)
+                final = self._empty(n, self.state_dim)
+                _lib.check(self._lib.hsrb_step_episode(self._h, P(action), int(steps), self.max_episode_steps, int(self.autoreset),
+                                                       P(obs), P(reward), P(term), P(trunc), P(final), P(ep_l), P(ep_r), P(ep_s),
+                                                       P(taken), P(bad), self._stream()))
+        self._time_steps += 1
+        term_b, trunc_b = term.bool(), trunc.bool()
+        info = {"log count": {"success": term_b}, "substeps_taken": taken, "bad_state": bad, "terminated": term_b,
+                "truncated": trunc_b, "final_observation": final, "episode": {"l": ep_l, "r": ep_r, "substeps": ep_s}}
+        return obs, reward, term_b | trunc_b, info
+
+    # ------------------------------------------------------------------ episode ages and counters
+    def set_episode_ages(self, ages=None):
+        """TimeLimit._elapsed_steps of every environment (None: zeros); the sums of the running episodes restart at 0."""
+        a = None if ages is None else torch.as_tensor(ages, dtype=torch.int32, device=self.device).reshape(self.n_envs).contiguous()
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_set_episode_ages(self._h, _lib.ptr(a), self._stream()))
+            torch.cuda.current_stream(self.device).synchronize()  # the input may be a temporary
+
+    def episode_ages(self) -> torch.Tensor:
+        """Actions since each environment's last reset: int32 [N]."""
+        out = self._empty(self.n_envs, dtype=torch.int32)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_get_episode_ages(self._h, _lib.ptr(out), self._stream()))
+        return out
+
+    def episode_stats(self) -> dict:
+        """Cumulative counters of the episode kernel: the keys of dist.EPISODE_STAT_KEYS (``substeps``: summed substeps of
+        the finished episodes, ``bad_states``: steps with a non-zero bad_state) plus ``truncations``, ``length`` (summed
+        episode length in actions), ``resets`` (auto-resets) and ``actions`` (environment actions stepped)."""
+        v = (ctypes.c_int64 * 8)()
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_episode_stats(self._h, v, self._stream()))
+        keys = ["episodes", "successes", "truncations", "length", "substeps", "bad_states", "resets", "actions"]
+        return dict(zip(keys, [int(x) for x in v]))
+
     def step_host(self, action, steps: Optional[int] = None, out=None):
         """Same call with HOST buffers (numpy / pinned torch CPU tensors), copies inside: the end-to-end path.  Runs on
         torch's current stream, i.e. after any reset / set_state / step issued before it."""
         if self._obs_type == "openai":
             raise NotImplementedError("step_host returns the kernel's qpos|qvel observation; use step() for obs_type='openai'")
+        if self._episodes:
+            raise NotImplementedError("step_host has no episode loop; use step() with max_episode_steps / autoreset")
         steps = steps or self.steps_per_action
         if isinstance(action, torch.Tensor):
             if action.dtype != torch.float32 or not action.is_contiguous() or action.numel() != self.n_envs * self.nu or action.is_cuda:
@@ -324,7 +400,7 @@ class BatchedHSREnv:
         self._time_steps += 1
         return out
 
-    def _observation(self, state: torch.Tensor) -> torch.Tensor:
+    def _observation(self, state: Optional[torch.Tensor]) -> torch.Tensor:
         """HSREnv._get_observation (hsr/env.py:71-113): the kernel's qpos|qvel, or the 25-d 'openai' observation built
         from it on the device (hsr_env_b200/kin.py states the intent of the reference's dead branch)."""
         if self._obs_type != "openai":
@@ -444,9 +520,14 @@ class BatchedHSREnv:
 class HSREnv(BatchedHSREnv):
     """Single-environment facade: numpy in / numpy out, scalars for reward and done, like the reference."""
 
-    def __init__(self, xml_file, goals, starts=None, steps_per_action: int = 300, **kw):
+    def __init__(self, xml_file, goals, starts=None, steps_per_action: int = 300, max_episode_steps: Optional[int] = None, **kw):
+        """``max_episode_steps``: gym.wrappers.TimeLimit (hsr/__init__.py:22): done at the limit, with
+        ``info["TimeLimit.truncated"]``.  No auto-reset: the caller's loop resets, as hsr/control.py:73-75 does."""
         kw.setdefault("n_envs", 1)
         assert kw["n_envs"] == 1
+        if kw.get("autoreset"):
+            raise ValueError("HSREnv does not auto-reset: reset() when done, as hsr/control.py:73-75 does")
+        kw["max_episode_steps"] = max_episode_steps
         super().__init__(xml_file, goals, starts, steps_per_action, **kw)
         self.init_qpos = self.model.qpos0.copy()
         self.init_qvel = np.zeros(self.nv)
@@ -456,10 +537,12 @@ class HSREnv(BatchedHSREnv):
 
     def step(self, action, steps=None):
         obs, reward, done, info = super().step(np.asarray(action, np.float32), steps)
-        success = bool(done[0].item())
-        info = {"log count": {"success": success and self._time_steps > 0}, "substeps_taken": int(info["substeps_taken"][0]),
-                "bad_state": int(info["bad_state"][0])}
-        return obs[0].double().cpu().numpy(), float(reward[0].item()), success, info
+        success = bool(info["terminated"][0].item()) if self._episodes else bool(done[0].item())
+        out = {"log count": {"success": success and self._time_steps > 0}, "substeps_taken": int(info["substeps_taken"][0]),
+               "bad_state": int(info["bad_state"][0])}
+        if self.max_episode_steps and bool(done[0].item()) and int(info["episode"]["l"][0].item()) >= self.max_episode_steps:
+            out["TimeLimit.truncated"] = not success   # what gym.wrappers.TimeLimit.step sets at the limit
+        return obs[0].double().cpu().numpy(), float(reward[0].item()), bool(done[0].item()), out
 
     def block_pos(self):
         return super().block_pos()[0, 0].double().cpu().numpy()

@@ -27,7 +27,12 @@ SIGNATURES = {
     "hsrb_set_starts": (c_int, [c_void_p, c_int, POINTER(c_int32), POINTER(c_int32), POINTER(c_float), POINTER(c_float)]),
     "hsrb_reset": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_step": (c_int, [c_void_p, c_void_p, c_int] + [c_void_p] * 7),
-    "hsrb_step_host": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hsrb_step_episode": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int] + [c_void_p] * 11),
+    "hsrb_episode_update": (c_int, [c_void_p, c_int, c_int] + [c_void_p] * 11),
+    "hsrb_set_episode_ages": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "hsrb_get_episode_ages": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "hsrb_episode_stats": (c_int, [c_void_p, POINTER(c_int64), c_void_p]),
+    "hsrb_step_host":(c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_get_state": (c_int, [c_void_p] + [c_void_p] * 5),
     "hsrb_set_state": (c_int, [c_void_p] + [c_void_p] * 5),
     "hsrb_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),

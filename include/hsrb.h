@@ -78,6 +78,42 @@ int hsrb_reset(hsrb_t* h, const uint8_t* mask, float* obs, void* stream);
 int hsrb_step(hsrb_t* h, const float* ctrl, int nsubsteps, float* obs, float* reward, uint8_t* done, uint8_t* success,
               int32_t* substeps_taken, uint8_t* bad_state, void* stream);
 
+/* gym.wrappers.TimeLimit(max_episode_steps) + the caller's `if done: env.reset()`   hsr/__init__.py:22, control.py:73-75
+ * The action kernel exactly as hsrb_step runs it, then one episode kernel.  Each environment has an episode age: the
+ * actions since its last reset (hsrb_reset or auto-reset set it to 0, a step adds 1).  terminated = success (hsrb_step's
+ * done); truncated = age >= max_episode_steps && !terminated (max_episode_steps 0: no limit); done = terminated |
+ * truncated.  With autoreset != 0 every done environment is reset in the same call, after the step, with the Philox draw
+ * hsrb_reset(mask = done) would make (key = seed, global env id; counter = its episode, which goes up by one): obs then
+ * holds the new episode's first observation for those environments.  final_obs[N, nq+nv] holds, for every environment,
+ * the observation the step produced, before any reset.  reward, terminated, truncated, substeps_taken and bad_state
+ * describe the step taken.  Where done: ep_length[N] = the episode's length in actions, ep_return[N] = its summed reward,
+ * ep_substeps[N] = its summed substeps (int32); elsewhere they are left as they were.  Without autoreset nothing is reset:
+ * the caller resets (hsrb_reset) the environments it sees done, until then they report done again on every step.  Any
+ * output may be NULL.  The ages, the sums of the running episodes and the counters of hsrb_episode_stats are allocated
+ * (zero) on the first call of any hsrb_*episode* function; from then on hsrb_reset zeroes the ages and sums of the
+ * environments it resets. */
+int hsrb_step_episode(hsrb_t* h, const float* ctrl, int nsubsteps, int max_episode_steps, int autoreset, float* obs, float* reward,
+                      uint8_t* terminated, uint8_t* truncated, float* final_obs, int32_t* ep_length, float* ep_return,
+                      int32_t* ep_substeps, int32_t* substeps_taken, uint8_t* bad_state, void* stream);
+
+/* The episode kernel of hsrb_step_episode alone, on the outputs of the hsrb_step before it (terminated = its done,
+ * required; reward / substeps_taken / bad_state NULL = 0): lets the caller compute an observation of its own (e.g. the
+ * 'openai' one, hsrb_openai_obs) of the stepped state before the reset and of the reset state after it.  obs (nullable)
+ * receives the new observation of the environments it resets; the other outputs are those of hsrb_step_episode. */
+int hsrb_episode_update(hsrb_t* h, int max_episode_steps, int autoreset, const uint8_t* terminated, const float* reward,
+                        const int32_t* substeps_taken, const uint8_t* bad_state, float* obs, uint8_t* truncated, float* final_obs,
+                        int32_t* ep_length, float* ep_return, int32_t* ep_substeps, void* stream);
+
+/* TimeLimit._elapsed_steps of every environment (hsr/__init__.py:22): age[N] int32 device arrays.  set (NULL = zeros)
+ * also restarts the summed reward / substeps of the running episodes at 0: checkpoints, or staggered episode phases. */
+int hsrb_set_episode_ages(hsrb_t* h, const int32_t* age, void* stream);
+int hsrb_get_episode_ages(hsrb_t* h, int32_t* age, void* stream);
+
+/* Cumulative counters of the episode kernel, copied to host (synchronises `stream`): [0] episodes finished (done),
+ * [1] of them terminated (success), [2] truncated, [3] summed episode length in actions, [4] summed substeps of the
+ * finished episodes, [5] steps with a non-zero bad_state, [6] auto-resets, [7] environment actions stepped. */
+int hsrb_episode_stats(hsrb_t* h, int64_t* out8_host, void* stream);
+
 /* Same call with HOST buffers (the way the reference's caller holds its numpy arrays, hsr/control.py:48-63):
  * copies ctrl host->device, steps, copies obs/reward/done/substeps device->host, all enqueued on `stream` - the
  * CALLER's stream, so the step is ordered after whatever the caller launched there before (hsrb_reset,

@@ -22,6 +22,19 @@ if [ "${1:-}" == cap4 ]; then
   echo "== asan cap4"; grep -cE "ERROR: AddressSanitizer|runtime error" $LOG; tail -n 6 $LOG
   exit 0
 fi
+# tools/emu_sanitize.sh episode: ASan + UBSan, the episode kernel (hsrb_episode.cuh: TimeLimit + auto-reset) through
+# tests/test_episode_emu.py -> profiles/r04_emu_asan_episode.log
+if [ "${1:-}" == episode ]; then
+  SAN="-fsanitize=address,undefined -fno-omit-frame-pointer"; PRE=$(gcc -print-file-name=libasan.so)
+  g++ -O1 -g -std=c++17 -fPIC -shared -ffp-contract=off $SAN -D__CUDACC__ -DHSRB_SIMT_EMU -include tests/simt_emu/simt_emu.h \
+      -I tests/simt_emu -o /tmp/libepisode_emu_asan.so tests/simt_emu/emu_episode.cpp -lpthread || exit 1
+  LOG=$OUT/r04_emu_asan_episode.log
+  ASAN_OPTIONS=detect_leaks=0:halt_on_error=0 LD_PRELOAD=$PRE EMU_EPISODE_LIB=/tmp/libepisode_emu_asan.so \
+  timeout 3000 python -m pytest tests/test_episode_emu.py -q -p no:cacheprovider > $LOG 2>&1
+  echo "exit $?" >> $LOG
+  echo "== asan episode"; grep -cE "ERROR: AddressSanitizer|runtime error" $LOG; tail -n 6 $LOG
+  exit 0
+fi
 for MODE in asan tsan; do
   if [ $MODE == asan ]; then SAN="-fsanitize=address,undefined -fno-omit-frame-pointer"; PRE=$(gcc -print-file-name=libasan.so); else SAN="-fsanitize=thread"; PRE=$(gcc -print-file-name=libtsan.so); fi
   LIB=/tmp/libpush_emu_$MODE.so
