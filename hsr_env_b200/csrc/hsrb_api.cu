@@ -21,11 +21,6 @@
 #include "hsrb_wpe.cuh"
 #include "hsrb_episode.cuh"
 
-cudaError_t hsrb_push_prepare(int G, int nv, size_t smem, int threads, int* bps);
-cudaError_t hsrb_push_launch(int G, int nv, const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s);
-cudaError_t hsrb_wpe_prepare(size_t smem, int threads, int* bps);
-cudaError_t hsrb_wpe_launch(const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s, bool lock);
-
 namespace {
 
 thread_local char g_err[512] = "";
@@ -44,6 +39,89 @@ int fail(int code, const char* fmt, ...) {
     if (e_ != cudaSuccess) return fail(-2, "%s: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
 
+// Experiment switches (INTEGRATION.md), read from the environment once, when the handle is created
+struct Knobs {
+  unsigned opts = 0;          // HSRB_OPTS: KArgs::opts
+  bool wpe_lock = true;       // HSRB_WPE_LOCK=0: free-running warps instead of the phase-locked wpe kernel
+  unsigned wpe_teams = 2;     // HSRB_WPE_TEAMS=1|2|4: teams per block of the phase-locked wpe kernel
+  bool wpe_sort = true;       // HSRB_WPE_SORT=0: identity launch order of the wpe kernel instead of the work-sorted one
+  int wpe_wpb = 0;            // HSRB_WPE_WPB: warps per block of the wpe kernel (0: derived from the batch size)
+  bool general_lock = true;   // HSRB_GENERAL_LOCK=0: one-warp-per-block general kernel for STEP launches
+};
+
+Knobs read_knobs() {
+  Knobs k;
+  const auto off = [](const char* name) { const char* v = getenv(name); return v && v[0] == '0'; };
+  if (const char* o = getenv("HSRB_OPTS")) k.opts = (unsigned)strtoul(o, nullptr, 0);
+  k.wpe_lock = !off("HSRB_WPE_LOCK");
+  if (const char* t = getenv("HSRB_WPE_TEAMS")) k.wpe_teams = (unsigned)atoi(t);
+  k.wpe_sort = !off("HSRB_WPE_SORT");
+  if (const char* w = getenv("HSRB_WPE_WPB")) k.wpe_wpb = atoi(w);
+  k.general_lock = !off("HSRB_GENERAL_LOCK");
+  return k;
+}
+
+__global__ void fill_iota(int* p, int n) { const int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = i; }
+
+// Work-sorted launch order of the warp-per-environment kernel (hsrb_wpe_kernel_t): the kernel writes a work estimate per
+// environment, a radix sort (cub, descending, stable: ties keep the environment order) turns it into the order of the next
+// launch (slot r -> block r % grid, warp r / grid: the heaviest warps of every block form team 0).  Results do not depend
+// on it.
+struct SortBufs {
+  int *work = nullptr, *work_sorted = nullptr, *iota = nullptr, *order = nullptr;
+  void* tmp = nullptr;
+  size_t tmp_bytes = 0;
+  bool valid = false;   // order holds the order of the previous launch
+  int alloc(int n, cudaStream_t s) {
+    if (work) return 0;
+    const size_t nb = sizeof(int) * (size_t)n;
+    CU(cudaMalloc(&work, nb)); CU(cudaMalloc(&work_sorted, nb)); CU(cudaMalloc(&iota, nb)); CU(cudaMalloc(&order, nb));
+    CU(cudaMemsetAsync(work, 0, nb, s));
+    fill_iota<<<(n + 255) / 256, 256, 0, s>>>(iota, n);
+    CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, work, work_sorted, iota, order, n, 0, 24, s));
+    CU(cudaMalloc(&tmp, tmp_bytes));
+    return 0;
+  }
+  int update(int n, cudaStream_t s) {   // the next launch's order
+    CU(cub::DeviceRadixSort::SortPairsDescending(tmp, tmp_bytes, work, work_sorted, iota, order, n, 0, 24, s));
+    valid = true;
+    return 0;
+  }
+  void free() { cudaFree(work); cudaFree(work_sorted); cudaFree(iota); cudaFree(order); cudaFree(tmp); }
+};
+
+// Episode loop (hsrb_step_episode), allocated on first use: ages and sums of the running episodes, cumulative counters,
+// and stand-ins for the step outputs the caller does not want
+struct EpisodeBufs {
+  int *age = nullptr, *sub = nullptr;
+  float* ret = nullptr;
+  unsigned long long* counters = nullptr;
+  unsigned char *term = nullptr, *bad = nullptr;
+  float* reward = nullptr;
+  int* taken = nullptr;
+  int lanes = 0;   // layout the episode kernel was prepared for
+  int alloc(int n_envs, cudaStream_t s) {   // zeroed on the caller's stream
+    if (age) return 0;
+    const size_t n = (size_t)n_envs;
+    CU(cudaMalloc(&age, sizeof(int) * n)); CU(cudaMalloc(&sub, sizeof(int) * n)); CU(cudaMalloc(&ret, sizeof(float) * n));
+    CU(cudaMalloc(&counters, sizeof(unsigned long long) * EP_COUNT));
+    CU(cudaMalloc(&term, n)); CU(cudaMalloc(&bad, n));
+    CU(cudaMalloc(&reward, sizeof(float) * n)); CU(cudaMalloc(&taken, sizeof(int) * n));
+    CU(cudaMemsetAsync(age, 0, sizeof(int) * n, s)); CU(cudaMemsetAsync(sub, 0, sizeof(int) * n, s));
+    CU(cudaMemsetAsync(ret, 0, sizeof(float) * n, s));
+    CU(cudaMemsetAsync(counters, 0, sizeof(unsigned long long) * EP_COUNT, s));
+    return 0;
+  }
+  void free() {
+    cudaFree(age); cudaFree(sub); cudaFree(ret); cudaFree(counters); cudaFree(term); cudaFree(bad); cudaFree(reward); cudaFree(taken);
+  }
+};
+
+// The action kernels.  K_GENERAL (hsrb_step_kernel<G>) also runs every reset, forward and debug launch; the others
+// run STEP launches only.  A new kernel is one more entry here, its configure_* function and one line in select().
+enum Kernel { K_GENERAL, K_LOCK, K_PUSH, K_WPE, K_COUNT };
+const int kPathCode[K_COUNT] = {1, 1, 2, 3};   // what hsrb_set_path and hsrb_launch_info report
+
 }  // namespace
 
 struct hsrb {
@@ -51,136 +129,124 @@ struct hsrb {
   ModelT<float> dm;         // same table with device pointers
   unsigned char* d_model = nullptr;
   EnvCfg<float> cfg;
-  int n = 0, device = 0, S = 0;
+  int n = 0, device = 0, S = 0, num_sm = 0;
   unsigned long long seed = 0, env_off = 0;
   float* d_state = nullptr;
   unsigned* d_episode = nullptr;
   unsigned long long* d_stats = nullptr;
-  // launch configuration
-  int lanes = 0, lanes_req = 0;
-  unsigned ws_bytes = 0;
-  int blocks_per_sm = 0, grid = 0, num_sm = 0;
-  bool configured = false;
+  long long launches = 0;
+  Knobs knobs;
+  int lanes_req = 0;        // hsrb_config's lanes per environment (0: the plan's choice)
+  int path = 0;             // hsrb_set_path
+  Plan plan[K_COUNT];       // launch configuration per kernel, worked out on first use
+  // sliding base + at most one free box (hsrb_push.cuh, hsrb_wpe.cuh)
+  PushInfo fast;
+  PushTables fast_tab;
+  unsigned char* d_fast_tab = nullptr;
+  bool fast_ok = false, wpe_ok = false;
+  char fast_why[128] = "";
+  SortBufs sort;
+  EpisodeBufs ep;
   // scratch for the host-buffer entry point
   float *d_ctrl = nullptr, *d_obs = nullptr, *d_reward = nullptr;
   unsigned char* d_done = nullptr;
   int* d_taken = nullptr;
-  long long launches = 0;
-  // fast path (hsrb_push.cuh): sliding base + at most one free box
-  PushInfo fast;
-  PushTables fast_tab;
-  unsigned char* d_fast_tab = nullptr;
-  bool fast_ok = false;
-  int path = 0;             // 0 auto, 1 general kernel, 2 fast kernel
-  bool fast_configured = false;
-  int fast_lanes = 8, fast_threads = 0, fast_grid = 0, fast_bps = 0;
-  unsigned fast_ws = 0;
-  char fast_why[128] = "";
-  // phase-locked general kernel (hsrb_step_lock_kernel): STEP launches of the general path
-  bool lock_configured = false;
-  int lock_threads = 0, lock_grid = 0, lock_bps = 0;
-  // warp-per-environment kernel of the same family (hsrb_wpe.cuh)
-  bool wpe_ok = false, wpe_configured = false;
-  int wpe_threads = 0, wpe_grid = 0, wpe_bps = 0;
-  unsigned wpe_ws = 0;
-  // work-sorted launch order of the wpe kernel: the kernel writes a work estimate per environment, the next launch takes
-  // the environments heaviest first (slot r -> block r % grid, warp r / grid: the heaviest warps of every block form team 0)
-  int *d_work = nullptr, *d_work_sorted = nullptr, *d_iota = nullptr, *d_order = nullptr;
-  void* d_sort_tmp = nullptr;
-  size_t sort_tmp_bytes = 0;
-  bool order_valid = false;
-  // episode loop (hsrb_step_episode), allocated on first use: ages and sums of the running episodes, cumulative counters,
-  // and stand-ins for the step outputs the caller does not want
-  int *d_age = nullptr, *d_ep_sub = nullptr;
-  float* d_ep_ret = nullptr;
-  unsigned long long* d_ep_counters = nullptr;
-  unsigned char *d_ep_term = nullptr, *d_ep_bad = nullptr;
-  float* d_ep_reward = nullptr;
-  int* d_ep_taken = nullptr;
-  int ep_lanes = 0;   // layout the episode kernel was prepared for
 };
 
 namespace {
 
-__global__ void fill_iota(int* p, int n) { const int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) p[i] = i; }
-
-cudaError_t prepare(int G, size_t smem, int* bps) {
-  switch (G) {
-    case 4: return hsrb_prepare_step_4(smem, bps);
-    case 8: return hsrb_prepare_step_8(smem, bps);
-    case 16: return hsrb_prepare_step_16(smem, bps);
-    default: return hsrb_prepare_step_32(smem, bps);
-  }
-}
-cudaError_t launch(int G, const KArgs& a, int grid, size_t smem, cudaStream_t s) {
-  switch (G) {
-    case 4: return hsrb_launch_step_4(a, grid, smem, s);
-    case 8: return hsrb_launch_step_8(a, grid, smem, s);
-    case 16: return hsrb_launch_step_16(a, grid, smem, s);
-    default: return hsrb_launch_step_32(a, grid, smem, s);
-  }
-}
-cudaError_t launch_aux(int G, const KArgs& a, int grid, size_t smem, cudaStream_t s) {
-  switch (G) {
-    case 4: return hsrb_launch_aux_4(a, grid, smem, s);
-    case 8: return hsrb_launch_aux_8(a, grid, smem, s);
-    case 16: return hsrb_launch_aux_16(a, grid, smem, s);
-    default: return hsrb_launch_aux_32(a, grid, smem, s);
-  }
+// The kernel a STEP launch of the handle runs.  The fast kernels take the sliding-base family in its env_wrapper goal form
+// only (one block against the goal point); among them, auto (path 0) and path 3 take the warp-per-environment kernel,
+// phase-locked, two teams per block - measured on B200, round 2, TimeLimit workload: 48.4 M substeps/s at 4096 envs
+// (lock-step 8-lane kernel 34.6 M, free-running warps 32.9 M), 65.8 M at 131072 envs (52.3 M / 53.2 M).  A goal list
+// under path 3 runs the general kernel; under path 2 it is an error.
+int select(const hsrb* h, Kernel* k) {
+  const bool fast = h->fast_ok && h->path != 1 && h->cfg.ngoal == 0;
+  if (fast && h->wpe_ok && h->path != 2) *k = K_WPE;
+  else if (fast) *k = K_PUSH;
+  else if (h->path == 2) return fail(-3, "fast path not available for this model: %s", h->fast_why);
+  else if (h->knobs.general_lock && h->hm.m.npair <= 256 && !h->lanes_req) *k = K_LOCK;
+  else *k = K_GENERAL;
+  return 0;
 }
 
 // Choose lanes-per-environment and the grid: as many lanes per env as keeps every environment resident in
 // one wave (more lanes = shorter dependent chain per substep), otherwise fewer lanes / a grid-stride loop.
-int configure(hsrb* h) {
-  if (h->configured) return 0;
-  h->ws_bytes = (unsigned)ws_carve<float>(h->dm, nullptr, nullptr);
+int configure_general(const hsrb* h, Plan& p) {
+  p.ws = (unsigned)ws_carve<float>(h->dm, nullptr, nullptr);
+  p.ncon_max = h->dm.ncon_max; p.nefc_max = h->dm.nefc_max;
+  p.threads = 32;
   // lanes per environment: the widest layout that holds every environment in one wave; if none does, shared memory
   // decides how many environments an SM holds (one warp per block, 32/G workspaces per block), and among the layouts
   // within 10 % of the best residency the narrowest one wins: the single-lane stages (kinematics, bias forces, Euler)
   // then run for 32/G environments at once.  Measured on B200 (tools/sweep_lanes.py): C3 (nv = 13, 16384 envs)
   // G = 8: 3.5 M substeps/s against 2.6 M (G = 4, one block per SM) and 1.1 M (G = 32); C5 (nv = 26): G = 32 0.53 M
   // against 0.29 M (G = 16)
-  int cands[4] = {32, 16, 8, 4};
-  int best = 0;
+  const struct { int G; cudaError_t (*prepare)(const Plan&, int*); cudaError_t (*launch)(const Plan&, const KArgs&, cudaStream_t); } cands[4] = {
+      {32, hsrb_step32_prepare, hsrb_step32_launch}, {16, hsrb_step16_prepare, hsrb_step16_launch},
+      {8, hsrb_step8_prepare, hsrb_step8_launch}, {4, hsrb_step4_prepare, hsrb_step4_launch}};
+  int best = -1;
   long long res[4] = {0, 0, 0, 0};
   int bpsv[4] = {0, 0, 0, 0};
   long long resmax = 0;
   for (int k = 0; k < 4; k++) {
-    int G = cands[k];
+    const int G = cands[k].G;
     if (h->lanes_req && G != h->lanes_req) continue;
-    size_t smem = (size_t)h->ws_bytes * (32 / G);
-    if (smem > 227 * 1024) continue;
+    p.smem = (size_t)p.ws * (32 / G);
+    if (p.smem > 227 * 1024) continue;
     int bps = 0;
-    if (prepare(G, smem, &bps) != cudaSuccess || bps <= 0) { cudaGetLastError(); continue; }
+    if (cands[k].prepare(p, &bps) != cudaSuccess || bps <= 0) { cudaGetLastError(); continue; }
     bpsv[k] = bps;
     res[k] = (long long)bps * h->num_sm * (32 / G);
     if (res[k] > resmax) resmax = res[k];
   }
-  for (int k = 0; k < 4 && !best; k++)
-    if (res[k] >= h->n) { best = cands[k]; h->blocks_per_sm = bpsv[k]; }
-  for (int k = 3; k >= 0 && !best; k--)
-    if (res[k] > 0 && res[k] * 10 >= resmax * 9) { best = cands[k]; h->blocks_per_sm = bpsv[k]; }
-  if (!best) return fail(-3, "no launch configuration fits: workspace %u bytes per environment", h->ws_bytes);
-  h->lanes = best;
-  size_t smem = (size_t)h->ws_bytes * (32 / best);
-  CU(prepare(best, smem, &h->blocks_per_sm));
-  int gpb = 32 / best;
-  int need = (h->n + gpb - 1) / gpb;
-  int cap = h->blocks_per_sm * h->num_sm;
-  h->grid = need < cap ? need : cap;
-  if (h->grid < 1) h->grid = 1;
-  h->configured = true;
+  for (int k = 0; k < 4 && best < 0; k++)
+    if (res[k] >= h->n) best = k;
+  for (int k = 3; k >= 0 && best < 0; k--)
+    if (res[k] > 0 && res[k] * 10 >= resmax * 9) best = k;
+  if (best < 0) return fail(-3, "no launch configuration fits: workspace %u bytes per environment", p.ws);
+  p.lanes = cands[best].G;
+  p.launch = cands[best].launch;
+  p.bps = bpsv[best];
+  p.smem = (size_t)p.ws * (32 / p.lanes);
+  const int gpb = 32 / p.lanes;
+  const int need = (h->n + gpb - 1) / gpb;
+  const int cap = p.bps * h->num_sm;
+  p.grid = need < cap ? need : cap;
+  if (p.grid < 1) p.grid = 1;
   return 0;
 }
 
-int configure_fast(hsrb* h) {
-  if (h->fast_configured) return 0;
-  ModelT<float> mm = h->dm;
-  h->fast_ws = (unsigned)push::carve(mm, nullptr, nullptr);
-  if (const char* o = getenv("HSRB_PUSH_PAD")) h->fast_ws += 16u * (unsigned)atoi(o);   // experiments: stride of the environment slices
+// STEP launches of the general path: one warp per environment, as many warps per block as shared memory holds
+int configure_lock(const hsrb* h, Plan& p) {
+  p.ws = (unsigned)ws_carve<float>(h->dm, nullptr, nullptr);
+  p.ncon_max = h->dm.ncon_max; p.nefc_max = h->dm.nefc_max;
+  p.lanes = 32;
+  p.launch = hsrb_step_lock_launch;
+  const size_t tail = lock_tail_bytes();
+  int wpb = (int)((227 * 1024 - tail) / p.ws);
+  if (wpb < 1) return fail(-3, "no launch configuration fits: workspace %u bytes per environment", p.ws);
+  if (wpb > HSRB_LOCK_MAXWARPS) wpb = HSRB_LOCK_MAXWARPS;
+  const int need_w = (h->n + h->num_sm - 1) / h->num_sm;
+  if (wpb > need_w) wpb = need_w;
+  p.threads = 32 * wpb;
+  p.smem = (size_t)p.ws * wpb + tail;
+  CU(hsrb_step_lock_prepare(p, &p.bps));
+  if (p.bps < 1) return fail(-3, "phase-locked general kernel does not fit on an SM (%zu bytes of shared memory)", p.smem);
+  const int need = (h->n + wpb - 1) / wpb;
+  const int cap = p.bps * h->num_sm;
+  p.grid = need < cap ? need : cap;
+  return 0;
+}
+
+int configure_push(const hsrb* h, Plan& p) {
+  p.ws = (unsigned)push::carve(h->dm, nullptr, nullptr);
+  p.ncon_max = PUSH_MAXCON; p.nefc_max = 2 + PUSH_ROWS;
+  p.fam = &h->fast;
+  p.launch = hsrb_push_launch;
   // lanes per environment: the caller's choice (hsrb_config) when it is one this kernel has, else 8
   const int G = (h->lanes_req == 8 || h->lanes_req == 16 || h->lanes_req == 32) ? h->lanes_req : 8;
-  h->fast_lanes = G;
+  p.lanes = G;
   const int epw = 32 / G;
   // warps per block so that all environments are resident in one wave when they fit: n / (envs per warp) / SMs
   int warps_needed = (h->n + epw - 1) / epw;
@@ -189,189 +255,91 @@ int configure_fast(hsrb* h) {
   const int wpb_max = G == 16 ? 14 : 8;   // __launch_bounds__ of the kernel (hsrb_push.cuh)
   if (wpb == 7 && wpb_max >= 8) wpb = 8;   // two warps on each of the four schedulers: 128 blocks x 32 envs beat 147 x 28 (measured +2 %)
   if (wpb > wpb_max) wpb = wpb_max;
-  if (const char* o = getenv("HSRB_PUSH_WPB")) { int v = atoi(o); if (v >= 1 && v <= wpb_max) wpb = v; }   // experiments
   // shared memory: at most 227 KB per block
-  const size_t tail = push::shared_tail(mm);
-  while (wpb > 1 && (size_t)h->fast_ws * (wpb * epw) + tail > 227 * 1024) wpb--;
-  h->fast_threads = 32 * wpb;
-  size_t smem = (size_t)h->fast_ws * (h->fast_threads / G) + tail;
-  CU(hsrb_push_prepare(G, h->fast.nv, smem, h->fast_threads, &h->fast_bps));
-  if (h->fast_bps < 1) return fail(-3, "fast kernel does not fit on an SM (%zu bytes of shared memory)", smem);
-  int epb = h->fast_threads / G;
-  int need = (h->n + epb - 1) / epb;
-  int cap = h->fast_bps * h->num_sm;
-  h->fast_grid = need < cap ? need : cap;
-  h->fast_configured = true;
+  const size_t tail = push::shared_tail(h->dm);
+  while (wpb > 1 && (size_t)p.ws * (wpb * epw) + tail > 227 * 1024) wpb--;
+  p.threads = 32 * wpb;
+  p.smem = (size_t)p.ws * (p.threads / G) + tail;
+  CU(hsrb_push_prepare(p, &p.bps));
+  if (p.bps < 1) return fail(-3, "fast kernel does not fit on an SM (%zu bytes of shared memory)", p.smem);
+  const int epb = p.threads / G;
+  const int need = (h->n + epb - 1) / epb;
+  const int cap = p.bps * h->num_sm;
+  p.grid = need < cap ? need : cap;
   return 0;
 }
 
-// the fast kernels test the env_wrapper-form goal only (one block against the goal point)
-bool use_fast(const hsrb* h) { return h->fast_ok && h->path != 1 && h->cfg.ngoal == 0; }
-// which of the two: path 3 = warp-per-environment kernel (hsrb_wpe.cuh), 2 = 8-lane lock-step kernel (hsrb_push.cuh);
-// 0 (auto) = the warp-per-environment kernel, phase-locked, two teams per block - measured on B200, round 2, TimeLimit
-// workload: 48.4 M substeps/s at 4096 envs (lock-step 8-lane kernel 34.6 M, free-running warps 32.9 M), 65.8 M at
-// 131072 envs (52.3 M / 53.2 M); HSRB_FAST_KERNEL=push|wpe overrides (experiments)
-bool use_wpe(const hsrb* h) {
-  if (!use_fast(h) || !h->wpe_ok) return false;
-  if (h->path == 3) return true;
-  if (h->path == 2) return false;
-  const char* o = getenv("HSRB_FAST_KERNEL");
-  return !(o && o[0] == 'p');
-}
-
-int configure_wpe(hsrb* h) {
-  if (h->wpe_configured) return 0;
-  h->wpe_ws = (unsigned)wpe::slice_bytes();
+int configure_wpe(const hsrb* h, Plan& p) {
+  p.ws = (unsigned)wpe::slice_bytes();
+  p.ncon_max = WPE_MAXCON; p.nefc_max = WPE_MAXROW;
+  p.fam = &h->fast;
+  p.lock = h->knobs.wpe_lock;
+  p.lanes = 32;
+  p.launch = hsrb_wpe_launch;
   const size_t tail = wpe::shared_tail(h->dm);
   // one warp per environment; all environments resident in one wave when they fit (warps per block = n / SMs),
   // otherwise the most warps shared memory and the register file hold, and a grid-stride loop over the environments
   int wpb = (h->n + h->num_sm - 1) / h->num_sm;
   if (wpb < 1) wpb = 1;
   if (wpb > WPE_MAXWARPS) wpb = WPE_MAXWARPS;
-  if (const char* o = getenv("HSRB_WPE_WPB")) { int v = atoi(o); if (v >= 1 && v <= WPE_MAXWARPS) wpb = v; }   // experiments
-  while (wpb > 1 && (size_t)h->wpe_ws * wpb + tail > 227 * 1024) wpb--;
-  h->wpe_threads = 32 * wpb;
-  const size_t smem = (size_t)h->wpe_ws * wpb + tail;
-  CU(hsrb_wpe_prepare(smem, h->wpe_threads, &h->wpe_bps));
-  if (h->wpe_bps < 1) return fail(-3, "warp-per-environment kernel does not fit on an SM (%zu bytes of shared memory)", smem);
+  if (h->knobs.wpe_wpb >= 1 && h->knobs.wpe_wpb <= WPE_MAXWARPS) wpb = h->knobs.wpe_wpb;
+  while (wpb > 1 && (size_t)p.ws * wpb + tail > 227 * 1024) wpb--;
+  p.threads = 32 * wpb;
+  p.smem = (size_t)p.ws * wpb + tail;
+  CU(hsrb_wpe_prepare(p, &p.bps));
+  if (p.bps < 1) return fail(-3, "warp-per-environment kernel does not fit on an SM (%zu bytes of shared memory)", p.smem);
   const int need = (h->n + wpb - 1) / wpb;
-  const int cap = h->wpe_bps * h->num_sm;
-  h->wpe_grid = need < cap ? need : cap;
-  if (wpb > 1 && h->wpe_grid < cap && 2 * h->wpe_grid > cap) h->wpe_grid = cap;   // 4096 envs: 148 blocks of 27-28 instead of 147 of 28 + an idle SM
-  if (const char* o = getenv("HSRB_WPE_GRID")) { int v = atoi(o); if (v >= 1 && v < h->wpe_grid) h->wpe_grid = v; }   // experiments
-  h->wpe_configured = true;
+  const int cap = p.bps * h->num_sm;
+  p.grid = need < cap ? need : cap;
+  if (wpb > 1 && p.grid < cap && 2 * p.grid > cap) p.grid = cap;   // 4096 envs: 148 blocks of 27-28 instead of 147 of 28 + an idle SM
   return 0;
 }
 
-// STEP launches of the general path: one warp per environment, as many warps per block as shared memory holds
-int configure_lock(hsrb* h) {
-  if (h->lock_configured) return 0;
-  h->ws_bytes = (unsigned)ws_carve<float>(h->dm, nullptr, nullptr);
-  const size_t tail = lock_tail_bytes();
-  int wpb = (int)((227 * 1024 - tail) / h->ws_bytes);
-  if (wpb < 1) return fail(-3, "no launch configuration fits: workspace %u bytes per environment", h->ws_bytes);
-  if (wpb > HSRB_LOCK_MAXWARPS) wpb = HSRB_LOCK_MAXWARPS;
-  const int need_w = (h->n + h->num_sm - 1) / h->num_sm;
-  if (wpb > need_w) wpb = need_w;
-  if (const char* o = getenv("HSRB_LOCK_WPB")) { int v = atoi(o); if (v >= 1 && v <= wpb) wpb = v; }   // experiments
-  h->lock_threads = 32 * wpb;
-  const size_t smem = (size_t)h->ws_bytes * wpb + tail;
-  CU(hsrb_prepare_step_lock(smem, h->lock_threads, &h->lock_bps));
-  if (h->lock_bps < 1) return fail(-3, "phase-locked general kernel does not fit on an SM (%zu bytes of shared memory)", smem);
-  const int need = (h->n + wpb - 1) / wpb;
-  const int cap = h->lock_bps * h->num_sm;
-  h->lock_grid = need < cap ? need : cap;
-  h->lock_configured = true;
-  return 0;
-}
-bool use_lock(const hsrb* h) {
-  if (h->hm.m.npair > 256) return false;
-  const char* o = getenv("HSRB_GENERAL_LOCK");
-  return !(o && o[0] == '0');
-}
-
-// Work-sorted launch order of the warp-per-environment kernel (hsrb_wpe_kernel_t): the action
-// kernel writes a work estimate per environment, a radix sort (cub, descending, stable) turns it into the order of the next
-// launch.  HSRB_WPE_SORT=0 switches it off (experiments; results do not depend on it).
-bool use_sorted_order() {
-  const char* so = getenv("HSRB_WPE_SORT");
-  return !(so && so[0] == '0');
-}
-int sort_prepare(hsrb* h, KArgs& a, void* stream) {
-  if (!h->d_work) {
-    const size_t nb = sizeof(int) * (size_t)h->n;
-    CU(cudaMalloc(&h->d_work, nb)); CU(cudaMalloc(&h->d_work_sorted, nb)); CU(cudaMalloc(&h->d_iota, nb)); CU(cudaMalloc(&h->d_order, nb));
-    CU(cudaMemsetAsync(h->d_work, 0, nb, (cudaStream_t)stream));
-    fill_iota<<<(h->n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->d_iota, h->n);
-    CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, h->sort_tmp_bytes, h->d_work, h->d_work_sorted, h->d_iota, h->d_order, h->n, 0, 24,
-                                                 (cudaStream_t)stream));
-    CU(cudaMalloc(&h->d_sort_tmp, h->sort_tmp_bytes));
+// the plan of kernel k, worked out on first use
+int configure(hsrb* h, Kernel k, const Plan** out) {
+  Plan& p = h->plan[k];
+  if (!p.ready) {
+    Plan q = Plan();
+    const int rc = k == K_WPE ? configure_wpe(h, q) : k == K_PUSH ? configure_push(h, q) : k == K_LOCK ? configure_lock(h, q)
+                                                                                         : configure_general(h, q);
+    if (rc) return rc;
+    q.ready = true;
+    p = q;
   }
-  a.work = h->d_work; a.order = h->order_valid ? h->d_order : nullptr;
-  return 0;
-}
-int sort_update(hsrb* h, void* stream) {   // the next launch's order (ties keep the environment order)
-  CU(cub::DeviceRadixSort::SortPairsDescending(h->d_sort_tmp, h->sort_tmp_bytes, h->d_work, h->d_work_sorted, h->d_iota, h->d_order, h->n, 0, 24,
-                                               (cudaStream_t)stream));
-  h->order_valid = true;
+  *out = &p;
   return 0;
 }
 
 KArgs base_args(hsrb* h) {
   KArgs a;
   memset(&a, 0, sizeof(a));
-  a.m = h->dm; a.cfg = h->cfg; a.n = h->n; a.S = h->S; a.ws_bytes = h->ws_bytes;
+  a.m = h->dm; a.cfg = h->cfg; a.n = h->n; a.S = h->S;
   a.seed = h->seed; a.env_off = h->env_off; a.state = h->d_state; a.episode = h->d_episode; a.stats = h->d_stats;
-  if (const char* o = getenv("HSRB_OPTS")) a.opts = (unsigned)strtoul(o, nullptr, 0);   // experiment switches
+  a.opts = h->knobs.opts;
   return a;
 }
 
 int run(hsrb* h, KArgs& a, void* stream) {
-  if (a.mode == MODE_STEP && use_wpe(h)) {
-    int rc = configure_wpe(h);
-    if (rc) return rc;
-    a.ws_bytes = h->wpe_ws;
-    a.m.ncon_max = WPE_MAXCON; a.m.nefc_max = WPE_MAXROW;
-    const size_t smem = (size_t)h->wpe_ws * (h->wpe_threads / 32) + wpe::shared_tail(h->dm);
-    // phase-locked variant with two teams per block by default; HSRB_WPE_LOCK=0: free-running warps, HSRB_WPE_TEAMS=1|2|4
-    const char* lk = getenv("HSRB_WPE_LOCK");
-    const char* tm = getenv("HSRB_WPE_TEAMS");
-    const bool lock = !(lk && lk[0] == '0');
-    const unsigned teams = tm ? (unsigned)atoi(tm) : 2u;
-    if (!(a.opts & 0xf0u)) a.opts |= (teams & 15u) << 4;
-    const bool sorted = use_sorted_order();
-    if (sorted) { int rc2 = sort_prepare(h, a, stream); if (rc2) return rc2; }
-    CU(hsrb_wpe_launch(a, h->fast, h->wpe_grid, h->wpe_threads, smem, (cudaStream_t)stream, lock));
-    if (sorted) { int rc2 = sort_update(h, stream); if (rc2) return rc2; }
-    h->launches++;
-    return 0;
-  }
-  if (a.mode == MODE_STEP && use_fast(h)) {
-    int rc = configure_fast(h);
-    if (rc) return rc;
-    a.ws_bytes = h->fast_ws;
-    a.m.ncon_max = PUSH_MAXCON; a.m.nefc_max = 2 + PUSH_ROWS;
-    size_t smem = (size_t)h->fast_ws * (h->fast_threads / h->fast_lanes) + push::shared_tail(h->dm);
-    CU(hsrb_push_launch(h->fast_lanes, h->fast.nv, a, h->fast, h->fast_grid, h->fast_threads, smem, (cudaStream_t)stream));
-    h->launches++;
-    return 0;
-  }
-  if (a.mode == MODE_STEP && h->path == 2) return fail(-3, "fast path not available for this model: %s", h->fast_why);
-  if (a.mode == MODE_STEP && use_lock(h) && !h->lanes_req) {
-    int rc = configure_lock(h);
-    if (rc) return rc;
-    a.ws_bytes = h->ws_bytes;
-    a.m.ncon_max = h->dm.ncon_max; a.m.nefc_max = h->dm.nefc_max;
-    const size_t smem = (size_t)h->ws_bytes * (h->lock_threads / 32) + lock_tail_bytes();
-    // (the work-sorted launch order of the wpe kernel was tried here too: no gain on configs[2] / [4], 2.80 vs 2.88 and 1.28 vs
-    // 1.35 M substeps/s - configs[2] resets every environment before every action, configs[4] runs four warps per block)
-    CU(hsrb_launch_step_lock(a, h->lock_grid, h->lock_threads, smem, (cudaStream_t)stream));
-    h->launches++;
-    return 0;
-  }
-  int rc = configure(h);
-  if (rc) return rc;
-  a.ws_bytes = h->ws_bytes;
-  a.m.ncon_max = h->dm.ncon_max; a.m.nefc_max = h->dm.nefc_max;
-  size_t smem = (size_t)h->ws_bytes * (32 / h->lanes);
-  if (a.mode == MODE_RESET || a.mode == MODE_FORWARD) CU(launch_aux(h->lanes, a, h->grid, smem, (cudaStream_t)stream));   // the lean instance
-  else CU(launch(h->lanes, a, h->grid, smem, (cudaStream_t)stream));
-  h->launches++;
-  return 0;
-}
-
-// episode buffers, zeroed on the caller's stream
-int episode_alloc(hsrb* h, void* stream) {
-  if (h->d_age) return 0;
-  const size_t n = (size_t)h->n;
   cudaStream_t s = (cudaStream_t)stream;
-  CU(cudaMalloc(&h->d_age, sizeof(int) * n)); CU(cudaMalloc(&h->d_ep_sub, sizeof(int) * n)); CU(cudaMalloc(&h->d_ep_ret, sizeof(float) * n));
-  CU(cudaMalloc(&h->d_ep_counters, sizeof(unsigned long long) * EP_COUNT));
-  CU(cudaMalloc(&h->d_ep_term, n)); CU(cudaMalloc(&h->d_ep_bad, n));
-  CU(cudaMalloc(&h->d_ep_reward, sizeof(float) * n)); CU(cudaMalloc(&h->d_ep_taken, sizeof(int) * n));
-  CU(cudaMemsetAsync(h->d_age, 0, sizeof(int) * n, s)); CU(cudaMemsetAsync(h->d_ep_sub, 0, sizeof(int) * n, s));
-  CU(cudaMemsetAsync(h->d_ep_ret, 0, sizeof(float) * n, s));
-  CU(cudaMemsetAsync(h->d_ep_counters, 0, sizeof(unsigned long long) * EP_COUNT, s));
+  Kernel k = K_GENERAL;
+  if (a.mode == MODE_STEP) { const int rc = select(h, &k); if (rc) return rc; }
+  const Plan* p = nullptr;
+  int rc = configure(h, k, &p);
+  if (rc) return rc;
+  a.ws_bytes = p->ws;
+  a.m.ncon_max = p->ncon_max; a.m.nefc_max = p->nefc_max;
+  const bool sorted = k == K_WPE && h->knobs.wpe_sort;
+  if (k == K_WPE && !(a.opts & 0xf0u)) a.opts |= (h->knobs.wpe_teams & 15u) << 4;
+  if (sorted) {
+    if ((rc = h->sort.alloc(h->n, s))) return rc;
+    a.work = h->sort.work; a.order = h->sort.valid ? h->sort.order : nullptr;
+  }
+  // (the work-sorted launch order was tried on the phase-locked general kernel too: no gain on configs[2] / [4], 2.80 vs
+  // 2.88 and 1.28 vs 1.35 M substeps/s - configs[2] resets every environment before every action, configs[4] runs four
+  // warps per block)
+  CU(p->launch(*p, a, s));
+  if (sorted && (rc = h->sort.update(h->n, s))) return rc;
+  h->launches++;
   return 0;
 }
 
@@ -379,25 +347,26 @@ int episode_alloc(hsrb* h, void* stream) {
 int run_episode(hsrb* h, int max_steps, int autoreset, const unsigned char* term, const float* reward, const int* taken,
                 const unsigned char* bad, float* obs, unsigned char* truncated, float* final_obs, int* ep_length, float* ep_return,
                 int* ep_substeps, void* stream) {
-  int rc = episode_alloc(h, stream);
+  int rc = h->ep.alloc(h->n, (cudaStream_t)stream);
   if (rc) return rc;
-  rc = configure(h);
+  const Plan* p = nullptr;
+  rc = configure(h, K_GENERAL, &p);
   if (rc) return rc;
-  if (h->ep_lanes != h->lanes) {
-    CU(hsrb_episode_prepare(h->lanes));
-    h->ep_lanes = h->lanes;
+  if (h->ep.lanes != p->lanes) {
+    CU(hsrb_episode_prepare(*p));
+    h->ep.lanes = p->lanes;
   }
   EpArgs e;
   memset(&e, 0, sizeof(e));
   e.k = base_args(h);
-  e.k.ws_bytes = h->ws_bytes;
+  e.k.ws_bytes = p->ws;
   e.k.obs = obs;
   e.max_steps = max_steps; e.autoreset = autoreset;
   e.terminated = term; e.reward = reward; e.taken = taken; e.bad = bad;
-  e.age = h->d_age; e.ret = h->d_ep_ret; e.sub = h->d_ep_sub;
+  e.age = h->ep.age; e.ret = h->ep.ret; e.sub = h->ep.sub;
   e.truncated = truncated; e.final_obs = final_obs; e.ep_length = ep_length; e.ep_return = ep_return; e.ep_substeps = ep_substeps;
-  e.counters = h->d_ep_counters;
-  CU(hsrb_episode_launch(h->lanes, e, h->grid, (size_t)h->ws_bytes * (32 / h->lanes), (cudaStream_t)stream));
+  e.counters = h->ep.counters;
+  CU(hsrb_episode_launch(*p, e, (cudaStream_t)stream));
   h->launches++;
   return 0;
 }
@@ -566,6 +535,7 @@ int hsrb_create(const void* model_blob, size_t bytes, int n_envs, int device, ui
   }
   if (device < 0 || device >= ndev) { delete h; return fail(-1, "device %d out of range (%d visible)", device, ndev); }
   h->n = n_envs; h->device = device; h->seed = seed; h->env_off = env_id_offset;
+  h->knobs = read_knobs();
   h->S = h->hm.m.nq + 2 * h->hm.m.nv + 3;
   memset(&h->cfg, 0, sizeof(h->cfg));
   h->cfg.qidx0 = 0; h->cfg.qidx1 = 2;
@@ -624,17 +594,18 @@ int hsrb_set_path(hsrb_t* h, int path) {
   if (path >= 2 && !h->fast_ok) return fail(-3, "fast path not available for this model: %s", h->fast_why);
   if (path == 3 && !h->wpe_ok) return fail(-3, "warp-per-environment kernel not available for this model");
   h->path = path;
-  return use_wpe(h) ? 3 : (use_fast(h) ? 2 : 1);
+  Kernel k;
+  const int rc = select(h, &k);
+  return rc ? rc : kPathCode[k];
 }
 
 int hsrb_destroy(hsrb_t* h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
   cudaFree(h->d_fast_tab); cudaFree(h->d_model); cudaFree(h->d_state); cudaFree(h->d_episode); cudaFree(h->d_stats);
-  cudaFree(h->d_work); cudaFree(h->d_work_sorted); cudaFree(h->d_iota); cudaFree(h->d_order); cudaFree(h->d_sort_tmp);
   cudaFree(h->d_ctrl); cudaFree(h->d_obs); cudaFree(h->d_reward); cudaFree(h->d_done); cudaFree(h->d_taken);
-  cudaFree(h->d_age); cudaFree(h->d_ep_sub); cudaFree(h->d_ep_ret); cudaFree(h->d_ep_counters);
-  cudaFree(h->d_ep_term); cudaFree(h->d_ep_bad); cudaFree(h->d_ep_reward); cudaFree(h->d_ep_taken);
+  h->sort.free();
+  h->ep.free();
   delete h;
   return 0;
 }
@@ -656,12 +627,10 @@ int hsrb_config(hsrb_t* h, int lanes_per_env, int ncon_max, int nefc_max) {
   h->lanes_req = lanes_per_env;
   if (ncon_max > 0) h->dm.ncon_max = h->hm.m.ncon_max = ncon_max;
   if (nefc_max > 0) h->dm.nefc_max = h->hm.m.nefc_max = nefc_max;
-  h->configured = false;
-  h->fast_configured = false;
-  h->wpe_configured = false;
-  h->lock_configured = false;
+  for (Plan& p : h->plan) p = Plan();
   CU(cudaSetDevice(h->device));
-  return configure(h);
+  const Plan* p = nullptr;
+  return configure(h, K_GENERAL, &p);
 }
 
 int hsrb_set_goals(hsrb_t* h, const float* goal_lohi, const float* block_lohi, float geofence, float min_sep, int qidx0,
@@ -724,9 +693,9 @@ int hsrb_set_starts(hsrb_t* h, int nstart, const int32_t* qpos_adr, const int32_
 #if defined(WPE_CHAIN_CLOCKS)
 // experiment hook (not part of include/hsrb.h): the per-environment work array of the last wpe launch -> host
 extern "C" int hsrb_debug_work(hsrb_t* h, int* out_host) {
-  if (!h || !h->d_work) return -1;
+  if (!h || !h->sort.work) return -1;
   cudaDeviceSynchronize();
-  return cudaMemcpy(out_host, h->d_work, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : -2;
+  return cudaMemcpy(out_host, h->sort.work, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : -2;
 }
 #endif
 
@@ -736,8 +705,8 @@ int hsrb_reset(hsrb_t* h, const uint8_t* mask, float* obs, void* stream) {
   KArgs a = base_args(h);
   a.mode = MODE_RESET; a.mask = mask; a.obs = obs; a.nsub = 0;
   const int rc = run(h, a, stream);
-  if (rc || !h->d_age) return rc;
-  CU(hsrb_episode_clear(mask, h->n, h->d_age, h->d_ep_ret, h->d_ep_sub, (cudaStream_t)stream));
+  if (rc || !h->ep.age) return rc;
+  CU(hsrb_episode_clear(mask, h->n, h->ep.age, h->ep.ret, h->ep.sub, (cudaStream_t)stream));
   return 0;
 }
 
@@ -759,13 +728,13 @@ int hsrb_step_episode(hsrb_t* h, const float* ctrl, int nsubsteps, int max_episo
   if (!h) return fail(-1, "null handle");
   if (max_episode_steps < 0) return fail(-1, "max_episode_steps < 0");
   CU(cudaSetDevice(h->device));
-  int rc = episode_alloc(h, stream);
+  int rc = h->ep.alloc(h->n, (cudaStream_t)stream);
   if (rc) return rc;
   // what the episode kernel reads goes to the handle's buffers when the caller does not want it
-  uint8_t* term = terminated ? terminated : h->d_ep_term;
-  float* rew = reward ? reward : h->d_ep_reward;
-  int32_t* taken = substeps_taken ? substeps_taken : h->d_ep_taken;
-  uint8_t* bad = bad_state ? bad_state : h->d_ep_bad;
+  uint8_t* term = terminated ? terminated : h->ep.term;
+  float* rew = reward ? reward : h->ep.reward;
+  int32_t* taken = substeps_taken ? substeps_taken : h->ep.taken;
+  uint8_t* bad = bad_state ? bad_state : h->ep.bad;
   rc = hsrb_step(h, ctrl, nsubsteps, obs, rew, term, nullptr, taken, bad, stream);
   if (rc) return rc;
   return run_episode(h, max_episode_steps, autoreset, term, rew, taken, bad, obs, truncated, final_obs, ep_length, ep_return,
@@ -786,23 +755,23 @@ int hsrb_episode_update(hsrb_t* h, int max_episode_steps, int autoreset, const u
 int hsrb_set_episode_ages(hsrb_t* h, const int32_t* age, void* stream) {
   if (!h) return fail(-1, "null handle");
   CU(cudaSetDevice(h->device));
-  int rc = episode_alloc(h, stream);
-  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
+  int rc = h->ep.alloc(h->n, s);
+  if (rc) return rc;
   const size_t n = (size_t)h->n;
-  if (age) CU(cudaMemcpyAsync(h->d_age, age, sizeof(int) * n, cudaMemcpyDeviceToDevice, s));
-  else CU(cudaMemsetAsync(h->d_age, 0, sizeof(int) * n, s));
-  CU(cudaMemsetAsync(h->d_ep_ret, 0, sizeof(float) * n, s));
-  CU(cudaMemsetAsync(h->d_ep_sub, 0, sizeof(int) * n, s));
+  if (age) CU(cudaMemcpyAsync(h->ep.age, age, sizeof(int) * n, cudaMemcpyDeviceToDevice, s));
+  else CU(cudaMemsetAsync(h->ep.age, 0, sizeof(int) * n, s));
+  CU(cudaMemsetAsync(h->ep.ret, 0, sizeof(float) * n, s));
+  CU(cudaMemsetAsync(h->ep.sub, 0, sizeof(int) * n, s));
   return 0;
 }
 
 int hsrb_get_episode_ages(hsrb_t* h, int32_t* age, void* stream) {
   if (!h || !age) return fail(-1, "bad arguments");
   CU(cudaSetDevice(h->device));
-  int rc = episode_alloc(h, stream);
+  int rc = h->ep.alloc(h->n, (cudaStream_t)stream);
   if (rc) return rc;
-  CU(cudaMemcpyAsync(age, h->d_age, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  CU(cudaMemcpyAsync(age, h->ep.age, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 
@@ -810,10 +779,10 @@ int hsrb_episode_stats(hsrb_t* h, int64_t* out8, void* stream) {
   static_assert(EP_COUNT == 8, "hsrb.h documents 8 counters");
   if (!h || !out8) return fail(-1, "bad arguments");
   CU(cudaSetDevice(h->device));
-  int rc = episode_alloc(h, stream);
+  int rc = h->ep.alloc(h->n, (cudaStream_t)stream);
   if (rc) return rc;
   unsigned long long v[EP_COUNT];
-  CU(cudaMemcpyAsync(v, h->d_ep_counters, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  CU(cudaMemcpyAsync(v, h->ep.counters, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   CU(cudaStreamSynchronize((cudaStream_t)stream));
   for (int i = 0; i < EP_COUNT; i++) out8[i] = (int64_t)v[i];
   return 0;
@@ -964,34 +933,16 @@ int hsrb_measure_fp32_peak(int device, double* tflops_out) {
   return 0;
 }
 
-int hsrb_launch_info(hsrb_t* h, int* out4) {  // out4: 6 ints
-  if (!h || !out4) return fail(-1, "bad arguments");
+int hsrb_launch_info(hsrb_t* h, int* out6) {
+  if (!h || !out6) return fail(-1, "bad arguments");
   CU(cudaSetDevice(h->device));
-  int rc = configure(h);
+  Kernel k;
+  const Plan* p = nullptr;
+  int rc = select(h, &k);
+  if (!rc) rc = configure(h, k, &p);
   if (rc) return rc;
-  if (use_wpe(h)) {
-    rc = configure_wpe(h);
-    if (rc) return rc;
-    out4[0] = 32; out4[1] = (int)h->wpe_ws; out4[2] = h->wpe_bps * (h->wpe_threads / 32); out4[3] = h->wpe_grid;
-    out4[4] = 3; out4[5] = h->wpe_threads;
-    return 0;
-  }
-  if (use_fast(h)) {
-    rc = configure_fast(h);
-    if (rc) return rc;
-    out4[0] = h->fast_lanes; out4[1] = (int)h->fast_ws; out4[2] = h->fast_bps * (h->fast_threads / h->fast_lanes); out4[3] = h->fast_grid;
-    out4[4] = 2; out4[5] = h->fast_threads;
-    return 0;
-  }
-  if (use_lock(h) && !h->lanes_req) {
-    rc = configure_lock(h);
-    if (rc) return rc;
-    out4[0] = 32; out4[1] = (int)h->ws_bytes; out4[2] = h->lock_bps * (h->lock_threads / 32); out4[3] = h->lock_grid;
-    out4[4] = 1; out4[5] = h->lock_threads;
-    return 0;
-  }
-  out4[0] = h->lanes; out4[1] = (int)h->ws_bytes; out4[2] = h->blocks_per_sm * (32 / h->lanes); out4[3] = h->grid;
-  out4[4] = 1; out4[5] = 32;
+  out6[0] = p->lanes; out6[1] = (int)p->ws; out6[2] = p->bps * (p->threads / p->lanes); out6[3] = p->grid;
+  out6[4] = kPathCode[k]; out6[5] = p->threads;
   return 0;
 }
 

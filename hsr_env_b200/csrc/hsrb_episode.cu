@@ -20,8 +20,8 @@ cudaError_t launch_g(const EpArgs& a, int grid, size_t smem, cudaStream_t s) {
 }
 }  // namespace
 
-cudaError_t hsrb_episode_prepare(int G) {
-  switch (G) {
+cudaError_t hsrb_episode_prepare(const Plan& p) {
+  switch (p.lanes) {
     case 4: return prepare_g<4>();
     case 8: return prepare_g<8>();
     case 16: return prepare_g<16>();
@@ -29,12 +29,12 @@ cudaError_t hsrb_episode_prepare(int G) {
   }
 }
 
-cudaError_t hsrb_episode_launch(int G, const EpArgs& a, int grid, size_t smem, cudaStream_t s) {
-  switch (G) {
-    case 4: return launch_g<4>(a, grid, smem, s);
-    case 8: return launch_g<8>(a, grid, smem, s);
-    case 16: return launch_g<16>(a, grid, smem, s);
-    default: return launch_g<32>(a, grid, smem, s);
+cudaError_t hsrb_episode_launch(const Plan& p, const EpArgs& a, cudaStream_t s) {   // one warp per block (p.threads)
+  switch (p.lanes) {
+    case 4: return launch_g<4>(a, p.grid, p.smem, s);
+    case 8: return launch_g<8>(a, p.grid, p.smem, s);
+    case 16: return launch_g<16>(a, p.grid, p.smem, s);
+    default: return launch_g<32>(a, p.grid, p.smem, s);
   }
 }
 

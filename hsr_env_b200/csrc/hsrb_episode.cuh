@@ -114,8 +114,8 @@ __global__ void __launch_bounds__(32) hsrb_episode_kernel(const __grid_constant_
   }
 }
 
-// host side (hsrb_episode.cu)
-cudaError_t hsrb_episode_prepare(int G);
-cudaError_t hsrb_episode_launch(int G, const EpArgs& a, int grid, size_t smem, cudaStream_t s);
+// host side (hsrb_episode.cu), in the general kernel's plan p: p.lanes picks G; prepare sets the shared-memory limit
+cudaError_t hsrb_episode_prepare(const Plan& p);
+cudaError_t hsrb_episode_launch(const Plan& p, const EpArgs& a, cudaStream_t s);
 // the environments in `mask` (null = all) start new episodes: their ages and sums restart at 0 (hsrb_reset)
 cudaError_t hsrb_episode_clear(const unsigned char* mask, int n, int* age, float* ret, int* sub, cudaStream_t s);

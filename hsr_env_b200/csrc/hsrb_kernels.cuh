@@ -344,28 +344,41 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
   }
 }
 #endif  // HSRB_STEP_LOCK_IMPL
-cudaError_t hsrb_prepare_step_lock(size_t smem, int threads, int* blocks_per_sm);
-cudaError_t hsrb_launch_step_lock(const KArgs& a, int grid, int threads, size_t smem, cudaStream_t s);
 
-// per-G entry points, one translation unit each (parallel compilation)
-#define HSRB_DECL_G(G)                                                \
-  cudaError_t hsrb_prepare_step_##G(size_t smem, int* blocks_per_sm); \
-  cudaError_t hsrb_launch_step_##G(const KArgs& a, int grid, size_t smem, cudaStream_t s); \
-  cudaError_t hsrb_launch_aux_##G(const KArgs& a, int grid, size_t smem, cudaStream_t s);
+// Launch configuration of one action kernel for one handle, worked out by hsrb_api.cu (configure) on first use.  Every
+// kernel translation unit exports the same two entry points: X_prepare(p, &bps) sets the kernel's shared-memory limit
+// and returns the resident blocks per SM at p.threads / p.smem; X_launch(p, a, s) launches the template instance p and
+// a.mode call for.
+struct PushInfo;
+struct Plan {
+  bool ready;
+  int lanes, threads, grid, bps;   // lanes per environment, threads per block, blocks, resident blocks per SM
+  unsigned ws;                     // shared-memory bytes of one environment's workspace (KArgs::ws_bytes)
+  size_t smem;                     // dynamic shared memory of a block
+  int ncon_max, nefc_max;          // contacts / constraint rows the kernel holds per environment
+  const PushInfo* fam;             // push / wpe kernels: constants of the sliding-base family
+  bool lock;                       // wpe kernel: the phase-locked instance
+  cudaError_t (*launch)(const Plan& p, const KArgs& a, cudaStream_t s);
+};
+
+cudaError_t hsrb_step_lock_prepare(const Plan& p, int* bps);
+cudaError_t hsrb_step_lock_launch(const Plan& p, const KArgs& a, cudaStream_t s);
+
+// per-G entry points of hsrb_step_kernel, one translation unit each (parallel compilation)
+#define HSRB_DECL_G(G)                                          \
+  cudaError_t hsrb_step##G##_prepare(const Plan& p, int* bps); \
+  cudaError_t hsrb_step##G##_launch(const Plan& p, const KArgs& a, cudaStream_t s);
 HSRB_DECL_G(4) HSRB_DECL_G(8) HSRB_DECL_G(16) HSRB_DECL_G(32)
 
 #define HSRB_DEFINE_G(G)                                                                                               \
-  cudaError_t hsrb_prepare_step_##G(size_t smem, int* bps) {                                                           \
+  cudaError_t hsrb_step##G##_prepare(const Plan& p, int* bps) {                                                        \
     cudaError_t e = cudaFuncSetAttribute(hsrb_step_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); /* per function, shared by all handles */ \
     if (e == cudaSuccess) e = cudaFuncSetAttribute(hsrb_step_kernel<G, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); \
     if (e != cudaSuccess) return e;                                                                                    \
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_kernel<G>, 32, smem);                          \
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_kernel<G>, p.threads, p.smem);                 \
   }                                                                                                                    \
-  cudaError_t hsrb_launch_step_##G(const KArgs& a, int grid, size_t smem, cudaStream_t s) {                            \
-    hsrb_step_kernel<G><<<grid, 32, smem, s>>>(a);                                                                     \
-    return cudaGetLastError();                                                                                         \
-  }                                                                                                                    \
-  cudaError_t hsrb_launch_aux_##G(const KArgs& a, int grid, size_t smem, cudaStream_t s) { /* reset / forward launches */ \
-    hsrb_step_kernel<G, false><<<grid, 32, smem, s>>>(a);                                                              \
+  cudaError_t hsrb_step##G##_launch(const Plan& p, const KArgs& a, cudaStream_t s) {                                   \
+    if (a.mode == MODE_RESET || a.mode == MODE_FORWARD) hsrb_step_kernel<G, false><<<p.grid, p.threads, p.smem, s>>>(a); /* the lean instance */ \
+    else hsrb_step_kernel<G><<<p.grid, p.threads, p.smem, s>>>(a);                                                     \
     return cudaGetLastError();                                                                                         \
   }

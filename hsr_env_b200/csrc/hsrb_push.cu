@@ -3,36 +3,32 @@
 #include "hsrb_push.cuh"
 
 template <int G, int NV>
-static cudaError_t prepare_t(size_t smem, int threads, int* bps) {
+static cudaError_t prepare_t(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_push_kernel<G, NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);   // per function, not per handle: handles with different layouts share it
   if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_push_kernel<G, NV>, threads, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_push_kernel<G, NV>, p.threads, p.smem);
 }
 
-template <int G>
-static cudaError_t prepare_g(int nv, size_t smem, int threads, int* bps) {
-  return nv == 8 ? prepare_t<G, 8>(smem, threads, bps) : prepare_t<G, 2>(smem, threads, bps);
-}
-
-cudaError_t hsrb_push_prepare(int G, int nv, size_t smem, int threads, int* bps) {
-  switch (G) {
-    case 8: return prepare_g<8>(nv, smem, threads, bps);
-    case 16: return prepare_g<16>(nv, smem, threads, bps);
-    default: return prepare_g<32>(nv, smem, threads, bps);
-  }
-}
-
-template <int G>
-static void launch_g(int nv, const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s) {
-  if (nv == 8) hsrb_push_kernel<G, 8><<<grid, threads, smem, s>>>(a, f);
-  else hsrb_push_kernel<G, 2><<<grid, threads, smem, s>>>(a, f);
-}
-
-cudaError_t hsrb_push_launch(int G, int nv, const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s) {
-  switch (G) {
-    case 8: launch_g<8>(nv, a, f, grid, threads, smem, s); break;
-    case 16: launch_g<16>(nv, a, f, grid, threads, smem, s); break;
-    default: launch_g<32>(nv, a, f, grid, threads, smem, s); break;
-  }
+template <int G, int NV>
+static cudaError_t launch_t(const Plan& p, const KArgs& a, cudaStream_t s) {
+  hsrb_push_kernel<G, NV><<<p.grid, p.threads, p.smem, s>>>(a, *p.fam);
   return cudaGetLastError();
+}
+
+cudaError_t hsrb_push_prepare(const Plan& p, int* bps) {
+  const bool blk = p.fam->nv == 8;
+  switch (p.lanes) {
+    case 8: return blk ? prepare_t<8, 8>(p, bps) : prepare_t<8, 2>(p, bps);
+    case 16: return blk ? prepare_t<16, 8>(p, bps) : prepare_t<16, 2>(p, bps);
+    default: return blk ? prepare_t<32, 8>(p, bps) : prepare_t<32, 2>(p, bps);
+  }
+}
+
+cudaError_t hsrb_push_launch(const Plan& p, const KArgs& a, cudaStream_t s) {
+  const bool blk = p.fam->nv == 8;
+  switch (p.lanes) {
+    case 8: return blk ? launch_t<8, 8>(p, a, s) : launch_t<8, 2>(p, a, s);
+    case 16: return blk ? launch_t<16, 8>(p, a, s) : launch_t<16, 2>(p, a, s);
+    default: return blk ? launch_t<32, 8>(p, a, s) : launch_t<32, 2>(p, a, s);
+  }
 }

@@ -1275,3 +1275,7 @@ __global__ void __launch_bounds__(G == 16 ? 448 : 256) hsrb_push_kernel(const __
     __syncwarp();
   }
 }
+
+// host side (hsrb_push.cu): p.lanes picks G, p.fam->nv picks NV
+cudaError_t hsrb_push_prepare(const Plan& p, int* bps);
+cudaError_t hsrb_push_launch(const Plan& p, const KArgs& a, cudaStream_t s);

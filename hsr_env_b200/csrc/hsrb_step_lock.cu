@@ -2,13 +2,13 @@
 #define HSRB_STEP_LOCK_IMPL 1
 #include "hsrb_kernels.cuh"
 
-cudaError_t hsrb_prepare_step_lock(size_t smem, int threads, int* bps) {
+cudaError_t hsrb_step_lock_prepare(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_step_lock_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_lock_kernel, threads, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_lock_kernel, p.threads, p.smem);
 }
 
-cudaError_t hsrb_launch_step_lock(const KArgs& a, int grid, int threads, size_t smem, cudaStream_t s) {
-  hsrb_step_lock_kernel<<<grid, threads, smem, s>>>(a);
+cudaError_t hsrb_step_lock_launch(const Plan& p, const KArgs& a, cudaStream_t s) {
+  hsrb_step_lock_kernel<<<p.grid, p.threads, p.smem, s>>>(a);
   return cudaGetLastError();
 }

@@ -3,16 +3,17 @@
 #define HSRB_WPE_IMPL 1
 #include "hsrb_wpe.cuh"
 
-cudaError_t hsrb_wpe_prepare(size_t smem, int threads, int* bps) {
+// occupancy of the free-running instance for both: the plan's layout is the same whichever p.lock launches
+cudaError_t hsrb_wpe_prepare(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_wpe_kernel_t<false>, threads, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_wpe_kernel_t<false>, p.threads, p.smem);
 }
 
-cudaError_t hsrb_wpe_launch(const KArgs& a, const PushInfo& f, int grid, int threads, size_t smem, cudaStream_t s, bool lock) {
-  if (lock) hsrb_wpe_kernel_t<true><<<grid, threads, smem, s>>>(a, f);
-  else hsrb_wpe_kernel_t<false><<<grid, threads, smem, s>>>(a, f);
+cudaError_t hsrb_wpe_launch(const Plan& p, const KArgs& a, cudaStream_t s) {
+  if (p.lock) hsrb_wpe_kernel_t<true><<<p.grid, p.threads, p.smem, s>>>(a, *p.fam);
+  else hsrb_wpe_kernel_t<false><<<p.grid, p.threads, p.smem, s>>>(a, *p.fam);
   return cudaGetLastError();
 }
 

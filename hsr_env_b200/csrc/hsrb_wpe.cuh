@@ -1376,3 +1376,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) hsrb_wpe_kernel_t(const 
 #endif
 }
 #endif  // HSRB_WPE_IMPL
+
+// host side (hsrb_wpe.cu): p.lock picks the instance
+cudaError_t hsrb_wpe_prepare(const Plan& p, int* bps);
+cudaError_t hsrb_wpe_launch(const Plan& p, const KArgs& a, cudaStream_t s);

@@ -40,7 +40,8 @@ int hsrb_config(hsrb_t* h, int lanes_per_env, int ncon_max, int nefc_max);
 /* Kernel selection: 0 = auto (for the sliding base with at most one free box - the README block-push family - the
  * warp-per-environment kernel hsrb_wpe.cuh; else the general kernel), 1 = general kernel, 2 = the 8-lane lock-step
  * kernel of the family (hsrb_push.cuh), 3 = the warp-per-environment kernel (2, 3: error if the model is outside the
- * family).  Returns the path that will run (1, 2 or 3). */
+ * family).  The fast kernels take the single-goal form of hsrb_set_goals only: with a goal list, 3 runs the general
+ * kernel and 2 is an error.  Returns the path that will run (1, 2 or 3), or the error hsrb_step would return. */
 int hsrb_set_path(hsrb_t* h, int path);
 
 /* GoalSpec(a=block_space, b=goal_space, distance=geofence)  /root/reference/hsr/util.py:70-74, env.py:161-172
@@ -160,8 +161,9 @@ int hsrb_debug_substep(hsrb_t* h, const float* ctrl, double* dump, void* stream)
  * rows, solver, integration) - zero unless the library was built with -DHSRB_PHASE_CLOCKS. */
 int hsrb_stats(hsrb_t* h, int64_t* out16_host, void* stream);
 
-/* Introspection used by bench.py: lanes per env, shared-memory bytes per env, resident envs per SM, grid,
- * path (1 general, 2 fast), threads per block. */
+/* Introspection used by bench.py, for the kernel the next hsrb_step would launch: lanes per env, shared-memory bytes
+ * per env, resident envs per SM, grid, path (1 general kernel, 2 8-lane lock-step kernel, 3 warp-per-environment
+ * kernel: the codes hsrb_set_path returns), threads per block.  Fails where that hsrb_step would fail to launch. */
 int hsrb_launch_info(hsrb_t* h, int* out6_host);
 
 /* Measurement aid of bench.py (no reference counterpart): the device's FP32 FMA-loop peak in TFLOP/s (8 independent FMA
