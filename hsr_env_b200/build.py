@@ -13,8 +13,10 @@ from pathlib import Path
 
 CSRC = Path(__file__).resolve().parent / "csrc"
 LIB = CSRC / "libhsrb.so"
-TUS = ["hsrb_api.cu", "hsrb_push.cu", "hsrb_wpe.cu", "hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu", "hsrb_episode.cu"]
-HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "hsrb_episode.cuh", "../../include/hsrb.h"]
+TUS = ["hsrb_api.cu", "hsrb_push.cu", "hsrb_wpe.cu", "hsrb_wpe_params.cu", "hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu", "hsrb_episode.cu",
+       "hsrb_step_g4_params.cu", "hsrb_step_g8_params.cu", "hsrb_step_g16_params.cu", "hsrb_step_g32_params.cu",
+       "hsrb_step_lock_params.cu"]
+HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "hsrb_wpe_kernel.cuh", "hsrb_episode.cuh", "../../include/hsrb.h"]
 # per-TU flags: the fast-path kernel uses the 2-ulp fp32 division / square root (MUFU.RCP / MUFU.RSQ sequences without
 # the IEEE fix-up path; measured +6 % substeps/s, one-step error vs the fp64 oracle unchanged at the 1e-7 level); the
 # general kernel and the reset / forward paths keep IEEE division.
@@ -22,6 +24,8 @@ TU_FLAGS = {"hsrb_push.cu": ([] if os.environ.get("HSRB_PRECISE_DIV") else ["--p
             + os.environ.get("NVCC_PUSH_EXTRA", "").split()}
 TU_FLAGS["hsrb_wpe.cu"] = ([] if os.environ.get("HSRB_PRECISE_DIV") else ["--prec-div=false", "--prec-sqrt=false"]) \
     + os.environ.get("NVCC_WPE_EXTRA", "").split()
+# the instance with per-environment parameters: same flags as the instances without
+TU_FLAGS["hsrb_wpe_params.cu"] = TU_FLAGS["hsrb_wpe.cu"]
 for _g in (4, 8, 16, 32):
     TU_FLAGS[f"hsrb_step_g{_g}.cu"] = os.environ.get("NVCC_STEP_EXTRA", "").split()
 # the episode kernel resets environments with the stages of the lean reset instance above: same (IEEE) flags, same bits
@@ -29,6 +33,9 @@ TU_FLAGS["hsrb_episode.cu"] = TU_FLAGS["hsrb_step_g8.cu"]
 # the phase-locked general kernel takes the same 2-ulp fp32 division / square root as the block-push kernels
 TU_FLAGS["hsrb_step_lock.cu"] = ([] if os.environ.get("HSRB_PRECISE_DIV") else ["--prec-div=false", "--prec-sqrt=false"]) \
     + os.environ.get("NVCC_STEP_EXTRA", "").split()
+# the instances with per-environment parameters: the flags of the instances without
+for _tu in ("hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu"):
+    TU_FLAGS[_tu.replace(".cu", "_params.cu")] = TU_FLAGS[_tu]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr", "-Xptxas", "-v"]

@@ -59,6 +59,63 @@ template <> struct Lim<double> {
   HSR_HD static double minval() { return 1e-15; }
 };
 
+// ------------------------------------------------------------------------------------------------ per-environment parameters
+// Multipliers of model constants (DESIGN 4.3b), applied once where the constant is read, as a rounded product that no later
+// multiply-add absorbs: a scale of 1 reads the model's bits, a power of two reads the bits of a model whose arrays were scaled.
+//   [PRM_FRICTION] pair_friction (all five), [PRM_BLOCK_MASS] body_mass and body_inertia of the bodies in block_body,
+//   [PRM_GAIN] act_kp, [PRM_DAMPING] dof_damping.
+// The stages take the policy as a template argument: NoScale (the default) reads the model as it is and compiles to the
+// code without parameters; EnvScale holds one environment's multipliers.
+enum { PRM_FRICTION = 0, PRM_BLOCK_MASS, PRM_GAIN, PRM_DAMPING, PRM_COUNT };
+HSR_HD float mul_rn(float v, float s) {
+#if defined(__CUDA_ARCH__)
+  return __fmul_rn(v, s);
+#else
+  volatile float p = v * s;   // stored: never contracted into a later multiply-add
+  return p;
+#endif
+}
+HSR_HD double mul_rn(double v, double s) {
+#if defined(__CUDA_ARCH__)
+  return __dmul_rn(v, s);
+#else
+  volatile double p = v * s;
+  return p;
+#endif
+}
+struct NoScale {
+  template <typename T> HSR_HD const T* friction(const T* f, T*) const { return f; }
+  template <typename T> HSR_HD T block(const ModelT<T>&, int, T v) const { return v; }
+  template <typename T> HSR_HD const T* inertia(const ModelT<T>& m, int b, T*) const { return m.body_inertia + 6 * b; }
+  template <typename T> HSR_HD T gain(T v) const { return v; }
+  template <typename T> HSR_HD T damping(T v) const { return v; }
+  HSR_HD float scale(int) const { return 1.f; }
+  HSR_HD void unit(int) {}
+};
+struct EnvScale {
+  float s[PRM_COUNT];
+  // the five coefficients of a pair, scaled into buf
+  template <typename T> HSR_HD const T* friction(const T* f, T* buf) const {
+    for (int k = 0; k < 5; k++) buf[k] = mul_rn(f[k], (T)s[PRM_FRICTION]);
+    return buf;
+  }
+  // a mass or inertia entry of body b
+  template <typename T> HSR_HD T block(const ModelT<T>& m, int b, T v) const {
+    for (int k = 0; k < m.nblock; k++)
+      if (m.block_body[k] == b) return mul_rn(v, (T)s[PRM_BLOCK_MASS]);
+    return v;
+  }
+  // the six inertia entries of body b, scaled into buf
+  template <typename T> HSR_HD const T* inertia(const ModelT<T>& m, int b, T* buf) const {
+    for (int k = 0; k < 6; k++) buf[k] = block(m, b, m.body_inertia[6 * b + k]);
+    return buf;
+  }
+  template <typename T> HSR_HD T gain(T v) const { return mul_rn(v, (T)s[PRM_GAIN]); }
+  template <typename T> HSR_HD T damping(T v) const { return mul_rn(v, (T)s[PRM_DAMPING]); }
+  HSR_HD float scale(int k) const { return s[k]; }
+  HSR_HD void unit(int k) { s[k] = 1.f; }
+};
+
 enum { FLAG_CON_OVERFLOW = 1, FLAG_BAD_NUM = 2, FLAG_CHOL = 4 };
 enum { WI_NCON = 0, WI_NEFC = 1, WI_NLIMIT = 2, WI_FLAGS = 3, WI_ITER = 4, WI_NARROW = 5, WI_LSEVAL = 6, WI_KFLOP = 7,
        WI_SUMCON = 8, WI_SUMEFC = 9, WI_NPFLOP = 10, WI_TLAST = 11, WI_PHASE0 = 12, WI_COUNT = 20 };
@@ -292,8 +349,8 @@ HSR_HD void kinematics_trig(const ModelT<T>& m, WS<T>& w, const Grp& g) {
   g.sync();
 }
 
-template <typename T>
-HSR_HDC void kinematics_lane0(const ModelT<T>& m, WS<T>& w) {
+template <typename T, typename Sc = NoScale>
+HSR_HDC void kinematics_lane0(const ModelT<T>& m, WS<T>& w, const Sc& sc = Sc()) {
   // world
   for (int k = 0; k < 3; k++) { w.xpos[k] = 0; w.xipos[k] = 0; }
   for (int k = 0; k < 9; k++) w.xmat[k] = (k % 4 == 0) ? GT(1) : GT(0);
@@ -351,7 +408,7 @@ HSR_HDC void kinematics_lane0(const ModelT<T>& m, WS<T>& w) {
     V3<GT> acc = mk<GT>(0, 0, 0);
     GT mt = 0;
     for (int b = r; b < m.nbody; b++)
-      if (m.body_root[b] == r) { acc = acc + ld3(w.xipos + 3 * b) * (GT)m.body_mass[b]; mt += (GT)m.body_mass[b]; }
+      if (m.body_root[b] == r) { acc = acc + ld3(w.xipos + 3 * b) * (GT)sc.block(m, b, m.body_mass[b]); mt += (GT)sc.block(m, b, m.body_mass[b]); }
     if (mt > 0) acc = acc * (GT(1) / mt);
     for (int b = r; b < m.nbody; b++)
       if (m.body_root[b] == r) st3(w.com + 3 * b, acc);
@@ -362,12 +419,13 @@ HSR_HDC void kinematics_lane0(const ModelT<T>& m, WS<T>& w) {
     V3<T> c = cvt<T>(ld3(w.xipos + 3 * b) - ld3(w.com + 3 * b));
     T Rt_[9];
     for (int k = 0; k < 9; k++) Rt_[k] = (T)R[k];
-    const T* ib = m.body_inertia + 6 * b;
+    T ibuf[6];
+    const T* ib = sc.inertia(m, b, ibuf);
     T Ib[9] = {ib[0], ib[3], ib[4], ib[3], ib[1], ib[5], ib[4], ib[5], ib[2]};
     T tmp[9], Iw[9], Rt[9];
     for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) Rt[3 * i + j] = Rt_[3 * j + i];
     mulm(Rt_, Ib, tmp); mulm(tmp, Rt, Iw);
-    T mass = m.body_mass[b];
+    T mass = sc.block(m, b, m.body_mass[b]);
     T cc = dot(c, c);
     T* I = w.binert + 10 * b;
     I[0] = Iw[0] + mass * (cc - c.x * c.x); I[1] = Iw[4] + mass * (cc - c.y * c.y); I[2] = Iw[8] + mass * (cc - c.z * c.z);
@@ -570,8 +628,8 @@ template <typename T> HSR_HD void cross_force(const T* v, const T* f, T* r) {
 }
 
 // lane 0: RNE bias, passive, actuation -> qfrc_smooth
-template <typename T>
-HSR_HDC void smooth_lane0(const ModelT<T>& m, WS<T>& w) {
+template <typename T, typename Sc = NoScale>
+HSR_HDC void smooth_lane0(const ModelT<T>& m, WS<T>& w, const Sc& sc = Sc()) {
   int nv = m.nv;
   T (*cvel)[6] = reinterpret_cast<T(*)[6]>(w.cvel);
   T (*cacc)[6] = reinterpret_cast<T(*)[6]>(w.cacc);
@@ -611,12 +669,12 @@ HSR_HDC void smooth_lane0(const ModelT<T>& m, WS<T>& w) {
     const T* c = w.cdof + 6 * i;
     const T* f = cfrc[m.dof_body[i]];
     T bias = c[0] * f[0] + c[1] * f[1] + c[2] * f[2] + c[3] * f[3] + c[4] * f[4] + c[5] * f[5];
-    w.qfrc_smooth[i] = -m.dof_damping[i] * w.qvel[i] - bias;
+    w.qfrc_smooth[i] = -sc.damping(m.dof_damping[i]) * w.qvel[i] - bias;
   }
   for (int a = 0; a < m.nu; a++) {
     T c = w.ctrl[a];
     if (m.act_ctrllimited[a]) c = fmin(fmax(c, m.act_ctrlrange[2 * a]), m.act_ctrlrange[2 * a + 1]);
-    T f = m.act_kp[a] * c - m.act_kp[a] * m.act_gear[a] * w.qpos[m.act_qposadr[a]];
+    T f = sc.gain(m.act_kp[a]) * c - sc.gain(m.act_kp[a]) * m.act_gear[a] * w.qpos[m.act_qposadr[a]];
     if (m.act_forcelimited[a]) f = fmin(fmax(f, m.act_forcerange[2 * a]), m.act_forcerange[2 * a + 1]);
     w.qfrc_smooth[m.act_dof[a]] += m.act_gear[a] * f;
   }
@@ -1227,8 +1285,8 @@ HSR_HDC void row_params(const ModelT<T>& m, const T* solref, const T* solimp, T 
 }
 
 // rows: active joint limits (joint order) then contacts (elliptic, dim rows each)
-template <typename T, typename Grp>
-HSR_HDC void make_constraint(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC void make_constraint(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, const Sc& sc = Sc()) {
   int nv = m.nv;
   // limit rows (recomputed by every lane; lane 0 writes)
   if (g.lane == 0) {
@@ -1272,7 +1330,8 @@ HSR_HDC void make_constraint(const ModelT<T>& m, WS<T>& w, const Grp& g, int nli
   for (int c = g.lane; c < ncon; c += Grp::G) {
     int pk = w.con_pair[c];
     int dim = m.pair_condim[pk], r0 = w.con_adr[c];
-    const T* fri = m.pair_friction + 5 * pk;
+    T fbuf[5];
+    const T* fri = sc.friction(m.pair_friction + 5 * pk, fbuf);
     T diag = m.geom_invweight[m.pair_geom1[pk]] + m.geom_invweight[m.pair_geom2[pk]];
     GT R0 = 0;
     for (int r = 0; r < dim; r++) {
@@ -1309,8 +1368,8 @@ HSR_HD int cone_zone(const T* x, int dim, T mu, const T* fri, T& N, T& Tn) {
 //   cone zone (U_a = jar_a s_a, u = U / T, s_0 = mu, s_a = fri_a-1, k = mu (N - mu T) / T):
 //       Dm (p p^T + k q q^T) - Dm k sum_{a>=1} s_a^2 J_a J_a^T,  p = mu J_0 - mu sum_{a>=1} u_a s_a J_a,  q = sum_{a>=1} u_a s_a J_a
 //   i.e. the 6x6 cone block Dm S (v v^T - k (I_t - u u^T)) S of the row formulation, v = e_0 - mu u, never formed.
-template <typename T, typename Grp>
-HSR_HDC T constraint_update(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, bool full) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC T constraint_update(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, bool full, const Sc& sc = Sc()) {
   int nv = m.nv;
   T cost = 0;
   for (int i = g.lane; i < nlimit; i += Grp::G) {
@@ -1325,7 +1384,8 @@ HSR_HDC T constraint_update(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlim
   for (int c = g.lane; c < ncon; c += Grp::G) {
     int pk = w.con_pair[c];
     int dim = m.pair_condim[pk], r0 = w.con_adr[c];
-    const T* fri = m.pair_friction + 5 * pk;
+    T fbuf[5];
+    const T* fri = sc.friction(m.pair_friction + 5 * pk, fbuf);
     T mu = w.con_mu[c];
     const T* x = w.jar + r0;
     T N, Tn;
@@ -1431,8 +1491,8 @@ HSR_HDC void ls_eval(const ModelT<T>& m, const WS<T>& w, const Grp& g, int nlimi
 }
 
 // exact line search along w.search (safeguarded Newton on the 1-D derivative with bracketing)
-template <typename T, typename Grp>
-HSR_HDC T linesearch(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, T gtol) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC T linesearch(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, T gtol, const Sc& sc = Sc()) {
   int nv = m.nv;
   T a1 = 0, a2 = 0;
   for (int i = g.lane; i < nv; i += Grp::G) {
@@ -1443,7 +1503,8 @@ HSR_HDC T linesearch(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int
   for (int c = g.lane; c < ncon; c += Grp::G) {
     int pk = w.con_pair[c];
     int dim = m.pair_condim[pk], r0 = w.con_adr[c];
-    const T* fri = m.pair_friction + 5 * pk;
+    T fbuf[5];
+    const T* fri = sc.friction(m.pair_friction + 5 * pk, fbuf);
     T mu = w.con_mu[c];
     T* q = w.lsq + HSR_LSQ * c;
     T uu = 0, uv = 0, vv = 0, Q0 = 0, Q1 = 0, Q2 = 0;
@@ -1493,8 +1554,9 @@ HSR_HDC T linesearch(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int
 // block vote per pass keeps every warp of the block in the same code region) can drive the loop itself:
 //   newton_begin (warm start, cost of the starting point) -> while (newton_pass) -> newton_end (J^T f, counters).
 template <typename T> struct NewtonState { T cost, scale; int it; };
-template <typename T, typename Grp>
-HSR_HDC bool newton_begin(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc, NewtonState<T>& ns) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC bool newton_begin(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc, NewtonState<T>& ns,
+                          const Sc& sc = Sc()) {
   int nv = m.nv;
   ns.it = 0; ns.cost = 0; ns.scale = T(1) / (m.meaninertia * T(nv > 1 ? nv : 1));
   if (nefc == 0) {
@@ -1505,23 +1567,24 @@ HSR_HDC bool newton_begin(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit
   // warm start: lower cost of qacc_warmstart / qacc_smooth
   T gw = residuals(m, w, g, w.warm, nefc);
   g.sync();
-  T cw = constraint_update(m, w, g, nlimit, ncon, false) + gw;
+  T cw = constraint_update(m, w, g, nlimit, ncon, false, sc) + gw;
   g.sync();
   T gs = residuals(m, w, g, w.qacc_smooth, nefc);
   g.sync();
-  T cs = constraint_update(m, w, g, nlimit, ncon, false) + gs;
+  T cs = constraint_update(m, w, g, nlimit, ncon, false, sc) + gs;
   bool use_warm = cw <= cs;
   for (int i = g.lane; i < nv; i += Grp::G) w.qacc[i] = use_warm ? w.warm[i] : w.qacc_smooth[i];
   g.sync();
   T gauss = use_warm ? residuals(m, w, g, w.qacc, nefc) : gs;
   g.sync();
-  ns.cost = constraint_update(m, w, g, nlimit, ncon, true) + gauss;
+  ns.cost = constraint_update(m, w, g, nlimit, ncon, true, sc) + gauss;
   g.sync();
   return true;
 }
 // one pass: gradient, convergence tests, Hessian, Newton direction, line search, update; false = the solver has stopped
-template <typename T, typename Grp>
-HSR_HDC bool newton_pass(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc, NewtonState<T>& ns) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC bool newton_pass(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc, NewtonState<T>& ns,
+                         const Sc& sc = Sc()) {
   const int nv = m.nv;
   const T scale = ns.scale;
   {
@@ -1575,7 +1638,7 @@ HSR_HDC bool newton_pass(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit,
     }
     g.sync();
     T gtol = m.tolerance * m.ls_tolerance * sn / scale;
-    T alpha = linesearch(m, w, g, nlimit, ncon, gtol);
+    T alpha = linesearch(m, w, g, nlimit, ncon, gtol, sc);
     if (alpha == 0) return false;
     T gsum = 0;
     for (int i = g.lane; i < nv; i += Grp::G) {
@@ -1586,7 +1649,7 @@ HSR_HDC bool newton_pass(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit,
     gsum = g.sum(gsum);
     g.sync();
     T old = ns.cost;
-    ns.cost = constraint_update(m, w, g, nlimit, ncon, true) + gsum;
+    ns.cost = constraint_update(m, w, g, nlimit, ncon, true, sc) + gsum;
     g.sync();
     ns.it++;
     // improvement of this step.  The reference tests old - cost; in fp32 that difference of two large numbers
@@ -1609,23 +1672,23 @@ HSR_HDC void newton_end(const ModelT<T>& m, WS<T>& w, const Grp& g, int nefc, co
   if (g.lane == 0) w.wi[WI_ITER] += ns.it;
   g.sync();
 }
-template <typename T, typename Grp>
-HSR_HDC void solve_newton(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC void solve_newton(const ModelT<T>& m, WS<T>& w, const Grp& g, int nlimit, int ncon, int nefc, const Sc& sc = Sc()) {
   NewtonState<T> ns;
-  if (!newton_begin(m, w, g, nlimit, ncon, nefc, ns)) return;
-  while (newton_pass(m, w, g, nlimit, ncon, nefc, ns)) {}
+  if (!newton_begin(m, w, g, nlimit, ncon, nefc, ns, sc)) return;
+  while (newton_pass(m, w, g, nlimit, ncon, nefc, ns, sc)) {}
   newton_end(m, w, g, nefc, ns);
 }
 
 // ------------------------------------------------------------------------------------------------ B.8 Euler
 // qacc_int = (M + dt*diag(damping))^-1 (qfrc_smooth + qfrc_constraint) -> w.grad, rows across the lanes of the group
-template <typename T, typename Grp>
-HSR_HD void euler_solve(const ModelT<T>& m, WS<T>& w, const Grp& g) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HD void euler_solve(const ModelT<T>& m, WS<T>& w, const Grp& g, const Sc& sc = Sc()) {
   const int nv = m.nv;
   const T dt = m.timestep;
   T* x = w.grad;  // scratch
   if (m.any_damping) {
-    for (int k = g.lane; k < nv * nv; k += Grp::G) { const int i = k / nv; w.H[k] = w.M[k] + ((k - i * nv == i) ? dt * m.dof_damping[i] : T(0)); }
+    for (int k = g.lane; k < nv * nv; k += Grp::G) { const int i = k / nv; w.H[k] = w.M[k] + ((k - i * nv == i) ? dt * sc.damping(m.dof_damping[i]) : T(0)); }
     for (int i = g.lane; i < nv; i += Grp::G) x[i] = w.qfrc_smooth[i] + w.tmpv[i];
     g.sync();
     if (!chol_factor_g(w.H, nv, w.invd, g) && g.lane == 0) w.wi[WI_FLAGS] |= FLAG_CHOL;
@@ -1700,11 +1763,11 @@ HSR_HDC int algorithmic_flops(const ModelT<T>& m, int nc, int ne, int it, int ls
 }
 
 // mj_forward up to and including the constraint solve (sim.forward(), /root/reference/hsr/env.py:176)
-template <typename T, typename Grp>
-HSR_HDC void forward(const ModelT<T>& m, WS<T>& w, const Grp& g) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HDC void forward(const ModelT<T>& m, WS<T>& w, const Grp& g, const Sc& sc = Sc()) {
   HSR_PHASE_START(w, g);
   kinematics_trig(m, w, g);
-  if (g.lane == 0) kinematics_lane0(m, w);
+  if (g.lane == 0) kinematics_lane0(m, w, sc);
   g.sync();
   HSR_PHASE(w, g, PH_KIN);
   cdof_geoms(m, w, g);
@@ -1712,7 +1775,7 @@ HSR_HDC void forward(const ModelT<T>& m, WS<T>& w, const Grp& g) {
   mass_matrix(m, w, g);
   g.sync();
   HSR_PHASE(w, g, PH_CRB);
-  if (g.lane == 0) smooth_lane0(m, w);
+  if (g.lane == 0) smooth_lane0(m, w, sc);
   g.sync();
   smooth_solve(m, w, g);
   HSR_PHASE(w, g, PH_SMOOTH);
@@ -1728,13 +1791,13 @@ HSR_HDC void forward(const ModelT<T>& m, WS<T>& w, const Grp& g) {
   int ncon = collision(m, w, g, nrow);
   g.sync();
   HSR_PHASE(w, g, PH_COLLIDE);
-  make_constraint(m, w, g, nlimit, ncon);
+  make_constraint(m, w, g, nlimit, ncon, sc);
   int it0 = w.wi[WI_ITER], ls0 = w.wi[WI_LSEVAL];
   g.sync();
   if (g.lane == 0) { w.wi[WI_NCON] = ncon; w.wi[WI_NEFC] = nrow; w.wi[WI_NLIMIT] = nlimit; }
   g.sync();
   HSR_PHASE(w, g, PH_ROWS);
-  solve_newton(m, w, g, nlimit, ncon, nrow);
+  solve_newton(m, w, g, nlimit, ncon, nrow, sc);
   HSR_PHASE(w, g, PH_SOLVE);
   if (g.lane == 0) {
     w.wi[WI_SUMCON] += ncon; w.wi[WI_SUMEFC] += nrow;
@@ -1744,10 +1807,10 @@ HSR_HDC void forward(const ModelT<T>& m, WS<T>& w, const Grp& g) {
 }
 
 // mj_step (sim.step(), /root/reference/hsr/env.py:123)
-template <typename T, typename Grp>
-HSR_HD void substep(const ModelT<T>& m, WS<T>& w, const Grp& g) {
-  forward(m, w, g);
-  euler_solve(m, w, g);
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HD void substep(const ModelT<T>& m, WS<T>& w, const Grp& g, const Sc& sc = Sc()) {
+  forward(m, w, g, sc);
+  euler_solve(m, w, g, sc);
   if (g.lane == 0) euler_lane0(m, w);
   g.sync();
   HSR_PHASE(w, g, PH_EULER);
@@ -1787,12 +1850,13 @@ HSR_HD bool goal_reached(const ModelT<T>& m, const EnvCfg<T>& cfg, const WS<T>& 
 
 // HSREnv.step inner loop (/root/reference/hsr/env.py:118-131): up to nsub substeps, goal test after every
 // substep, freeze at the first success.  Returns the number of substeps executed.
-template <typename T, typename Grp>
-HSR_HD int env_action(const ModelT<T>& m, const EnvCfg<T>& cfg, WS<T>& w, const Grp& g, int nsub, bool& success) {
+template <typename T, typename Grp, typename Sc = NoScale>
+HSR_HD int env_action(const ModelT<T>& m, const EnvCfg<T>& cfg, WS<T>& w, const Grp& g, int nsub, bool& success,
+                      const Sc& sc = Sc()) {
   int taken = 0;
   success = false;
   for (int s = 0; s < nsub; s++) {
-    substep(m, w, g);
+    substep(m, w, g, sc);
     taken++;
     if (goal_reached(m, cfg, w)) { success = true; break; }
   }
@@ -1901,6 +1965,14 @@ HSR_HDC void reset_lane0(const ModelT<T>& m, const EnvCfg<T>& cfg, WS<T>& w, uin
       w.qpos[a + k] = (T)uniform32(r[k & 3], (float)cfg.start_lo[s][k], (float)cfg.start_hi[s][k]);
     }
   }
+}
+
+// The per-environment multipliers (PRM_*) a reset draws when the handle has parameter ranges: U[lo, hi) from draw block
+// 8192 of the same stream as reset_lane0 (same key, same episode), which reset_lane0 never reads.
+HSR_HD void sample_env_params(const float* lo, const float* hi, uint64_t seed, uint32_t env_id, uint32_t episode, float* out) {
+  uint32_t r[4];
+  philox4x32_10(episode, 8192, (uint32_t)(seed >> 32), 0, (uint32_t)seed, env_id, r);
+  for (int k = 0; k < PRM_COUNT; k++) out[k] = uniform32(r[k], lo[k], hi[k]);
 }
 
 }  // namespace hsr

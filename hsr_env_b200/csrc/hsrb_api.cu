@@ -10,6 +10,7 @@
 #include <cuda_runtime.h>
 #include <cub/device/device_radix_sort.cuh>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstdio>
@@ -117,6 +118,33 @@ struct EpisodeBufs {
   }
 };
 
+__global__ void fill_f32(float* p, size_t n, float v) {
+  const size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+  if (i < n) p[i] = v;
+}
+
+// Per-environment parameters (hsrb_set_env_params, hsrb_set_env_param_ranges), allocated on first use.  A handle that
+// never calls those functions launches the instances without parameters.
+struct ParamBufs {
+  float* d = nullptr;        // [N, PRM_COUNT] multipliers, 1.0 until set or drawn
+  bool on = false;           // STEP / DEBUG launches pass d: the instances with parameters
+  bool draw = false;         // resets redraw the reset environments' rows ~ U[lo, hi)
+  float lo[PRM_COUNT], hi[PRM_COUNT];
+  int alloc(int n, cudaStream_t s) {
+    if (d) return 0;
+    const size_t cnt = (size_t)n * PRM_COUNT;
+    CU(cudaMalloc(&d, sizeof(float) * cnt));
+    return nominal(n, s);
+  }
+  int nominal(int n, cudaStream_t s) {
+    const size_t cnt = (size_t)n * PRM_COUNT;
+    fill_f32<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(d, cnt, 1.f);
+    CU(cudaGetLastError());
+    return 0;
+  }
+  void free() { cudaFree(d); }
+};
+
 // The action kernels.  K_GENERAL (hsrb_step_kernel<G>) also runs every reset, forward and debug launch; the others
 // run STEP launches only.  A new kernel is one more entry here, its configure_* function and one line in select().
 enum Kernel { K_GENERAL, K_LOCK, K_PUSH, K_WPE, K_COUNT };
@@ -147,6 +175,7 @@ struct hsrb {
   char fast_why[128] = "";
   SortBufs sort;
   EpisodeBufs ep;
+  ParamBufs prm;
   // scratch for the host-buffer entry point
   float *d_ctrl = nullptr, *d_obs = nullptr, *d_reward = nullptr;
   unsigned char* d_done = nullptr;
@@ -159,11 +188,14 @@ namespace {
 // only (one block against the goal point); among them, auto (path 0) and path 3 take the warp-per-environment kernel,
 // phase-locked, two teams per block - measured on B200, round 2, TimeLimit workload: 48.4 M substeps/s at 4096 envs
 // (lock-step 8-lane kernel 34.6 M, free-running warps 32.9 M), 65.8 M at 131072 envs (52.3 M / 53.2 M).  A goal list
-// under path 3 runs the general kernel; under path 2 it is an error.
+// under path 3 runs the general kernel; under path 2 it is an error.  Per-environment parameters (hsrb_set_env_params) have
+// instances in every kernel but the lock-step 8-lane one: under path 2 they are an error as well.
 int select(const hsrb* h, Kernel* k) {
   const bool fast = h->fast_ok && h->path != 1 && h->cfg.ngoal == 0;
   if (fast && h->wpe_ok && h->path != 2) *k = K_WPE;
-  else if (fast) *k = K_PUSH;
+  else if (fast && h->prm.on && h->path == 2)
+    return fail(-3, "per-environment parameters are not available in the lock-step fast kernel (path 2, kernel='lockstep')");
+  else if (fast && !h->prm.on) *k = K_PUSH;
   else if (h->path == 2) return fail(-3, "fast path not available for this model: %s", h->fast_why);
   else if (h->knobs.general_lock && h->hm.m.npair <= 256 && !h->lanes_req) *k = K_LOCK;
   else *k = K_GENERAL;
@@ -316,6 +348,10 @@ KArgs base_args(hsrb* h) {
   a.m = h->dm; a.cfg = h->cfg; a.n = h->n; a.S = h->S;
   a.seed = h->seed; a.env_off = h->env_off; a.state = h->d_state; a.episode = h->d_episode; a.stats = h->d_stats;
   a.opts = h->knobs.opts;
+  if (h->prm.on) {
+    a.params = h->prm.d; a.prm_draw = h->prm.draw;
+    for (int k = 0; k < PRM_COUNT; k++) { a.prm_lo[k] = h->prm.lo[k]; a.prm_hi[k] = h->prm.hi[k]; }
+  }
   return a;
 }
 
@@ -606,6 +642,7 @@ int hsrb_destroy(hsrb_t* h) {
   cudaFree(h->d_ctrl); cudaFree(h->d_obs); cudaFree(h->d_reward); cudaFree(h->d_done); cudaFree(h->d_taken);
   h->sort.free();
   h->ep.free();
+  h->prm.free();
   delete h;
   return 0;
 }
@@ -698,6 +735,56 @@ extern "C" int hsrb_debug_work(hsrb_t* h, int* out_host) {
   return cudaMemcpy(out_host, h->sort.work, sizeof(int) * (size_t)h->n, cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : -2;
 }
 #endif
+
+int hsrb_set_env_params(hsrb_t* h, const float* params, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  CU(cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!params) {   // nominal model, no ranges, the instances without parameters
+    h->prm.on = false; h->prm.draw = false;
+    return h->prm.d ? h->prm.nominal(h->n, s) : 0;
+  }
+  int rc = h->prm.alloc(h->n, s);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(h->prm.d, params, sizeof(float) * (size_t)h->n * PRM_COUNT, cudaMemcpyDeviceToDevice, s));
+  h->prm.on = true;
+  return 0;
+}
+
+int hsrb_get_env_params(hsrb_t* h, float* params, void* stream) {
+  if (!h || !params) return fail(-1, "bad arguments");
+  CU(cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t cnt = (size_t)h->n * PRM_COUNT;
+  if (h->prm.d) CU(cudaMemcpyAsync(params, h->prm.d, sizeof(float) * cnt, cudaMemcpyDeviceToDevice, s));
+  else {
+    fill_f32<<<(unsigned)((cnt + 255) / 256), 256, 0, s>>>(params, cnt, 1.f);
+    CU(cudaGetLastError());
+  }
+  return 0;
+}
+
+int hsrb_set_env_param_ranges(hsrb_t* h, const float* lo_host, const float* hi_host) {
+  if (!h) return fail(-1, "null handle");
+  if (!lo_host != !hi_host) return fail(-1, "lo and hi must both be given or both be NULL");
+  if (!lo_host) { h->prm.draw = false; return 0; }   // parameters persist across resets
+  static const char* const names[PRM_COUNT] = {"friction", "block_mass", "actuator_gain", "damping"};
+  for (int k = 0; k < PRM_COUNT; k++) {
+    const float lo = lo_host[k], hi = hi_host[k];
+    const bool positive = k == PRM_FRICTION || k == PRM_BLOCK_MASS;   // > 0; gain and damping >= 0
+    if (!std::isfinite(lo) || !std::isfinite(hi) || !(lo <= hi) || (positive ? !(lo > 0.f) : !(lo >= 0.f)))
+      return fail(-1, "%s range [%g, %g]: needs finite lo <= hi with lo %s 0", names[k], (double)lo, (double)hi, positive ? ">" : ">=");
+  }
+  CU(cudaSetDevice(h->device));
+  if (!h->prm.d) {   // first use: filled with 1.0 before any stream of the caller's can read it
+    int rc = h->prm.alloc(h->n, nullptr);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(nullptr));
+  }
+  for (int k = 0; k < PRM_COUNT; k++) { h->prm.lo[k] = lo_host[k]; h->prm.hi[k] = hi_host[k]; }
+  h->prm.draw = true; h->prm.on = true;
+  return 0;
+}
 
 int hsrb_reset(hsrb_t* h, const uint8_t* mask, float* obs, void* stream) {
   if (!h) return fail(-1, "null handle");

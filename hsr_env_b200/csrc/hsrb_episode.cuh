@@ -6,7 +6,8 @@
 // reward go to ep_length / ep_return where done; the cumulative counters (EP_*) are warp-aggregated.  With autoreset the
 // done environments are reset in the same launch with the stages MODE_RESET of hsrb_step_kernel runs (reset_lane0,
 // kinematics_trig, kinematics_lane0, between load_state and store_state): the same Philox draw as hsrb_reset(mask =
-// done), so both loops give the same bits.  Environments that are not reset load and store no state.
+// done), so both loops give the same bits, parameter draws included.  Environments that are not reset load and store no
+// state.
 //
 // Layout: the lean launch of the general path (configure() in hsrb_api.cu): G lanes per environment, one warp per block,
 // 32 / G workspaces of ws_bytes in shared memory (only the reset stages use them), a grid-stride loop.
@@ -81,6 +82,7 @@ __global__ void __launch_bounds__(32) hsrb_episode_kernel(const __grid_constant_
         const unsigned ep = k.episode[env];
         k.episode[env] = ep + 1;
         reset_lane0(k.m, k.cfg, w, k.seed, (uint32_t)(k.env_off + (unsigned long long)env), ep);
+        reset_params(k, env, ep);
       }
       g.sync();
       kinematics_trig(k.m, w, g);

@@ -39,7 +39,26 @@ struct KArgs {
   unsigned long long* stats;
   const int* order;        // wpe kernel: environment of launch slot r (heaviest first), or null = identity
   int* work;               // wpe kernel: [N] work estimate of this action per environment (the next launch's sort key)
+  // per-environment parameters (hsrb_set_env_params): [N, PRM_COUNT] multipliers, or null: the model as it is, and the
+  // instances without parameters.  prm_draw: resets redraw the reset environments' rows ~ U[prm_lo, prm_hi)
+  float* params;
+  int prm_draw;
+  float prm_lo[PRM_COUNT], prm_hi[PRM_COUNT];
 };
+
+// the scale policy of an instance (hsr_core.h): PARAMS = false reads the model as it is
+template <bool PARAMS> struct ScaleOf { typedef NoScale type; };
+template <> struct ScaleOf<true> { typedef EnvScale type; };
+__device__ __forceinline__ void load_scale(NoScale&, const KArgs&, int) {}
+__device__ __forceinline__ void load_scale(EnvScale& sc, const KArgs& a, int env) {
+  for (int k = 0; k < PRM_COUNT; k++) sc.s[k] = a.params[(size_t)env * PRM_COUNT + k];
+}
+// lane 0 of a reset: the environment's parameter draw (hsr_core.h sample_env_params), same key and episode as reset_lane0
+__device__ __forceinline__ void reset_params(const KArgs& a, int env, unsigned ep) {
+  if (a.prm_draw)
+    sample_env_params(a.prm_lo, a.prm_hi, a.seed, (uint32_t)(a.env_off + (unsigned long long)env), ep,
+                      a.params + (size_t)env * PRM_COUNT);
+}
 
 enum { MODE_STEP = 0, MODE_DEBUG = 1, MODE_FORWARD = 2, MODE_RESET = 3 };
 
@@ -64,7 +83,8 @@ __device__ __forceinline__ void store_state(const KArgs& a, WS<float>& w, const 
 // FULL = false: the same kernel without the STEP / DEBUG modes (reset and forward launches): a few KB of code instead of
 // several hundred, which matters when it runs between two action kernels on a cold L2 (bench.py flushes L2 between timed
 // steps: the masked reset through the full kernel's binary cost 1.4-2.6 ms of instruction fetch from DRAM, 0.03 ms warm).
-template <int G, bool FULL = true>
+// Only the lean instance draws parameters at reset.  PARAMS = true (FULL only): STEP / DEBUG with a.params.
+template <int G, bool FULL = true, bool PARAMS = false>
 __global__ void __launch_bounds__(32) hsrb_step_kernel(const __grid_constant__ KArgs a) {
   HSRB_DYN_SMEM(smem);
   DevGrp<G> g;
@@ -79,11 +99,13 @@ __global__ void __launch_bounds__(32) hsrb_step_kernel(const __grid_constant__ K
     g.sync();
     bool success = false;
     int taken = 0;
+    typename ScaleOf<PARAMS>::type sc;
+    load_scale(sc, a, env);
     if (FULL && a.mode == MODE_STEP) {
-      taken = env_action(a.m, a.cfg, w, g, a.nsub, success);
+      taken = env_action(a.m, a.cfg, w, g, a.nsub, success, sc);
     } else if (FULL && a.mode == MODE_DEBUG) {
-      forward(a.m, w, g);
-      euler_solve(a.m, w, g);
+      forward(a.m, w, g, sc);
+      euler_solve(a.m, w, g, sc);
       if (g.lane == 0) euler_lane0(a.m, w);
       g.sync();
       if (g.lane == 0) debug_dump(a.m, w, a.dump + (size_t)env * a.dump_stride);
@@ -97,6 +119,7 @@ __global__ void __launch_bounds__(32) hsrb_step_kernel(const __grid_constant__ K
           unsigned ep = a.episode[env];
           a.episode[env] = ep + 1;
           reset_lane0(a.m, a.cfg, w, a.seed, (uint32_t)(a.env_off + (unsigned long long)env), ep);
+          if (!FULL) reset_params(a, env, ep);
         }
         g.sync();
         kinematics_trig(a.m, w, g);
@@ -163,6 +186,7 @@ struct LockQueue {
 __host__ __device__ inline size_t lock_tail_bytes() { return sizeof(LockQueue) + 16; }
 
 #if defined(HSRB_STEP_LOCK_IMPL)   // defined by the translation unit that owns the kernel (hsrb_step_lock.cu, the emulated build)
+template <bool PARAMS = false>   // true: STEP launches with a.params
 __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel(const __grid_constant__ KArgs a) {
   HSRB_DYN_SMEM(smem);
   typedef DevGrp<32> Grp;
@@ -179,7 +203,9 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
   for (int env0 = blockIdx.x * wpb; env0 < a.n; env0 += gridDim.x * wpb) {
     const int env = env0 + wib;
     const bool valid = env < a.n;
+    typename ScaleOf<PARAMS>::type sc;
     if (valid) {
+      load_scale(sc, a, env);
       load_state<32>(a, w, g, env);
       for (int i = g.lane; i < m.nu; i += 32) w.ctrl[i] = a.ctrl ? a.ctrl[(size_t)env * m.nu + i] : 0.f;
     }
@@ -197,7 +223,7 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
       if (!finished) {
         HSR_PHASE_START(w, g);
         kinematics_trig(m, w, g);
-        if (g.lane == 0) kinematics_lane0(m, w);
+        if (g.lane == 0) kinematics_lane0(m, w, sc);
         g.sync();
         HSR_PHASE(w, g, PH_KIN);
       }
@@ -211,7 +237,7 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
       }
       if (PH) __syncthreads();
       if (!finished) {
-        if (g.lane == 0) smooth_lane0(m, w);
+        if (g.lane == 0) smooth_lane0(m, w, sc);
         g.sync();
         smooth_solve(m, w, g);
         HSR_PHASE(w, g, PH_SMOOTH);
@@ -279,7 +305,7 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
       }
       if (PH) __syncthreads();
       if (!finished) {
-        make_constraint(m, w, g, nlimit, ncon);
+        make_constraint(m, w, g, nlimit, ncon, sc);
         it0 = w.wi[WI_ITER]; ls0 = w.wi[WI_LSEVAL];
         g.sync();
         if (g.lane == 0) { w.wi[WI_NCON] = ncon; w.wi[WI_NEFC] = nrow; w.wi[WI_NLIMIT] = nlimit; }
@@ -289,14 +315,14 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
       if (PH) __syncthreads();
       if (PL) {
         NewtonState<float> ns;
-        bool act = !finished && newton_begin(m, w, g, nlimit, ncon, nrow, ns);
+        bool act = !finished && newton_begin(m, w, g, nlimit, ncon, nrow, ns, sc);
         const bool solved = act;
         while (__syncthreads_or(act)) {
-          if (act) act = newton_pass(m, w, g, nlimit, ncon, nrow, ns);
+          if (act) act = newton_pass(m, w, g, nlimit, ncon, nrow, ns, sc);
         }
         if (solved) newton_end(m, w, g, nrow, ns);
       } else if (!finished) {
-        solve_newton(m, w, g, nlimit, ncon, nrow);
+        solve_newton(m, w, g, nlimit, ncon, nrow, sc);
       }
       if (!finished) {
         HSR_PHASE(w, g, PH_SOLVE);
@@ -308,7 +334,7 @@ __global__ void __launch_bounds__(32 * HSRB_LOCK_MAXWARPS) hsrb_step_lock_kernel
       }
       __syncthreads();
       if (!finished) {
-        euler_solve(m, w, g);
+        euler_solve(m, w, g, sc);
         if (g.lane == 0) euler_lane0(m, w);
         g.sync();
         HSR_PHASE(w, g, PH_EULER);
@@ -363,22 +389,39 @@ struct Plan {
 
 cudaError_t hsrb_step_lock_prepare(const Plan& p, int* bps);
 cudaError_t hsrb_step_lock_launch(const Plan& p, const KArgs& a, cudaStream_t s);
+// the instances with per-environment parameters live in translation units of their own (hsrb_step_lock_params.cu,
+// hsrb_step_g*_params.cu): a function the two instances of one unit share is inlined differently than when one calls it
+cudaError_t hsrb_step_lock_params_prepare();
+cudaError_t hsrb_step_lock_params_launch(const Plan& p, const KArgs& a, cudaStream_t s);
 
 // per-G entry points of hsrb_step_kernel, one translation unit each (parallel compilation)
-#define HSRB_DECL_G(G)                                          \
-  cudaError_t hsrb_step##G##_prepare(const Plan& p, int* bps); \
-  cudaError_t hsrb_step##G##_launch(const Plan& p, const KArgs& a, cudaStream_t s);
+#define HSRB_DECL_G(G)                                                                    \
+  cudaError_t hsrb_step##G##_prepare(const Plan& p, int* bps);                           \
+  cudaError_t hsrb_step##G##_launch(const Plan& p, const KArgs& a, cudaStream_t s);      \
+  cudaError_t hsrb_step##G##_params_prepare();                                           \
+  cudaError_t hsrb_step##G##_params_launch(const Plan& p, const KArgs& a, cudaStream_t s);
 HSRB_DECL_G(4) HSRB_DECL_G(8) HSRB_DECL_G(16) HSRB_DECL_G(32)
 
 #define HSRB_DEFINE_G(G)                                                                                               \
   cudaError_t hsrb_step##G##_prepare(const Plan& p, int* bps) {                                                        \
     cudaError_t e = cudaFuncSetAttribute(hsrb_step_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); /* per function, shared by all handles */ \
     if (e == cudaSuccess) e = cudaFuncSetAttribute(hsrb_step_kernel<G, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); \
+    if (e == cudaSuccess) e = hsrb_step##G##_params_prepare();                                                        \
     if (e != cudaSuccess) return e;                                                                                    \
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_kernel<G>, p.threads, p.smem);                 \
   }                                                                                                                    \
   cudaError_t hsrb_step##G##_launch(const Plan& p, const KArgs& a, cudaStream_t s) {                                   \
     if (a.mode == MODE_RESET || a.mode == MODE_FORWARD) hsrb_step_kernel<G, false><<<p.grid, p.threads, p.smem, s>>>(a); /* the lean instance */ \
+    else if (a.params) return hsrb_step##G##_params_launch(p, a, s); /* STEP / DEBUG with parameters */             \
     else hsrb_step_kernel<G><<<p.grid, p.threads, p.smem, s>>>(a);                                                     \
+    return cudaGetLastError();                                                                                         \
+  }
+// the STEP / DEBUG instance with per-environment parameters
+#define HSRB_DEFINE_G_PARAMS(G)                                                                                        \
+  cudaError_t hsrb_step##G##_params_prepare() {                                                                        \
+    return cudaFuncSetAttribute(hsrb_step_kernel<G, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024); \
+  }                                                                                                                    \
+  cudaError_t hsrb_step##G##_params_launch(const Plan& p, const KArgs& a, cudaStream_t s) {                            \
+    hsrb_step_kernel<G, true, true><<<p.grid, p.threads, p.smem, s>>>(a);                                              \
     return cudaGetLastError();                                                                                         \
   }

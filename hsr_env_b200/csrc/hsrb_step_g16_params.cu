@@ -1,0 +1,3 @@
+// Action kernel with per-environment parameters, 16 lanes per environment (see hsrb_kernels.cuh).
+#include "hsrb_kernels.cuh"
+HSRB_DEFINE_G_PARAMS(16)

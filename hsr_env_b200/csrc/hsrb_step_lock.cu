@@ -3,12 +3,14 @@
 #include "hsrb_kernels.cuh"
 
 cudaError_t hsrb_step_lock_prepare(const Plan& p, int* bps) {
-  cudaError_t e = cudaFuncSetAttribute(hsrb_step_lock_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  cudaError_t e = cudaFuncSetAttribute(hsrb_step_lock_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = hsrb_step_lock_params_prepare();
   if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_lock_kernel, p.threads, p.smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_lock_kernel<false>, p.threads, p.smem);
 }
 
 cudaError_t hsrb_step_lock_launch(const Plan& p, const KArgs& a, cudaStream_t s) {
-  hsrb_step_lock_kernel<<<p.grid, p.threads, p.smem, s>>>(a);
+  if (a.params) return hsrb_step_lock_params_launch(p, a, s);
+  hsrb_step_lock_kernel<false><<<p.grid, p.threads, p.smem, s>>>(a);
   return cudaGetLastError();
 }

@@ -7,11 +7,13 @@
 cudaError_t hsrb_wpe_prepare(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+  if (e == cudaSuccess) e = hsrb_wpe_params_prepare(p);
   if (e != cudaSuccess) return e;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_wpe_kernel_t<false>, p.threads, p.smem);
 }
 
 cudaError_t hsrb_wpe_launch(const Plan& p, const KArgs& a, cudaStream_t s) {
+  if (a.params) return hsrb_wpe_params_launch(p, a, s);
   if (p.lock) hsrb_wpe_kernel_t<true><<<p.grid, p.threads, p.smem, s>>>(a, *p.fam);
   else hsrb_wpe_kernel_t<false><<<p.grid, p.threads, p.smem, s>>>(a, *p.fam);
   return cudaGetLastError();

@@ -26,6 +26,11 @@ from .util import GoalSpec  # noqa: F401  (re-exported, as hsr.env does)
 
 _BLOBS = Path(__file__).resolve().parent / "blobs"
 
+# Columns of the per-environment physics parameters (include/hsrb.h hsrb_set_env_params): multipliers of pair_friction,
+# of the block bodies' mass and inertia, of act_kp and of dof_damping.  1.0 is the model as compiled.
+PARAM_NAMES = ("friction", "block_mass", "actuator_gain", "damping")
+_PARAM_POSITIVE = (True, True, False, False)   # > 0, or >= 0
+
 
 def get_xml_filepath(xml_filename=Path("models/world.xml")) -> Path:
     """hsr/env.py:16-17: relative model paths resolve inside the package's asset directory."""
@@ -88,7 +93,10 @@ class BatchedHSREnv:
             kernel: str = "auto",
             max_episode_steps: Optional[int] = None,
             autoreset: bool = False,
+            randomize: Optional[dict] = None,
     ):
+        """``randomize``: domain randomization, ``{name: (lo, hi)}`` over ``PARAM_NAMES`` (a missing name: (1, 1)); every
+        reset, the auto-reset included, redraws the reset environments' parameters ~ U[lo, hi)."""
         if any([render, record, render_freq, record_freq, record_path]):
             raise NotImplementedError("render/record need an OpenGL viewer and are outside the batched backend "
                                       "(SURVEY.md §8f row f4)")
@@ -142,6 +150,8 @@ class BatchedHSREnv:
         self._episodes = self.max_episode_steps > 0 or self.autoreset
         self._parse_goal_specs()
         self._push_starts()
+        if randomize is not None:
+            self.set_param_ranges(randomize)
 
     # ------------------------------------------------------------------ goals
     def _body_id(self, name: str) -> int:
@@ -426,6 +436,55 @@ class BatchedHSREnv:
         with torch.cuda.device(self.device):
             _lib.check(self._lib.hsrb_compute_reward(self._h, _lib.ptr(reward), None, self._stream()))
         return reward
+
+    # ------------------------------------------------------------------ per-environment physics parameters
+    def set_param_ranges(self, ranges: Optional[dict]):
+        """``{name: (lo, hi)}`` over ``PARAM_NAMES`` (missing: (1, 1)): every reset redraws the reset environments'
+        parameters ~ U[lo, hi).  None: parameters persist across resets."""
+        if ranges is None:
+            _lib.check(self._lib.hsrb_set_env_param_ranges(self._h, None, None))
+            return
+        unknown = set(ranges) - set(PARAM_NAMES)
+        if unknown:
+            raise KeyError(f"unknown parameter(s) {sorted(unknown)}; names: {PARAM_NAMES}")
+        lo = (ctypes.c_float * 4)(*[float(ranges.get(k, (1.0, 1.0))[0]) for k in PARAM_NAMES])
+        hi = (ctypes.c_float * 4)(*[float(ranges.get(k, (1.0, 1.0))[1]) for k in PARAM_NAMES])
+        _lib.check(self._lib.hsrb_set_env_param_ranges(self._h, lo, hi))
+
+    def set_env_params(self, params):
+        """Per-environment multipliers: a [N, 4] tensor (columns ``PARAM_NAMES``), a dict of [N] tensors (missing names:
+        1.0), or None (nominal model, ranges cleared, the kernels without parameters).  friction and block_mass must be
+        > 0, actuator_gain and damping >= 0."""
+        if params is None:
+            with torch.cuda.device(self.device):
+                _lib.check(self._lib.hsrb_set_env_params(self._h, None, self._stream()))
+            return
+        if isinstance(params, dict):
+            unknown = set(params) - set(PARAM_NAMES)
+            if unknown:
+                raise KeyError(f"unknown parameter(s) {sorted(unknown)}; names: {PARAM_NAMES}")
+            cols = [torch.as_tensor(params[k], dtype=torch.float32, device=self.device).reshape(self.n_envs)
+                    if k in params else torch.ones(self.n_envs, device=self.device) for k in PARAM_NAMES]
+            p = torch.stack(cols, dim=1)
+        else:
+            p = torch.as_tensor(params, dtype=torch.float32, device=self.device).reshape(self.n_envs, len(PARAM_NAMES))
+        p = p.contiguous()
+        if not bool(torch.isfinite(p).all()):
+            raise ValueError("environment parameters must be finite")
+        for k, (name, positive) in enumerate(zip(PARAM_NAMES, _PARAM_POSITIVE)):
+            col = p[:, k]
+            if not bool((col > 0).all() if positive else (col >= 0).all()):
+                raise ValueError(f"{name} multipliers must be {'> 0' if positive else '>= 0'}")
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_set_env_params(self._h, _lib.ptr(p), self._stream()))
+            torch.cuda.current_stream(self.device).synchronize()  # the input may be a temporary
+
+    def env_params(self) -> torch.Tensor:
+        """The current multipliers: float32 [N, 4], columns ``PARAM_NAMES``."""
+        out = self._empty(self.n_envs, len(PARAM_NAMES))
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_get_env_params(self._h, _lib.ptr(out), self._stream()))
+        return out
 
     # ------------------------------------------------------------------ state access (sim.get_state / set_state)
     def get_state(self):

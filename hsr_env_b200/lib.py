@@ -32,6 +32,9 @@ SIGNATURES = {
     "hsrb_set_episode_ages": (c_int, [c_void_p, c_void_p, c_void_p]),
     "hsrb_get_episode_ages": (c_int, [c_void_p, c_void_p, c_void_p]),
     "hsrb_episode_stats": (c_int, [c_void_p, POINTER(c_int64), c_void_p]),
+    "hsrb_set_env_params": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "hsrb_get_env_params": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "hsrb_set_env_param_ranges": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float)]),
     "hsrb_step_host":(c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_get_state": (c_int, [c_void_p] + [c_void_p] * 5),
     "hsrb_set_state": (c_int, [c_void_p] + [c_void_p] * 5),

@@ -110,6 +110,22 @@ int hsrb_episode_update(hsrb_t* h, int max_episode_steps, int autoreset, const u
 int hsrb_set_episode_ages(hsrb_t* h, const int32_t* age, void* stream);
 int hsrb_get_episode_ages(hsrb_t* h, int32_t* age, void* stream);
 
+/* Per-environment physics parameters (domain randomization, DESIGN 4.3b): four fp32 multipliers per environment,
+ * [0] friction (all five pair_friction coefficients of every contact pair, > 0), [1] block_mass (body_mass and
+ * body_inertia of every body in block_body, > 0), [2] actuator_gain (act_kp, >= 0), [3] damping (dof_damping, >= 0),
+ * with the meaning of editing those model fields without recomputing the compile-time derived quantities.  Not part of
+ * the state.  params[N,4] device fp32, copied into the handle on `stream`; NULL: back to nominal (1.0), ranges cleared,
+ * and to the kernels without parameters.  The 8-lane lock-step kernel (path 2) has no instance with parameters: with
+ * parameters set, hsrb_step, hsrb_set_path(2) and hsrb_launch_info fail there (-3).  get: the current multipliers
+ * (1.0 when never set). */
+int hsrb_set_env_params(hsrb_t* h, const float* params, void* stream);
+int hsrb_get_env_params(hsrb_t* h, float* params, void* stream);
+/* lo_host[4], hi_host[4]: every reset (hsrb_reset's masked environments, the auto-reset of hsrb_step_episode /
+ * hsrb_episode_update) redraws the environment's params ~ U[lo, hi) from draw block 8192 of its Philox stream (key = seed,
+ * GLOBAL env id; counter = the episode the reset starts); the reset state is the same with or without ranges.  Values
+ * outside the domains above, NaN or lo > hi are rejected (-1).  NULL clears: params then persist across resets. */
+int hsrb_set_env_param_ranges(hsrb_t* h, const float* lo_host, const float* hi_host);
+
 /* Cumulative counters of the episode kernel, copied to host (synchronises `stream`): [0] episodes finished (done),
  * [1] of them terminated (success), [2] truncated, [3] summed episode length in actions, [4] summed substeps of the
  * finished episodes, [5] steps with a non-zero bad_state, [6] auto-resets, [7] environment actions stepped. */
