@@ -255,6 +255,7 @@ int configure_lock(const hsrb* h, Plan& p) {
   p.ncon_max = h->dm.ncon_max; p.nefc_max = h->dm.nefc_max;
   p.lanes = 32;
   p.launch = hsrb_step_lock_launch;
+  p.rollout = hsrb_step_lock_rollout_launch;
   const size_t tail = lock_tail_bytes();
   int wpb = (int)((227 * 1024 - tail) / p.ws);
   if (wpb < 1) return fail(-3, "no launch configuration fits: workspace %u bytes per environment", p.ws);
@@ -308,6 +309,7 @@ int configure_wpe(const hsrb* h, Plan& p) {
   p.lock = h->knobs.wpe_lock;
   p.lanes = 32;
   p.launch = hsrb_wpe_launch;
+  if (p.lock) p.rollout = hsrb_wpe_rollout_launch;   // the free-running variant has no instance with the action loop
   const size_t tail = wpe::shared_tail(h->dm);
   // one warp per environment; all environments resident in one wave when they fit (warps per block = n / SMs),
   // otherwise the most warps shared memory and the register file hold, and a grid-stride loop over the environments
@@ -355,7 +357,8 @@ KArgs base_args(hsrb* h) {
   return a;
 }
 
-int run(hsrb* h, KArgs& a, void* stream) {
+// nact > 0: a STEP launch of nact actions through the plan's rollout instance (hsrb_rollout; the caller checked there is one)
+int run(hsrb* h, KArgs& a, void* stream, int nact = 0) {
   cudaStream_t s = (cudaStream_t)stream;
   Kernel k = K_GENERAL;
   if (a.mode == MODE_STEP) { const int rc = select(h, &k); if (rc) return rc; }
@@ -373,7 +376,7 @@ int run(hsrb* h, KArgs& a, void* stream) {
   // (the work-sorted launch order was tried on the phase-locked general kernel too: no gain on configs[2] / [4], 2.80 vs
   // 2.88 and 1.28 vs 1.35 M substeps/s - configs[2] resets every environment before every action, configs[4] runs four
   // warps per block)
-  CU(p->launch(*p, a, s));
+  CU(nact ? p->rollout(*p, a, nact, s) : p->launch(*p, a, s));
   if (sorted && (rc = h->sort.update(h->n, s))) return rc;
   h->launches++;
   return 0;
@@ -807,6 +810,39 @@ int hsrb_step(hsrb_t* h, const float* ctrl, int nsubsteps, float* obs, float* re
   a.mode = MODE_STEP; a.ctrl = ctrl; a.nsub = nsubsteps; a.obs = obs; a.reward = reward; a.done = done;
   a.success = success; a.taken = substeps_taken; a.bad = bad_state;
   return run(h, a, stream);
+}
+
+int hsrb_rollout(hsrb_t* h, const float* ctrl, int nactions, int nsubsteps, float* obs, float* reward, uint8_t* done,
+                 int32_t* substeps_taken, uint8_t* bad_state, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  if (nactions < 0) return fail(-1, "nactions < 0");
+  if (!ctrl && h->hm.m.nu > 0) return fail(-1, "ctrl is NULL");
+  if (nsubsteps < 0) return fail(-1, "nsubsteps < 0");
+  if (nactions == 0) return 0;
+  CU(cudaSetDevice(h->device));
+  KArgs a = base_args(h);
+  a.mode = MODE_STEP; a.ctrl = ctrl; a.nsub = nsubsteps; a.obs = obs; a.reward = reward; a.done = done;
+  a.taken = substeps_taken; a.bad = bad_state;
+  Kernel k = K_GENERAL;
+  const Plan* p = nullptr;
+  int rc = select(h, &k);
+  if (!rc) rc = configure(h, k, &p);
+  if (rc) return rc;
+  if (p->rollout) return run(h, a, stream, nactions);   // one launch: the phase-locked wpe and general kernels
+  // every other kernel: one hsrb_step launch per action on slice k of each array
+  const size_t n = (size_t)h->n, nobs = (size_t)(h->hm.m.nq + h->hm.m.nv), nu = (size_t)h->hm.m.nu;
+  for (int i = 0; i < nactions; i++) {
+    KArgs b = a;
+    const size_t r = (size_t)i * n;
+    if (ctrl) b.ctrl = ctrl + r * nu;
+    if (obs) b.obs = obs + r * nobs;
+    if (reward) b.reward = reward + r;
+    if (done) b.done = done + r;
+    if (substeps_taken) b.taken = substeps_taken + r;
+    if (bad_state) b.bad = bad_state + r;
+    if ((rc = run(h, b, stream))) return rc;
+  }
+  return 0;
 }
 
 int hsrb_step_episode(hsrb_t* h, const float* ctrl, int nsubsteps, int max_episode_steps, int autoreset, float* obs, float* reward,

@@ -5,6 +5,7 @@
 cudaError_t hsrb_step_lock_prepare(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_step_lock_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = hsrb_step_lock_params_prepare();
+  if (e == cudaSuccess) e = hsrb_step_lock_rollout_prepare();
   if (e != cudaSuccess) return e;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_step_lock_kernel<false>, p.threads, p.smem);
 }

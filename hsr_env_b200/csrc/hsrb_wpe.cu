@@ -8,6 +8,7 @@ cudaError_t hsrb_wpe_prepare(const Plan& p, int* bps) {
   cudaError_t e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(hsrb_wpe_kernel_t<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = hsrb_wpe_params_prepare(p);
+  if (e == cudaSuccess) e = hsrb_wpe_rollout_prepare();
   if (e != cudaSuccess) return e;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(bps, hsrb_wpe_kernel_t<false>, p.threads, p.smem);
 }

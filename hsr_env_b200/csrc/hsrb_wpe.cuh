@@ -402,6 +402,7 @@ __device__ __forceinline__ int* team_jobs(Queue& Q, const Tab& t, int w) { retur
 #else
 #define WPE_PH(id) do { } while (0)
 #endif
+#define WPE_ROLLOUT 0
 #define WPE_ENTRY hsrb_wpe_kernel_t
 #define WPE_PARAMS false
 #include "hsrb_wpe_kernel.cuh"
@@ -413,6 +414,20 @@ __device__ __forceinline__ int* team_jobs(Queue& Q, const Tab& t, int w) { retur
 #include "hsrb_wpe_kernel.cuh"
 #undef WPE_ENTRY
 #undef WPE_PARAMS
+#undef WPE_ROLLOUT
+// the open-loop rollout instances (hsrb_rollout: K actions per environment in one launch; hsrb_wpe_rollout.cu)
+#define WPE_ROLLOUT 1
+#define WPE_ENTRY hsrb_wpe_rollout_kernel_t
+#define WPE_PARAMS false
+#include "hsrb_wpe_kernel.cuh"
+#undef WPE_ENTRY
+#undef WPE_PARAMS
+#define WPE_ENTRY hsrb_wpe_rollout_params_kernel_t
+#define WPE_PARAMS true
+#include "hsrb_wpe_kernel.cuh"
+#undef WPE_ENTRY
+#undef WPE_PARAMS
+#undef WPE_ROLLOUT
 #endif  // HSRB_WPE_IMPL
 
 // host side (hsrb_wpe.cu): p.lock picks the instance; a.params the instance with parameters (hsrb_wpe_params.cu)
@@ -420,3 +435,6 @@ cudaError_t hsrb_wpe_prepare(const Plan& p, int* bps);
 cudaError_t hsrb_wpe_params_prepare(const Plan& p);
 cudaError_t hsrb_wpe_params_launch(const Plan& p, const KArgs& a, cudaStream_t s);
 cudaError_t hsrb_wpe_launch(const Plan& p, const KArgs& a, cudaStream_t s);
+// the phase-locked instances with the action loop (hsrb_wpe_rollout.cu): nact actions in one launch
+cudaError_t hsrb_wpe_rollout_prepare();
+cudaError_t hsrb_wpe_rollout_launch(const Plan& p, const KArgs& a, int nact, cudaStream_t s);

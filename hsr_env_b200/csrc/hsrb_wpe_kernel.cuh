@@ -1,9 +1,16 @@
 // The body of the warp-per-environment kernel, included by hsrb_wpe.cuh once per entry point: WPE_ENTRY names the
 // __global__ template <bool LOCK>, WPE_PARAMS = true reads per-environment multipliers a.params (hsr_core.h EnvScale) per
-// environment of the grid-stride loop.  The body is written out in the entry itself, not in a __device__ function behind
-// it: the wrapper changes the code ptxas makes of the instances without parameters.
+// environment of the grid-stride loop.  WPE_ROLLOUT = 1 (hsrb_rollout) takes the number of actions nact as a parameter
+// after the existing ones and runs the per-slot body, from "state -> shared memory" to "results", once per action:
+// action k reads ctrl row k * n + env and writes output row k * n + env.  The body is written out in the entry itself, not
+// in a __device__ function behind it: the wrapper changes the code ptxas makes of the instances without parameters.
 template <bool LOCK>
+#if WPE_ROLLOUT
+__global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_constant__ KArgs a, const __grid_constant__ PushInfo fi,
+                                                                  const int nact) {
+#else
 __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_constant__ KArgs a, const __grid_constant__ PushInfo fi) {
+#endif
   constexpr bool PARAMS = WPE_PARAMS;
   constexpr unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
@@ -99,6 +106,18 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_c
       Mi = li < NV ? (li >= 2 ? mul_rn(fi.Mdiag[li], sc.scale(PRM_BLOCK_MASS)) : fi.Mdiag[li]) : 1.0f;
       dampi = li < NV ? sc.damping(fi.damp[li]) : 0.f;
     }
+#if WPE_ROLLOUT
+    // the environment's actions one after the other (invalid slots of the phase-locked variant too: they take part in the
+    // team barriers).  Each action starts as a launch of hsrb_step does: from the state row in HBM, which the previous
+    // action wrote (the __syncwarp closing the results orders the lanes' stores before these loads), with every per-action
+    // quantity re-initialised below
+#pragma unroll 1
+    for (int k = 0; k < nact; k++) {
+    const size_t krow = (size_t)k * (size_t)a.n;
+#define WPE_ROW(e) (krow + (size_t)(e))
+#else
+#define WPE_ROW(e) (e)
+#endif
     // ------------------------------------------------------------------ state -> shared memory
     if (valid) {
       const float* st = a.state + (size_t)env * a.S;
@@ -109,7 +128,7 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_c
         s.qfc[lane] = 0.f;
       }
       if (lane < 3) s.mocap[lane] = st[nq + 2 * NV + lane];
-      if (lane < 2) s.ctrl[lane] = (a.ctrl && lane < fi.act_n) ? a.ctrl[(size_t)env * m.nu + lane] : 0.f;
+      if (lane < 2) s.ctrl[lane] = (a.ctrl && lane < fi.act_n) ? a.ctrl[(size_t)WPE_ROW(env) * m.nu + lane] : 0.f;
       if (lane < 4) s.wi[lane] = 0;
       for (int i = lane; i < 4 * m.npair; i += 32) s.sep[i] = 0.f;     // no cached separating directions
       for (int i = lane; i < m.ngeom * 3; i += 32) s.gpos[i] = t.gbase[i];
@@ -953,14 +972,14 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_c
       for (int i = lane; i < nq + 2 * NV; i += 32) {
         const float v = i < nq ? s.qpos[i] : (i < nq + NV ? s.qvel[i - nq] : s.warm[i - nq - NV]);
         st[i] = v;
-        if (a.obs && i < nobs) a.obs[(size_t)env * nobs + i] = v;
+        if (a.obs && i < nobs) a.obs[(size_t)WPE_ROW(env) * nobs + i] = v;
       }
       if (lane == 0) {
-        if (a.reward) a.reward[env] = success ? 1.0f : 0.0f;
-        if (a.done) a.done[env] = success ? 1 : 0;
-        if (a.success) a.success[env] = success ? 1 : 0;
-        if (a.taken) a.taken[env] = taken;
-        if (a.bad) a.bad[env] = (unsigned char)flags;
+        if (a.reward) a.reward[WPE_ROW(env)] = success ? 1.0f : 0.0f;
+        if (a.done) a.done[WPE_ROW(env)] = success ? 1 : 0;
+        if (a.success) a.success[WPE_ROW(env)] = success ? 1 : 0;
+        if (a.taken) a.taken[WPE_ROW(env)] = taken;
+        if (a.bad) a.bad[WPE_ROW(env)] = (unsigned char)flags;
         // work estimate in k-cycles of an uncontended warp (tools/chain_clocks.py): fixed part, Newton iterations, refinements, rows
 #if defined(WPE_CHAIN_CLOCKS)
         if (a.work) a.work[env] = (int)((clock64() - ck_env0) >> 10);   // measured: k-cycles of this environment's action
@@ -978,6 +997,10 @@ __global__ void __launch_bounds__(32 * WPE_MAXWARPS, 1) WPE_ENTRY(const __grid_c
       }
       __syncwarp();
     }
+#if WPE_ROLLOUT
+    }
+#endif
+#undef WPE_ROW
   }
 #if defined(HSRB_PHASE_CLOCKS)
   if (LOCK && threadIdx.x == 0 && blockIdx.x == 0)

@@ -27,6 +27,7 @@ SIGNATURES = {
     "hsrb_set_starts": (c_int, [c_void_p, c_int, POINTER(c_int32), POINTER(c_int32), POINTER(c_float), POINTER(c_float)]),
     "hsrb_reset": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_step": (c_int, [c_void_p, c_void_p, c_int] + [c_void_p] * 7),
+    "hsrb_rollout": (c_int, [c_void_p, c_void_p, c_int, c_int] + [c_void_p] * 6),
     "hsrb_step_episode": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int] + [c_void_p] * 11),
     "hsrb_episode_update": (c_int, [c_void_p, c_int, c_int] + [c_void_p] * 11),
     "hsrb_set_episode_ages": (c_int, [c_void_p, c_void_p, c_void_p]),

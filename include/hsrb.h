@@ -79,6 +79,18 @@ int hsrb_reset(hsrb_t* h, const uint8_t* mask, float* obs, void* stream);
 int hsrb_step(hsrb_t* h, const float* ctrl, int nsubsteps, float* obs, float* reward, uint8_t* done, uint8_t* success,
               int32_t* substeps_taken, uint8_t* bad_state, void* stream);
 
+/* nactions x HSREnv.step with the actions given in advance (open-loop rollout)   env.py:115-135
+ * mujoco-py has no counterpart; MuJoCo's mujoco.rollout is the analogue.  ctrl[K, N, nu] (K = nactions); obs[K, N, nq+nv],
+ * reward / done / bad_state [K, N], substeps_taken[K, N] int32, all nullable: slice k holds what the k-th of K hsrb_step
+ * calls would return, bit for bit, and the state afterwards is the state after the K-th.  Nothing else happens between
+ * the actions: an environment that reached its goal starts the next action from that state, nothing is reset, episode
+ * ages and counters are untouched (as hsrb_step leaves them), and per-environment parameters apply as in hsrb_step.  The
+ * counters of hsrb_stats grow as over K steps, except launches: +1 when the selected kernel is the phase-locked wpe or
+ * general kernel (one launch for all K actions), +K for every other kernel (one hsrb_step launch per action).
+ * nactions < 0, nsubsteps < 0 or a NULL ctrl with nu > 0: -1; nactions == 0 does nothing.  Other errors are hsrb_step's. */
+int hsrb_rollout(hsrb_t* h, const float* ctrl, int nactions, int nsubsteps, float* obs, float* reward, uint8_t* done,
+                 int32_t* substeps_taken, uint8_t* bad_state, void* stream);
+
 /* gym.wrappers.TimeLimit(max_episode_steps) + the caller's `if done: env.reset()`   hsr/__init__.py:22, control.py:73-75
  * The action kernel exactly as hsrb_step runs it, then one episode kernel.  Each environment has an episode age: the
  * actions since its last reset (hsrb_reset or auto-reset set it to 0, a step adds 1).  terminated = success (hsrb_step's
