@@ -21,6 +21,7 @@
 #include "../../include/hsrb.h"
 #include "hsrb_wpe.cuh"
 #include "hsrb_episode.cuh"
+#include "hsrb_contacts.cuh"
 
 namespace {
 
@@ -176,6 +177,7 @@ struct hsrb {
   SortBufs sort;
   EpisodeBufs ep;
   ParamBufs prm;
+  int con_lanes = 0;        // layout the contact query kernel was prepared for (hsrb_contacts)
   // scratch for the host-buffer entry point
   float *d_ctrl = nullptr, *d_obs = nullptr, *d_reward = nullptr;
   unsigned char* d_done = nullptr;
@@ -1014,6 +1016,40 @@ int hsrb_debug_substep(hsrb_t* h, const float* ctrl, double* dump, void* stream)
   KArgs a = base_args(h);
   a.mode = MODE_DEBUG; a.ctrl = ctrl; a.nsub = 1; a.dump = dump; a.dump_stride = (unsigned)debug_size(h->dm);
   return run(h, a, stream);
+}
+
+int hsrb_contact_capacity(hsrb_t* h) {
+  if (!h) return fail(-1, "null handle");
+  return h->dm.ncon_max;   // the general plan's ncon_max (configure_general)
+}
+
+// mj_forward + data.contact / mj_contactForce / per-body contact wrenches of the current state, in the lean launch layout of
+// the general path whatever kernel hsrb_step selects (hsrb_contacts.cuh)
+int hsrb_contacts(hsrb_t* h, const float* ctrl, int max_contacts, int32_t* count, int32_t* pair, float* dist, float* pos,
+                  float* frame, float* force, float* body_wrench, uint8_t* bad_state, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  const bool rows = pair || dist || pos || frame || force;
+  if (rows && max_contacts < 1) return fail(-1, "max_contacts < 1 with per-contact outputs");
+  CU(cudaSetDevice(h->device));
+  const Plan* p = nullptr;
+  int rc = configure(h, K_GENERAL, &p);
+  if (rc) return rc;
+  if (h->con_lanes != p->lanes) {
+    CU(hsrb_contacts_prepare(*p));
+    h->con_lanes = p->lanes;
+  }
+  ConArgs c;
+  memset(&c, 0, sizeof(c));
+  c.k = base_args(h);
+  c.k.ws_bytes = p->ws;
+  c.k.m.ncon_max = p->ncon_max; c.k.m.nefc_max = p->nefc_max;
+  c.k.ctrl = ctrl;
+  c.C = rows ? max_contacts : 0;
+  c.count = count; c.pair = pair; c.dist = dist; c.pos = pos; c.frame = frame; c.force = force; c.wrench = body_wrench;
+  c.bad = bad_state;
+  CU(hsrb_contacts_launch(*p, c, (cudaStream_t)stream));
+  h->launches++;
+  return 0;
 }
 
 int hsrb_stats(hsrb_t* h, int64_t* out9, void* stream) {

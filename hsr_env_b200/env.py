@@ -568,6 +568,66 @@ class BatchedHSREnv:
     def in_range(self) -> torch.Tensor:
         return self.compute_reward() > 0
 
+    # ------------------------------------------------------------------ contacts (sim.data.contact, mj_contactForce, cfrc_ext)
+    def _query_action(self, action):
+        """The control of a contact query: None (zeros), or [N, nu] ([nu] for a single environment)."""
+        if action is None:
+            return None
+        a = torch.as_tensor(action, dtype=torch.float32, device=self.device)
+        if tuple(a.shape) != (self.n_envs, self.nu) and not (self.n_envs == 1 and tuple(a.shape) == (self.nu,)):
+            raise ValueError(f"action must be [{self.n_envs}, {self.nu}], got {list(a.shape)}")
+        return a.reshape(self.n_envs, self.nu).contiguous()
+
+    def contact_capacity(self) -> int:
+        """Contacts the query holds per environment (the general kernel's contact capacity)."""
+        return _lib.check(self._lib.hsrb_contact_capacity(self._h))
+
+    def contacts(self, action=None, max_contacts: Optional[int] = None) -> dict:
+        """Contacts and contact forces of the current state of every environment (mj_forward, then sim.data.contact and
+        mj_contactForce); the state is left exactly as it was.  ``action`` [N, nu] is the control the forces are computed
+        with (None: zeros); for the forces of the state a step just reached, pass that step's action.  Always the general
+        kernel's collision and solver stages, whatever kernel step() runs (DESIGN.md 4.3d).
+
+        Returns device tensors, C = ``max_contacts`` (default: ``contact_capacity()``): ``count`` [N] int32;
+        ``pair`` [N, C] int32 (candidate-pair index), ``geom`` / ``body`` [N, C, 2] int64 (geom1 / geom2 and their bodies),
+        ``dim`` [N, C] int64 (condim), ``dist`` [N, C], ``pos`` [N, C, 3], ``frame`` [N, C, 3, 3] (row 0 the normal from
+        geom1 to geom2), ``force`` [N, C, 6] (normal, 2 tangential, torsional, 2 rolling, in the contact frame) and
+        ``bad_state`` [N] uint8 (bit 0: the forward pass found more contacts than it holds).  Only the first
+        min(count, C) rows are contacts; padding rows hold -1 in the integer fields and 0 elsewhere."""
+        C = self.contact_capacity() if max_contacts is None else int(max_contacts)
+        if C < 1:
+            raise ValueError(f"max_contacts must be >= 1, got {C}")
+        ctrl = self._query_action(action)
+        n = self.n_envs
+        out = dict(count=self._empty(n, dtype=torch.int32), pair=self._empty(n, C, dtype=torch.int32), dist=self._empty(n, C),
+                   pos=self._empty(n, C, 3), frame=self._empty(n, C, 3, 3), force=self._empty(n, C, 6),
+                   bad_state=self._empty(n, dtype=torch.uint8))
+        P = _lib.ptr
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_contacts(self._h, P(ctrl), C, P(out["count"]), P(out["pair"]), P(out["dist"]), P(out["pos"]),
+                                               P(out["frame"]), P(out["force"]), None, P(out["bad_state"]), self._stream()))
+        if getattr(self, "_pair_tab", None) is None:
+            m = self.model
+            g = np.stack([m.pair_geom1, m.pair_geom2], axis=1).astype(np.int64)
+            tab = np.concatenate([g, m.geom_body[g], m.pair_condim[:, None]], axis=1)   # [npair, 5]: geom1 geom2 body1 body2 dim
+            self._pair_tab = torch.as_tensor(tab, dtype=torch.int64, device=self.device)
+        on = out["pair"] >= 0
+        t = torch.where(on[..., None], self._pair_tab[out["pair"].long().clamp(min=0)], torch.full_like(self._pair_tab[:1], -1))
+        out["geom"], out["body"], out["dim"] = t[..., 0:2], t[..., 2:4], t[..., 4]
+        return out
+
+    def contact_wrench(self, action=None) -> torch.Tensor:
+        """Per-body sum of the contact wrenches of the current state (the contact part of MuJoCo's cfrc_ext): [N, nbody, 6] =
+        (force xyz, torque xyz) in world axes, torque about the body's centre of mass - the order is (force, torque), not
+        cfrc_ext's (torque, force).  Body 0 (world) receives the reactions, so the rows sum to zero.  ``action`` as in
+        contacts()."""
+        ctrl = self._query_action(action)
+        out = self._empty(self.n_envs, self.nbody, 6)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_contacts(self._h, _lib.ptr(ctrl), 0, None, None, None, None, None, None, _lib.ptr(out),
+                                               None, self._stream()))
+        return out
+
     # ------------------------------------------------------------------ diagnostics
     def debug_substep(self, action):
         """One teacher-forced substep with per-stage outputs (parity tests); returns a float64 [N, D] tensor."""
@@ -648,6 +708,25 @@ class HSREnv(BatchedHSREnv):
 
     def compute_reward(self):
         return float(super().compute_reward()[0].item())
+
+    def contacts(self, action=None):
+        """sim.data.contact[:ncon] with mj_contactForce: numpy arrays of the ``ncon`` contacts of the current state
+        (BatchedHSREnv.contacts cut to its count), plus ``geom_names`` / ``body_names`` [ncon, 2] from the model's name
+        tables and ``bad_state``."""
+        c = super().contacts(action)
+        k = min(int(c["count"][0].item()), c["pair"].shape[1])
+        out = {key: c[key][0, :k].cpu().numpy() for key in ("pair", "geom", "body", "dim", "dist", "pos", "frame", "force")}
+        out["pos"], out["frame"], out["force"] = (out[key].astype(np.float64) for key in ("pos", "frame", "force"))
+        out["dist"] = out["dist"].astype(np.float64)
+        out["ncon"] = k
+        out["bad_state"] = int(c["bad_state"][0].item())
+        gn, bn = list(self.model.names.get("geom", [])), list(self.model.names.get("body", []))
+        out["geom_names"] = [(gn[a], gn[b]) for a, b in out["geom"]] if gn else []
+        out["body_names"] = [(bn[a], bn[b]) for a, b in out["body"]] if bn else []
+        return out
+
+    def contact_wrench(self, action=None):
+        return super().contact_wrench(action)[0].double().cpu().numpy()
 
     def in_range(self, a=None, b=None, distance=None):
         if a is None:

@@ -42,6 +42,8 @@ SIGNATURES = {
     "hsrb_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_openai_obs": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "hsrb_compute_reward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hsrb_contact_capacity": (c_int, [c_void_p]),
+    "hsrb_contacts": (c_int, [c_void_p, c_void_p, c_int] + [c_void_p] * 9),
     "hsrb_debug_size": (c_int, [c_void_p]),
     "hsrb_debug_substep": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_stats": (c_int, [c_void_p, POINTER(c_int64), c_void_p]),

@@ -175,6 +175,38 @@ int hsrb_openai_obs(hsrb_t* h, int finger_qposadr_l, int finger_qposadr_r, int f
  * agree with env.py:126,133): reward[N] / success[N] of the CURRENT state, no stepping. */
 int hsrb_compute_reward(hsrb_t* h, float* reward, uint8_t* success, void* stream);
 
+/* Contact query (DESIGN 4.3d): sim.data.ncon / sim.data.contact, mj_contactForce and the contact part of cfrc_ext for every
+ * environment.  It runs mj_forward on the CURRENT resident state and reads what it produced; it changes nothing: state,
+ * qacc_warmstart (which MuJoCo's mj_forward does write; this query deliberately does not), episode counters and parameters
+ * stay as they were, and a step after the query gives the bits of a step without it.
+ *   ctrl[N, nu] (NULL = zeros, as a NULL ctrl reads in hsrb_step): forces depend on the control through the actuation in
+ *   qacc_smooth, and ctrl is not part of the resident state; for the forces of the state a step just reached, pass the
+ *   action of that step.  Per-environment parameters (hsrb_set_env_params) apply as in hsrb_step.
+ *   Which code runs: always the general path's stages (hsr_core.h forward()) at the general plan's lanes and capacities
+ *   (hsrb_config), whatever kernel hsrb_step selects - as hsrb_forward, hsrb_compute_reward and hsrb_debug_substep do.
+ *   The warp-per-environment and 8-lane kernels have collision code and a fixed capacity of 8 contacts of their own;
+ *   their contacts are NOT what this call reports.
+ *   Contact order: the order of the general collision stage (that of hsrb_debug_substep's dump).
+ * Outputs, all nullable, C = max_contacts: count[N] = contacts the forward pass holds (<= hsrb_contact_capacity); per contact
+ * (only the first min(count, C) rows are contacts, later rows are padding with pair = -1 and floats 0, so every byte is
+ * defined): pair[N, C] int32 = the model's candidate-pair index (geom1 / geom2, condim and bodies follow from the model's
+ * pair tables); dist[N, C]; pos[N, C, 3] (world); frame[N, C, 9] = con_frame, row 0 the normal pointing from geom1 to
+ * geom2, rows 1-2 the tangents; force[N, C, 6] = the contact's constraint-row forces in the contact frame (mj_contactForce,
+ * elliptic cones: the efc_force rows): [0] normal, [1..2] tangential, [3] torsional, [4..5] rolling, rows past the pair's
+ * condim 0.  body_wrench[N, nbody, 6] = (force xyz, torque xyz) in world axes, torque about the body's centre of mass
+ * (xipos) - note the order differs from cfrc_ext's spatial (torque, force) - summed in double over the contacts in order:
+ * contact c has the frame wrench f_c = sum_{r<3} force[r] frame[r], tau_c = sum_{r>=3} force[r] frame[r-3], adds
+ * (f_c, tau_c + (pos - xipos) x f_c) to the body of pair_geom2 and the opposite to the body of pair_geom1 (cfrc_ext's
+ * sign); row 0 (world / static scene) receives its reactions too, so the rows sum to zero.  The rows and the wrenches use
+ * only the contacts the forward pass holds; when the collision stage found more than the capacity, bit 0 of bad_state[N]
+ * is set; bit 2 (4) is the Cholesky pivot clamp of the forward pass.
+ * max_contacts < 1 while any per-contact output is non-NULL: -1.  Other errors are hsrb_forward's.  hsrb_stats: launches
+ * +1, every other counter unchanged.  hsrb_contact_capacity: the contacts the query holds per environment (the general
+ * plan's ncon_max). */
+int hsrb_contact_capacity(hsrb_t* h);
+int hsrb_contacts(hsrb_t* h, const float* ctrl, int max_contacts, int32_t* count, int32_t* pair, float* dist, float* pos,
+                  float* frame, float* force, float* body_wrench, uint8_t* bad_state, void* stream);
+
 /* Teacher-forced parity hook: one substep from the current state with per-stage outputs
  * (xpos, M, qfrc_smooth, qacc_smooth, qacc, contacts, efc_J/D/aref/force, next qpos/qvel) as
  * dump[N, hsrb_debug_size()] doubles, layout = hsr::debug_dump (csrc/hsr_core.h). */
