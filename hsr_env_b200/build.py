@@ -15,8 +15,8 @@ CSRC = Path(__file__).resolve().parent / "csrc"
 LIB = CSRC / "libhsrb.so"
 TUS = ["hsrb_api.cu", "hsrb_push.cu", "hsrb_wpe.cu", "hsrb_wpe_params.cu", "hsrb_step_g4.cu", "hsrb_step_g8.cu", "hsrb_step_g16.cu", "hsrb_step_g32.cu", "hsrb_step_lock.cu", "hsrb_episode.cu",
        "hsrb_step_g4_params.cu", "hsrb_step_g8_params.cu", "hsrb_step_g16_params.cu", "hsrb_step_g32_params.cu",
-       "hsrb_step_lock_params.cu", "hsrb_wpe_rollout.cu", "hsrb_step_lock_rollout.cu", "hsrb_contacts.cu"]
-HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "hsrb_wpe_kernel.cuh", "hsrb_step_lock_kernel.cuh", "hsrb_episode.cuh", "hsrb_contacts.cuh", "../../include/hsrb.h"]
+       "hsrb_step_lock_params.cu", "hsrb_wpe_rollout.cu", "hsrb_step_lock_rollout.cu", "hsrb_contacts.cu", "hsrb_fd.cu"]
+HEADERS = ["hsr_core.h", "hsr_model.h", "hsrb_kernels.cuh", "hsrb_push.cuh", "hsrb_wpe.cuh", "hsrb_wpe_kernel.cuh", "hsrb_step_lock_kernel.cuh", "hsrb_episode.cuh", "hsrb_contacts.cuh", "hsrb_fd.cuh", "../../include/hsrb.h"]
 # per-TU flags: the fast-path kernel uses the 2-ulp fp32 division / square root (MUFU.RCP / MUFU.RSQ sequences without
 # the IEEE fix-up path; measured +6 % substeps/s, one-step error vs the fp64 oracle unchanged at the 1e-7 level); the
 # general kernel and the reset / forward paths keep IEEE division.
@@ -41,6 +41,8 @@ TU_FLAGS["hsrb_wpe_rollout.cu"] = TU_FLAGS["hsrb_wpe.cu"]
 TU_FLAGS["hsrb_step_lock_rollout.cu"] = TU_FLAGS["hsrb_step_lock.cu"]
 # the contact query runs the stages of the MODE_DEBUG instance of hsrb_step_g*.cu: same (IEEE) flags, same bits
 TU_FLAGS["hsrb_contacts.cu"] = TU_FLAGS["hsrb_step_g8.cu"]
+# so do the runs of the transition derivatives: a run's x' has the bits of hsrb_debug_substep on its input
+TU_FLAGS["hsrb_fd.cu"] = TU_FLAGS["hsrb_step_g8.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr", "-Xptxas", "-v"]

@@ -22,6 +22,7 @@
 #include "hsrb_wpe.cuh"
 #include "hsrb_episode.cuh"
 #include "hsrb_contacts.cuh"
+#include "hsrb_fd.cuh"
 
 namespace {
 
@@ -178,6 +179,10 @@ struct hsrb {
   EpisodeBufs ep;
   ParamBufs prm;
   int con_lanes = 0;        // layout the contact query kernel was prepared for (hsrb_contacts)
+  int fd_lanes = 0, fd_bps = 0;   // layout the transition-derivative kernels were prepared for, its resident blocks per SM
+  size_t fd_smem = 0;             // ... and the shared memory of a block fd_bps holds for
+  float* d_fd = nullptr;    // hsrb_transition_fd scratch, fd_words 4-byte words
+  size_t fd_words = 0;
   // scratch for the host-buffer entry point
   float *d_ctrl = nullptr, *d_obs = nullptr, *d_reward = nullptr;
   unsigned char* d_done = nullptr;
@@ -645,6 +650,7 @@ int hsrb_destroy(hsrb_t* h) {
   cudaSetDevice(h->device);
   cudaFree(h->d_fast_tab); cudaFree(h->d_model); cudaFree(h->d_state); cudaFree(h->d_episode); cudaFree(h->d_stats);
   cudaFree(h->d_ctrl); cudaFree(h->d_obs); cudaFree(h->d_reward); cudaFree(h->d_done); cudaFree(h->d_taken);
+  cudaFree(h->d_fd);
   h->sort.free();
   h->ep.free();
   h->prm.free();
@@ -1049,6 +1055,49 @@ int hsrb_contacts(hsrb_t* h, const float* ctrl, int max_contacts, int32_t* count
   c.bad = bad_state;
   CU(hsrb_contacts_launch(*p, c, (cudaStream_t)stream));
   h->launches++;
+  return 0;
+}
+
+// mjd_transitionFD for every environment: (environment, run) jobs in the lean launch layout of the general path whatever
+// kernel hsrb_step selects, then the forming kernel (hsrb_fd.cuh)
+int hsrb_transition_fd(hsrb_t* h, const float* ctrl, float eps, int centered, int nsubsteps, float* A, float* B,
+                       float* next_obs, uint8_t* bad_state, void* stream) {
+  if (!h) return fail(-1, "null handle");
+  if (!(eps > 0.f) || !std::isfinite(eps)) return fail(-1, "eps must be finite and > 0");
+  if (nsubsteps < 1) return fail(-1, "nsubsteps < 1");
+  CU(cudaSetDevice(h->device));
+  const Plan* p = nullptr;
+  int rc = configure(h, K_GENERAL, &p);
+  if (rc) return rc;
+  if (h->fd_lanes != p->lanes || h->fd_smem != p->smem) {
+    CU(hsrb_fd_prepare(*p, &h->fd_bps));
+    if (h->fd_bps < 1) return fail(-3, "transition-derivative kernel does not fit on an SM (%zu bytes of shared memory)", p->smem);
+    h->fd_lanes = p->lanes; h->fd_smem = p->smem;
+  }
+  FdArgs f;
+  memset(&f, 0, sizeof(f));
+  f.k = base_args(h);
+  f.k.ws_bytes = p->ws;
+  f.k.m.ncon_max = p->ncon_max; f.k.m.nefc_max = p->nefc_max;
+  f.k.ctrl = ctrl;
+  f.eps = eps;
+  f.rot_c = cos(0.5 * (double)eps); f.rot_s = sin(0.5 * (double)eps);
+  f.centered = centered ? 1 : 0;
+  f.nsub = nsubsteps;
+  f.nruns = fd_nruns(h->hm.m, centered != 0);
+  const size_t words = (size_t)h->n * f.nruns * fd_row(h->hm.m);
+  if (words > h->fd_words) {
+    CU(cudaFree(h->d_fd));
+    h->d_fd = nullptr; h->fd_words = 0;
+    CU(cudaMalloc(&h->d_fd, words * sizeof(float)));
+    h->fd_words = words;
+  }
+  f.scratch = h->d_fd;
+  f.A = A; f.B = B; f.next_obs = next_obs; f.bad = bad_state;
+  const long long blocks = ((long long)h->n * f.nruns + 32 / p->lanes - 1) / (32 / p->lanes);
+  const long long cap = (long long)h->fd_bps * h->num_sm;
+  CU(hsrb_fd_launch(*p, f, (int)(blocks < cap ? blocks : cap), (cudaStream_t)stream));
+  h->launches += 2;
   return 0;
 }
 

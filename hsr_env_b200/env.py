@@ -628,6 +628,33 @@ class BatchedHSREnv:
                                                None, self._stream()))
         return out
 
+    # ------------------------------------------------------------------ transition derivatives (mjd_transitionFD)
+    def transition_fd(self, action=None, eps: float = 1e-2, centered: bool = True, nsubsteps: int = 1) -> dict:
+        """Finite-difference linearisation of the dynamics of every environment at its current state (MuJoCo's
+        mjd_transitionFD): x = (dq, qvel) with dq the tangent-space displacement of qpos (a free joint: 3 + 3), u = ``action``
+        [N, nu] (None: zeros), x' = ``nsubsteps`` substeps with u held (no goal test, no freeze at success; ``nsubsteps`` =
+        steps_per_action linearises one action).  The state is left exactly as it was.  Always the general kernel's stages,
+        whatever kernel step() runs (DESIGN.md 4.3e).
+
+        Returns device tensors: ``A`` [N, 2nv, 2nv] (A[e, i, j] = dx'_i / dx_j), ``B`` [N, 2nv, nu], ``next_obs``
+        [N, nq + nv] (the unperturbed x' as qpos | qvel) and ``bad_state`` [N] uint8 (OR over the nominal and perturbed
+        runs).  Columns divide by the realised fp32 perturbation; ctrl-limited actuators follow MuJoCo's rule (one-sided
+        at a limit, a zero column outside the range)."""
+        eps, nsubsteps = float(eps), int(nsubsteps)
+        if not (eps > 0 and np.isfinite(eps)):
+            raise ValueError(f"eps must be finite and > 0, got {eps}")
+        if nsubsteps < 1:
+            raise ValueError(f"nsubsteps must be >= 1, got {nsubsteps}")
+        ctrl = self._query_action(action)
+        n, nx = self.n_envs, 2 * self.nv
+        out = dict(A=self._empty(n, nx, nx), B=self._empty(n, nx, self.nu), next_obs=self._empty(n, self.state_dim),
+                   bad_state=self._empty(n, dtype=torch.uint8))
+        P = _lib.ptr
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.hsrb_transition_fd(self._h, P(ctrl), eps, int(bool(centered)), nsubsteps, P(out["A"]),
+                                                    P(out["B"]), P(out["next_obs"]), P(out["bad_state"]), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ diagnostics
     def debug_substep(self, action):
         """One teacher-forced substep with per-stage outputs (parity tests); returns a float64 [N, D] tensor."""
@@ -727,6 +754,15 @@ class HSREnv(BatchedHSREnv):
 
     def contact_wrench(self, action=None):
         return super().contact_wrench(action)[0].double().cpu().numpy()
+
+    def transition_fd(self, action=None, **kw):
+        """mjd_transitionFD of the environment: float64 numpy ``A`` [2nv, 2nv], ``B`` [2nv, nu], ``next_obs`` [nq + nv] and
+        an int ``bad_state``; keyword arguments as BatchedHSREnv.transition_fd."""
+        a = None if action is None else np.asarray(action, np.float32)
+        r = super().transition_fd(a, **kw)
+        out = {k: r[k][0].double().cpu().numpy() for k in ("A", "B", "next_obs")}
+        out["bad_state"] = int(r["bad_state"][0].item())
+        return out
 
     def in_range(self, a=None, b=None, distance=None):
         if a is None:

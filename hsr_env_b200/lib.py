@@ -44,6 +44,7 @@ SIGNATURES = {
     "hsrb_compute_reward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_contact_capacity": (c_int, [c_void_p]),
     "hsrb_contacts": (c_int, [c_void_p, c_void_p, c_int] + [c_void_p] * 9),
+    "hsrb_transition_fd": (c_int, [c_void_p, c_void_p, c_float, c_int, c_int] + [c_void_p] * 5),
     "hsrb_debug_size": (c_int, [c_void_p]),
     "hsrb_debug_substep": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "hsrb_stats": (c_int, [c_void_p, POINTER(c_int64), c_void_p]),

@@ -207,6 +207,36 @@ int hsrb_contact_capacity(hsrb_t* h);
 int hsrb_contacts(hsrb_t* h, const float* ctrl, int max_contacts, int32_t* count, int32_t* pair, float* dist, float* pos,
                   float* frame, float* force, float* body_wrench, uint8_t* bad_state, void* stream);
 
+/* Transition derivatives (DESIGN 4.3e): MuJoCo's mjd_transitionFD(m, d, eps, flg_centered, A, B, NULL, NULL) for every
+ * environment.  The map differentiated is x' = nsubsteps substeps of the general path's substep() from the environment's
+ * CURRENT resident state with ctrl held, x = (dq, qvel) of 2nv coordinates (dq the tangent-space displacement of qpos as in
+ * MuJoCo: a free joint contributes 3 position + 3 rotation coordinates), u = ctrl[nu].  It is the derivative of the physics,
+ * not of hsrb_step's action: there is no goal test and no freeze at success.  nsubsteps = 1 is mjd_transitionFD;
+ * nsubsteps = steps_per_action linearises one env action.
+ *   Perturbations, on the fp32 values of the state and ctrl: a scalar coordinate (slide / hinge qpos, qvel, ctrl) becomes
+ *   fl(x + eps) / fl(x - eps), or the next float in that direction when the rounded value equals x; rotation k of a free
+ *   joint becomes normalize(q (x) [cos(eps/2), +-sin(eps/2) e_k]) (local frame), computed in double and rounded to fp32.
+ *   Every column divides by the REALISED perturbation h, computed in double from the fp32 values used (x+- - x, or
+ *   component k of mj_differentiatePos / mju_subQuat(q+-, q)), not by eps.  Output differences d+- = x'+- - x'0 are taken
+ *   in double, with mju_subQuat(q'+-, q'0) for free-joint rotations.  centered != 0: (d+ - d-) / (h+ - h-); else d+ / h+;
+ *   rounded to fp32 once.
+ *   Ctrl limits (MuJoCo's rule): for a ctrllimited actuator a side may be used only if u and u+-eps both lie in ctrlrange.
+ *   Centered: both sides -> centered, one side -> that one-sided difference, neither -> a zero column.  Forward: forward,
+ *   else backward, else zero.  A u outside its range therefore gets a zero column (the derivative of the ctrl clamp).
+ *   Every run, nominal and perturbed, starts from the resident qacc_warmstart and an empty separating-direction cache.
+ *   Per-environment parameters (hsrb_set_env_params) apply as in hsrb_step.  Which code runs: always the general path's
+ *   stages at the general plan's lanes and capacities, whatever kernel hsrb_step selects (as hsrb_contacts).
+ * Outputs, all nullable, row-major: A[N, 2nv, 2nv] with A[e, i, j] = dx'_i / dx_j; B[N, 2nv, nu]; next_obs[N, nq + nv] =
+ * the unperturbed x' as qpos | qvel; bad_state[N] = the OR of the flags of every run of the environment (bit 0 contact
+ * overflow, 1 non-finite, 2 Cholesky clamp).  ctrl[N, nu] device pointer, NULL = zeros.
+ * The call changes nothing: state, qacc_warmstart, episode counters, parameters and work counters stay as they were;
+ * hsrb_stats: launches +2 (the runs and the forming kernel).  Scratch: the handle keeps N * nruns * (nq + nv + 3) 4-byte
+ * words of device memory, nruns = 1 + 2 (2nv + nu) centered, 1 + 2nv + nu forward (x', flags and h of every run),
+ * allocated on first use, grown when a call needs more, freed by hsrb_destroy.
+ * eps <= 0 or not finite, or nsubsteps < 1: -1.  Other errors are hsrb_forward's. */
+int hsrb_transition_fd(hsrb_t* h, const float* ctrl, float eps, int centered, int nsubsteps, float* A, float* B,
+                       float* next_obs, uint8_t* bad_state, void* stream);
+
 /* Teacher-forced parity hook: one substep from the current state with per-stage outputs
  * (xpos, M, qfrc_smooth, qacc_smooth, qacc, contacts, efc_J/D/aref/force, next qpos/qvel) as
  * dump[N, hsrb_debug_size()] doubles, layout = hsr::debug_dump (csrc/hsr_core.h). */
